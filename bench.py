@@ -4,6 +4,7 @@ frames/sec on 32-frame 518 px clips at 1/2/4/8 GPUs, with roofline fractions).
 
   python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a path
   python bench.py --impl reference --steps K --warmup W    # the reference algorithm on host cores
+  python bench.py ... --dump-outputs DIR                   # also save the last timed step's disparity maps
 
 A step is one ``endodav.forward`` over one synthetic 32-frame 518x518 clip per GPU (ViT-S,
 DV-LoRA, 16-bit tcgen05 path: fp16 operands by default, --dtype bf16 runs the same kernels) -- BASELINE.json configs[1].  At N > 1 every rank runs its own
@@ -20,6 +21,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (it may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -40,6 +42,7 @@ WORKLOADS = {
 }
 METRIC = "frames/sec, 32-frame 518px clips"
 UNIT = "frames/s"
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
 
 
 def measured_peaks():
@@ -198,6 +201,22 @@ def run_reference(args):
 
 
 # --------------------------------------------------------------------------------------------
+def dump_outputs(out, directory):
+    """Write the disparity pyramid that a caller of the timed forward receives as DIR/disp<s>.npy (float32), so that
+    two builds can be compared output for output.  A pyramid above DUMP_LIMIT_BYTES is cut to the same share of every
+    map: a sorted sample of flat indices drawn with a fixed seed, identical from run to run."""
+    import numpy as np
+
+    arrays = {"disp%d" % s: out[("disp", s)].float().cpu().numpy() for s in range(4)}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES:
+            keep = a.size * DUMP_LIMIT_BYTES // total
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def time_forward(E, synthetic, workload, dtype, dev, steps, warmup):
     """Device-timed forward of another workload / dtype on this rank (resident inputs): ms per step, frames/s."""
     import torch
@@ -326,7 +345,11 @@ def main():
     ap.add_argument("--reference-device", default="cpu", choices=["cpu", "cuda"],
                     help="with --impl reference: 'cuda' prints the eager-PyTorch-on-this-GPU sanity line instead of the CPU reference arm")
     ap.add_argument("--no-extras", action="store_true", help="skip the extra measured lines (bf16, 224x280 workloads, video config 3)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the disparity maps of the last timed step (rank 0) to DIR/disp<s>.npy, float32, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -347,9 +370,10 @@ def main():
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
     W = max(3, args.warmup)
-    K = max(1, args.steps)
+    K = args.steps
 
     ctor, (B, T, H, Wd) = WORKLOADS[args.workload]
+    torch.manual_seed(0)   # the base init draws from the global RNG: the same weights in every run and on every rank
     model = E.endodav(dtype=args.dtype, **ctor)
     synthetic.randomize_(model, 1234)
     model = model.to(dev).eval()
@@ -373,7 +397,7 @@ def main():
             if len(pending) >= 2:
                 pending.pop(0).wait()
             pending.append(dist.gather(d0, gather_bufs if rank == 0 else None, dst=0, async_op=True))
-        return d0
+        return out
 
     def drain():
         while pending:
@@ -390,7 +414,7 @@ def main():
         torch.cuda.synchronize()
 
     for _ in range(W):
-        d0 = step(x)
+        step(x)
     eng = model._eng
     launches_per_step = eng.launch_count()
     ws_gb = eng.workspace.numel() / 1e9
@@ -403,7 +427,7 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(K):
-        d0 = step(x)
+        out = step(x)
     drain()          # the current stream waits for the outstanding gathers: they are inside the timed region
     e1.record()
     barrier()
@@ -414,6 +438,9 @@ def main():
         dist.all_reduce(t_ms, op=dist.ReduceOp.MAX)
     ms = float(t_ms.item())
     value = world * frames_per_step * K / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
+    del out
 
     # ---- same K steps with one CUDA event per launch: per-kernel device time ---------------------
     eng.profile(True)
@@ -451,7 +478,7 @@ def main():
                 h2d_ev[j] = torch.cuda.Event()
                 h2d_ev[j].record(h2d_s)
             main_s.wait_event(h2d_ev[j])
-            d0 = step(xbuf[j])
+            d0 = step(xbuf[j])[("disp", 0)]
             free_ev[j] = torch.cuda.Event()
             free_ev[j].record(main_s)
             with torch.cuda.stream(d2h_s):

@@ -1,4 +1,5 @@
 """Helpers shared by the golden-fixture tests (CPU and GPU)."""
+import hashlib
 import json
 import os
 
@@ -24,6 +25,19 @@ def load_case(name):
 
 def oracle_cfg(ctor):
     return weights.full_cfg({k: ctor[k] for k in ORACLE_KEYS if k in ctor})
+
+
+def assert_video_stub_matches(n, got):
+    """video_stub keeps, per video length n, a strided sample of the reference driver's depth and the SHA-256 of
+    its full float32 bytes: the sample localises a mismatch, the digest makes the comparison bit-exact."""
+    m, arrays = load_case("video_stub")
+    ref = arrays["n%d" % n]
+    st = m["stride"]
+    assert got.dtype == np.float32 and got.shape[1:] == tuple(m["input"]), (n, got.dtype, got.shape)
+    sample = got[:, ::st, ::st]
+    assert sample.shape == ref.shape, (n, sample.shape, ref.shape)
+    assert np.array_equal(sample, ref), (n, float(np.abs(sample - ref).max()))
+    assert hashlib.sha256(np.ascontiguousarray(got).tobytes()).hexdigest() == m["sha256"]["n%d" % n], n
 
 
 def subsample_like_golden(name, s, arr):

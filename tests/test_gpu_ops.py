@@ -229,7 +229,7 @@ def test_disp_head_fused(dtype, Fr, h, w, oh, ow, C, sig):
     assert float(err.max()) <= 2e-3 * max(1.0, float(ref.abs().max())), float(err.max())
 
 
-def test_linear_2sm_kernel_matches_default():
+def test_linear_2sm_kernel_matches_default(tmp_path):
     """The experimental cta_group::2 GEMM (gemm_tc2.cuh, EDV_GEMM_2SM=<min M>) must agree bit for bit with
     the default 1-SM kernel: same operands, same fp32 accumulation order per output element (act = none: the two
     kernels evaluate GELU with different, equally accurate formulas), and the TMA-store epilogue of the default
@@ -247,7 +247,7 @@ def test_linear_2sm_kernel_matches_default():
         "torch.save(eng.op_linear(A, W, b, 0).cpu(), sys.argv[1])" % os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
     outs = []
     for v, t in (("0", "1"), ("512", "1"), ("0", "0")):
-        path = "/tmp/edv_lin_%s_%s.pt" % (v, t)
+        path = str(tmp_path / ("lin_%s_%s.pt" % (v, t)))
         env = dict(os.environ, EDV_GEMM_2SM=v, EDV_GEMM_TMA_OUT=t)
         subprocess.run([sys.executable, "-c", code, path], check=True, env=env, timeout=300)
         outs.append(torch.load(path))

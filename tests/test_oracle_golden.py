@@ -7,7 +7,7 @@ import torch
 from oracle import endodav_oracle as orc
 from oracle import video_oracle as vo
 from oracle import weights
-from golden_util import load_case, manifest, oracle_cfg, subsample_like_golden
+from golden_util import assert_video_stub_matches, load_case, manifest, oracle_cfg, subsample_like_golden
 
 FWD = [k for k, v in manifest().items() if v["kind"] == "forward"]
 # fp32 CPU: summation order differs between the restatement (merged LoRA, functional ops)
@@ -92,14 +92,12 @@ def _stub(clip):
 def test_video_stub_bit_exact():
     """Window / keyframe / stitch arithmetic is bit-exact against the reference when the
     network is replaced by the same deterministic stub on both sides."""
-    m, arrays = load_case("video_stub")
+    m, _ = load_case("video_stub")
     H, W = m["input"]
     for N in m["n"]:
         v = weights.make_video_u8(N, H, W, 100 + N)
         got = vo.infer_video_depth(v, tuple(m["image_shape"]), _stub)
-        ref = arrays["n%d" % N]
-        assert got.shape == ref.shape
-        assert np.array_equal(got, ref), (N, float(np.abs(got - ref).max()))
+        assert_video_stub_matches(N, got)
 
 
 def test_window_slots_closed_form():

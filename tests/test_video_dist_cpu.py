@@ -14,7 +14,7 @@ import torch.multiprocessing as mp
 
 from endodav_b200 import video
 from oracle import weights
-from golden_util import load_case
+from golden_util import assert_video_stub_matches, load_case
 
 
 class _Shape:
@@ -61,7 +61,7 @@ def _worker(rank, world, port, n, hw, image_shape, out_path):
 
 @pytest.mark.parametrize("n", [5, 45, 100])
 def test_two_rank_gloo_matches_single_process_and_reference(n, tmp_path):
-    m, arrays = load_case("video_stub")
+    m, _ = load_case("video_stub")
     hw, ishape = m["input"], m["image_shape"]
     out = str(tmp_path / "r0.npy")
     mp.spawn(_worker, args=(2, _free_port(), n, hw, ishape, out), nprocs=2, join=True)
@@ -69,7 +69,7 @@ def test_two_rank_gloo_matches_single_process_and_reference(n, tmp_path):
     v = weights.make_video_u8(n, hw[0], hw[1], 100 + n)
     single = video.infer_video_depth(_Shape(ishape), v, forward_window=_fw, distributed=False)
     assert np.array_equal(dist2, single)
-    assert np.array_equal(single, arrays["n%d" % n])       # the reference's own driver, same stub
+    assert_video_stub_matches(n, single)       # the reference's own driver, same stub
 
 
 def test_shards_partition_the_window_list():
