@@ -77,18 +77,13 @@ void launch_temporal_mma(Launch& L, const void* qkv, void* out, int B, int Tn, i
   launch_temporal_mma_pb<T, HD, 1>(L, qkv, out, B, Tn, hw, rope);
 }
 
-inline bool temporal_simt_forced() {
-  static const bool v = [] { const char* e = getenv("EDV_TEMPORAL_SIMT"); return e && e[0] == '1'; }();
-  return v;
-}
-
 void temporal_attention(Launch& L, int dtype, const void* qkv, void* out, int B, int Tn, int hw, int C,
                                const float* rope) {
   if (!L.ok()) return;
   if (Tn > 32 || Tn < 1) return L.fail(EDV_ERR_ARG, "temporal attention: T must be in [1,32] (motion_module.py:185-197)");
   if (C % 8 != 0) return L.fail(EDV_ERR_ARG, "temporal attention: C must be a multiple of 8");
   const int hd = C / 8;
-  if (dtype != EDV_F32 && !temporal_simt_forced()) {
+  if (dtype != EDV_F32) {
 #define EDV_TM_CASE(HD_)                                                                                   \
     if (hd == HD_) {                                                                                       \
       if (dtype == EDV_BF16) launch_temporal_mma<bf16, HD_>(L, qkv, out, B, Tn, hw, rope);                 \

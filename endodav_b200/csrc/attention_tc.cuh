@@ -33,7 +33,6 @@
 #pragma once
 #include "attention_simt.cuh"
 #include "launch.h"
-#include <cstdlib>
 
 #include "tc_common.cuh"
 
@@ -43,12 +42,11 @@ constexpr int FA_BM = 128;      // query rows per tile
 constexpr int FA_BN = 128;      // keys per iteration
 constexpr int FA_HD = 64;
 constexpr int FA_STAGES = 4;
-constexpr int FA_POLY_DEFAULT = 0;   // every n-th pair of exponentials on the FMA pipe (0: all MUFU)
-constexpr int FA_SPLIT_DEFAULT = 1;  // softmax threads per query row (see the kernel header)
 constexpr uint32_t FA_TILE_BYTES = FA_BM * FA_HD * 2;  // 16 KB: one 128 x 64 16-bit tile
 constexpr int FA_QBUF = 2;           // Q double buffer (items i and i+1)
+constexpr int FA_THREADS = 384;      // producer warpgroup + two softmax warpgroups (see the header)
 constexpr int FA_STAGGER = 1000;     // cycles warpgroup B starts behind warpgroup A (see the header)
-constexpr size_t FA_SMEM = 1024 + (2 * FA_QBUF + 2 * FA_STAGES) * (size_t)FA_TILE_BYTES + 256 + 6 * 1024;   // + barriers + row max / sum exchange
+constexpr size_t FA_SMEM = 1024 + (2 * FA_QBUF + 2 * FA_STAGES) * (size_t)FA_TILE_BYTES + 256;   // + barriers
 
 __device__ __forceinline__ float ex2_approx(float x) {
   float y;
@@ -97,14 +95,6 @@ __device__ __forceinline__ void fma2_bcast(float& d0, float& d1, float a0, float
   asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(rd) : "l"(ra), "l"(rb), "l"(rc));
   asm("mov.b64 {%0, %1}, %2;" : "=f"(d0), "=f"(d1) : "l"(rd));
 }
-__device__ __forceinline__ void fma2(float& d0, float& d1, float a0, float a1, float b0, float b1, float c0, float c1) {
-  uint64_t ra, rb, rc, rd;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(ra) : "f"(a0), "f"(a1));
-  asm("mov.b64 %0, {%1, %2};" : "=l"(rb) : "f"(b0), "f"(b1));
-  asm("mov.b64 %0, {%1, %2};" : "=l"(rc) : "f"(c0), "f"(c1));
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(rd) : "l"(ra), "l"(rb), "l"(rc));
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(d0), "=f"(d1) : "l"(rd));
-}
 __device__ __forceinline__ void add2(float& d0, float& d1, float a0, float a1) {
   uint64_t ra, rd;
   asm("mov.b64 %0, {%1, %2};" : "=l"(ra) : "f"(a0), "f"(a1));
@@ -116,26 +106,6 @@ __device__ __forceinline__ float max3(float a, float b, float c) {
   float r;
   asm("max.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c));
   return r;
-}
-// 2^x for a PAIR on the FMA / ALU pipes (no MUFU), packed fp32x2: x = n + f (round to nearest), degree-3 minimax
-// polynomial for 2^f on [-0.5, 0.5] (max relative error 1.1e-4 < the 16-bit rounding of P: 4.9e-4 fp16,
-// 3.9e-3 bf16), exponent inserted with one integer multiply-add.
-__device__ __forceinline__ void ex2_poly2(float& p0, float& p1, float x0, float x1) {
-  x0 = fmaxf(x0, -125.f);
-  x1 = fmaxf(x1, -125.f);
-  float t0 = x0, t1 = x1;
-  add2(t0, t1, 12582912.f, 12582912.f);            // 1.5 * 2^23: n lands in the low mantissa bits
-  float n0 = t0, n1 = t1;
-  add2(n0, n1, -12582912.f, -12582912.f);
-  float f0, f1;
-  fma2_bcast(f0, f1, n0, n1, -1.0f, 0.f);          // -n
-  add2(f0, f1, x0, x1);                            // f = x - n
-  float q0, q1;
-  fma2_bcast(q0, q1, f0, f1, 0.05550410866f, 0.2402265069f);
-  fma2(q0, q1, q0, q1, f0, f1, 0.6931471806f, 0.6931471806f);
-  fma2(q0, q1, q0, q1, f0, f1, 1.0f, 1.0f);
-  p0 = __int_as_float(__float_as_int(q0) + (__float_as_int(t0) << 23));
-  p1 = __int_as_float(__float_as_int(q1) + (__float_as_int(t1) << 23));
 }
 
 struct FaItem {
@@ -152,24 +122,11 @@ __device__ __forceinline__ FaItem fa_item(int w, int nx, int heads, int S) {
   return it;
 }
 
-__device__ __forceinline__ void named_bar_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
-__device__ __forceinline__ void named_bar_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
-
-// PM: every PM-th PAIR of exponentials is evaluated with ex2_poly2 on the FMA pipe (0: all MUFU).
-// SPLIT: threads per query row.  1: two softmax warpgroups, thread = row (128 scores in registers).  2: FOUR softmax
-//     warpgroups (640 threads), a row's 128 scores are split between two threads of different warpgroups (same TMEM
-//     lane quarter); they exchange the row max through shared memory + a 64-thread named barrier once per key block
-//     and their partial row sums once per item.  Why: ONE warp sustains only ~13 cycles per MUFU instruction in this
-//     instruction mix (scoreboard round trips between ex2 and its consumers), so two warps per scheduler leave the MUFU
-//     pipe 35-40 % idle; four warps per scheduler can cover it (tools/microbench mix: 11.6 / 9.3 / 8.1 cycles per MUFU
-//     with 1 / 2 / 4 warps per scheduler).  MEASURED SLOWER (200 vs 172 us at 32 x 6 x 1370): the two tiles run in
-//     phase, so the four warps' exponentials coincide (1 800 cycles) and so do their longer non-MUFU phases (load 450,
-//     max + exchange 450, P store 250).  Forcing the tiles into anti-phase with a pair of named barriers around the
-//     exponentials (MUFU ping-pong, instructions pinned with data dependencies -- ptxas moves register-only code across
-//     BAR) gave 1 280-cycle phases but 198 us: a block then costs two exclusive phases plus the hand-over.  Kept as
-//     EDV_FA_SPLIT=2 for the record; the default is 1.
-template <typename T, int PM, int SPLIT>
-__global__ void __launch_bounds__(128 + 256 * SPLIT, 1)
+// Two threads per query row (four softmax warpgroups, row max / sum exchanged through shared memory) and evaluating
+// part of the exponentials as a polynomial on the FMA pipe were both measured slower than one thread per row with every
+// exp2 on the MUFU (DESIGN.md section 5, profiles/r2_fa_variants_timeline.txt).
+template <typename T>
+__global__ void __launch_bounds__(FA_THREADS, 1)
     flash_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, T* __restrict__ out, int S, int heads, int nx,
                               int total_items, long long* __restrict__ tim) {
   pdl_launch();   // PDL: the next kernel of the stream may start its prologue (common.cuh)
@@ -194,7 +151,6 @@ __global__ void __launch_bounds__(128 + 256 * SPLIT, 1)
   uint64_t* s_free = o_done + 2;                 // 2: warpgroup t holds S_t(j) in registers
   uint64_t* pv_done = s_free + 2;                // 2: O_t += P_t(j) V_j has completed
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(pv_done + 2);
-  float* xch = reinterpret_cast<float*>(bars + 32);   // SPLIT == 2: row max [parity][tile][half][row], then row sum [tile][half][row]
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int D = heads * FA_HD;
@@ -212,9 +168,9 @@ __global__ void __launch_bounds__(128 + 256 * SPLIT, 1)
     }
     for (int t = 0; t < 2; ++t) {
       mbar_init(&s_full[t], 1);
-      mbar_init(&p_full[t], 128 * SPLIT);
+      mbar_init(&p_full[t], 128);
       mbar_init(&o_done[t], 1);
-      mbar_init(&s_free[t], 128 * SPLIT);
+      mbar_init(&s_free[t], 128);
       mbar_init(&pv_done[t], 1);
     }
     fence_barrier_init();
@@ -229,8 +185,7 @@ __global__ void __launch_bounds__(128 + 256 * SPLIT, 1)
   if (tm_ && threadIdx.x == 0) tm_[1] = clock64();
 
   if (warp < 4) {
-   if (SPLIT == 1) asm volatile("setmaxnreg.dec.sync.aligned.u32 56;");
-   else asm volatile("setmaxnreg.dec.sync.aligned.u32 56;");   // 640 threads launch with 96: frees 128 x 40 registers ...
+   asm volatile("setmaxnreg.dec.sync.aligned.u32 56;");
    if (warp == 0) {
     // ===== TMA producer =====
     if (lane == 0) {
@@ -342,22 +297,16 @@ __global__ void __launch_bounds__(128 + 256 * SPLIT, 1)
    }
   } else {
     // ===== softmax warpgroups =====
-    if (SPLIT == 1) asm volatile("setmaxnreg.inc.sync.aligned.u32 224;");
-    else asm volatile("setmaxnreg.inc.sync.aligned.u32 104;");  // ... which is all the CTA pool holds: 512 x 8 <= 5120 (112 would wait forever)
-    constexpr int NC = FA_BN / SPLIT;     // scores per thread and key block
-    constexpr int OC = FA_HD / SPLIT;     // O columns per thread
-    const int g = (warp - 4) >> 2;        // softmax warpgroup
-    const int t = g & 1;                  // 0: tile A, 1: tile B
-    const int hh = g >> 1;                // which half of the row's columns (SPLIT == 2)
+    asm volatile("setmaxnreg.inc.sync.aligned.u32 224;");
+    const int t = (warp - 4) >> 2;        // softmax warpgroup = query tile (0: tile A, 1: tile B)
     const int q = warp & 3;               // TMEM lane quarter this warp may access
     const int r = q * 32 + lane;          // row inside the tile
     const uint32_t lane_off = (uint32_t)(q * 32) << 16;
-    const uint32_t tS = tmem_base + lane_off + t * FA_BN + hh * NC;
-    const uint32_t tO = tmem_base + lane_off + 256 + t * FA_HD + hh * OC;
-    const uint32_t tP = tmem_base + lane_off + 384 + t * 64 + hh * (NC / 2);
-    const int pair_bar = 1 + t * 4 + q;   // named barrier of the two warps that share these 32 rows
+    const uint32_t tS = tmem_base + lane_off + t * FA_BN;
+    const uint32_t tO = tmem_base + lane_off + 256 + t * FA_HD;
+    const uint32_t tP = tmem_base + lane_off + 384 + t * 64;
     constexpr float LOG2E = 1.4426950408889634f;
-    const bool stamp = tm_ && t == 0 && r == 0 && hh == 0;
+    const bool stamp = tm_ && t == 0 && r == 0;
     if (t == 1) {
       // start half a key block behind warpgroup A (see the header): the offset persists, both warpgroups run the same loop
       const long long c0 = clock64();
@@ -371,22 +320,22 @@ __global__ void __launch_bounds__(128 + 256 * SPLIT, 1)
       if (t >= im.nt) continue;
       const int row_base = im.f * S;
       float m_used = -INFINITY;           // max the exponentials are currently taken against (raw units)
-      float l = 0.f;                      // (partial, SPLIT == 2) row sum
+      float l = 0.f;                      // row sum
       for (int j = 0; j < n_iter; ++j, ++cnt) {
         mbar_wait(&s_full[t], cnt & 1);
         fence_after_sync();
         if (stamp && cnt == 0) tm_[2] = clock64();
-        uint32_t sv[NC];
+        uint32_t sv[FA_BN];
 #pragma unroll
-        for (int c = 0; c < NC; c += 32) tmem_ld32_nowait(tS + c, sv + c);
+        for (int c = 0; c < FA_BN; c += 32) tmem_ld32_nowait(tS + c, sv + c);
         tmem_ld_wait();
         fence_before_sync();
         mbar_arrive(&s_free[t]);          // S_t(j) is in registers: the tensor core may overwrite it with the next S_t
         if (stamp && cnt == 5) tm_[44] = clock64();
-        const int valid = S - j * FA_BN - hh * NC;  // keys of this thread's columns that belong to the frame
-        if (valid < NC) {
+        const int valid = S - j * FA_BN;  // keys of this block that belong to the frame
+        if (valid < FA_BN) {
 #pragma unroll
-          for (int i = 0; i < NC; ++i)
+          for (int i = 0; i < FA_BN; ++i)
             if (i >= valid) sv[i] = 0xff800000u;  // -inf
         }
         // row max: 8 independent chains of 3-input maxima (FMNMX3)
@@ -394,22 +343,14 @@ __global__ void __launch_bounds__(128 + 256 * SPLIT, 1)
 #pragma unroll
         for (int i = 0; i < 8; ++i) pm[i] = max3(__uint_as_float(sv[i]), __uint_as_float(sv[8 + i]), __uint_as_float(sv[16 + i]));
 #pragma unroll
-        for (int i = 24; i < NC - 8; i += 16) {
+        for (int i = 24; i < FA_BN - 8; i += 16) {
 #pragma unroll
           for (int c = 0; c < 8; ++c) pm[c] = max3(pm[c], __uint_as_float(sv[i + c]), __uint_as_float(sv[i + 8 + c]));
         }
 #pragma unroll
-        for (int c = 0; c < 8; ++c) pm[c] = fmaxf(pm[c], __uint_as_float(sv[NC - 8 + c]));
-        float mx = fmaxf(max3(pm[0], pm[1], pm[2]), fmaxf(max3(pm[3], pm[4], pm[5]), fmaxf(pm[6], pm[7])));
-        if (SPLIT == 2) {
-          // the other half of the row: parity double buffer, so one barrier per key block orders write -> read -> rewrite
-          float* xm = xch + ((cnt & 1) * 2 + t) * 256 + r;
-          xm[hh * 128] = mx;
-          named_bar_sync(pair_bar, 64);
-          mx = fmaxf(mx, xm[(hh ^ 1) * 128]);
-        }
-        // lazy rescale: keep the old reference max unless the row max grew by more than 2^8 (both halves of a row see
-        // the same mx and m_used, so they take the same decision)
+        for (int c = 0; c < 8; ++c) pm[c] = fmaxf(pm[c], __uint_as_float(sv[FA_BN - 8 + c]));
+        const float mx = fmaxf(max3(pm[0], pm[1], pm[2]), fmaxf(max3(pm[3], pm[4], pm[5]), fmaxf(pm[6], pm[7])));
+        // lazy rescale: keep the old reference max unless the row max grew by more than 2^8
         float factor = 1.f;
         const bool grow = mx > m_used + 8.f / LOG2E;
         if (grow) {
@@ -422,17 +363,12 @@ __global__ void __launch_bounds__(128 + 256 * SPLIT, 1)
         const float neg = -m_used * LOG2E;
         if (stamp && cnt == 5) tm_[45] = clock64();
         float ls0 = 0.f, ls1 = 0.f, ls2 = 0.f, ls3 = 0.f;   // two packed partial row sums
-        uint32_t pv[NC / 2];
+        uint32_t pv[FA_BN / 2];
 #pragma unroll
-        for (int i = 0; i < NC / 2; ++i) {
-          float x0, x1, p0, p1;
+        for (int i = 0; i < FA_BN / 2; ++i) {
+          float x0, x1;
           fma2_bcast(x0, x1, __uint_as_float(sv[2 * i]), __uint_as_float(sv[2 * i + 1]), LOG2E, neg);
-          if (PM > 0 && (i % (PM > 0 ? PM : 1)) == (PM > 0 ? PM - 1 : 0)) {
-            ex2_poly2(p0, p1, x0, x1);
-          } else {
-            p0 = ex2_approx(x0);
-            p1 = ex2_approx(x1);
-          }
+          const float p0 = ex2_approx(x0), p1 = ex2_approx(x1);
           if (i & 1) add2(ls2, ls3, p0, p1);
           else add2(ls0, ls1, p0, p1);
           pv[i] = pack_pair(p0, p1, T());
@@ -445,7 +381,7 @@ __global__ void __launch_bounds__(128 + 256 * SPLIT, 1)
           if (stamp && cnt == 5) tm_[47] = clock64();
           if (__any_sync(0xffffffffu, grow)) {
 #pragma unroll
-            for (int c = 0; c < OC; c += 32) {
+            for (int c = 0; c < FA_HD; c += 32) {
               uint32_t ov[32];
               tmem_ld32_nowait(tO + c, ov);
               tmem_ld_wait();
@@ -457,7 +393,7 @@ __global__ void __launch_bounds__(128 + 256 * SPLIT, 1)
         }
         // (j == 0: the last PV of this tile's previous item completed before its epilogue read O -- o_done)
 #pragma unroll
-        for (int c = 0; c < NC / 2; c += 32) tmem_st32(tP + c, pv + c);
+        for (int c = 0; c < FA_BN / 2; c += 32) tmem_st32(tP + c, pv + c);
         tmem_st_wait();
         fence_before_sync();
         mbar_arrive(&p_full[t]);
@@ -465,22 +401,14 @@ __global__ void __launch_bounds__(128 + 256 * SPLIT, 1)
         if (stamp && cnt < 16) tm_[3 + cnt] = clock64();
       }
       // ---- epilogue: O / l -> global ----
-      if (SPLIT == 2) {
-        // full row sum = the two halves' partial sums (the n_iter >= 1 row-max barriers since the previous item's
-        // exchange order the reuse of this buffer)
-        float* xl = xch + 1024 + t * 256 + r;
-        xl[hh * 128] = l;
-        named_bar_sync(pair_bar, 64);
-        l += xl[(hh ^ 1) * 128];
-      }
       mbar_wait(&o_done[t], items & 1);
       fence_after_sync();
       if (stamp && items == 0) tm_[20] = clock64();
       const float inv = 1.f / l;
       const int qi = im.q0 + t * FA_BM + r;
-      T* orow = out + ((long long)row_base + qi) * D + im.h * FA_HD + hh * OC;
+      T* orow = out + ((long long)row_base + qi) * D + im.h * FA_HD;
 #pragma unroll
-      for (int c = 0; c < OC; c += 32) {
+      for (int c = 0; c < FA_HD; c += 32) {
         uint32_t ov[32];
         tmem_ld32_nowait(tO + c, ov);
         tmem_ld_wait();
@@ -514,30 +442,17 @@ void launch_attention_tc(edv::Launch& L, int dtype, const void* qkv, void* out, 
   uint64_t str[1] = {(uint64_t)3 * D * 2};
   uint32_t box[2] = {(uint32_t)FA_HD, (uint32_t)FA_BM};
   if (!make_map(L, &tm, dtype, qkv, 2, dims, str, box, 128)) return;
-  // EDV_FA_POLY=<0|4|8>: every n-th pair of exponentials on the FMA pipe (0 = all MUFU); EDV_FA_SPLIT=<1|2>: threads per row
-  static int pm = -1, split = -1;
-  if (pm < 0) {
-    const char* env = getenv("EDV_FA_POLY");
-    pm = env ? atoi(env) : FA_POLY_DEFAULT;
-    if (pm != 0 && pm != 4 && pm != 8) pm = FA_POLY_DEFAULT;
-    const char* e2 = getenv("EDV_FA_SPLIT");
-    split = e2 ? atoi(e2) : FA_SPLIT_DEFAULT;
-    if (split != 1 && split != 2) split = FA_SPLIT_DEFAULT;
-  }
-  void (*kern)(const CUtensorMap, T*, int, int, int, int, long long*) =
-      split == 1 ? flash_attention_tc_kernel<T, 0, 1>
-                 : pm == 0 ? flash_attention_tc_kernel<T, 0, 2> : pm == 4 ? flash_attention_tc_kernel<T, 4, 2> : flash_attention_tc_kernel<T, 8, 2>;
-  const int slot = split == 1 ? 0 : pm == 0 ? 1 : pm == 4 ? 2 : 3;
-  static bool attr_done[4] = {false, false, false, false};
-  if (!attr_done[slot]) {
+  auto kern = flash_attention_tc_kernel<T>;
+  static bool attr_done = false;
+  if (!attr_done) {
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FA_SMEM);
-    attr_done[slot] = true;
+    attr_done = true;
   }
   const int nx = (S + 2 * FA_BM - 1) / (2 * FA_BM);
   const long long total = (long long)nx * heads * F;
   if (total > 0x7fffffffLL) return L.fail(EDV_ERR_ARG, "flash_attention_tc: too many work items");
   const int grid = (int)std::min<long long>(total, edv::num_sms());
-  edv::launch_k(kern, dim3(grid), dim3(128 + 256 * split), FA_SMEM, L.stream, tm, (T*)out, S, heads, nx, (int)total, timeline);
+  edv::launch_k(kern, dim3(grid), dim3(FA_THREADS), FA_SMEM, L.stream, tm, (T*)out, S, heads, nx, (int)total, timeline);
   L.check("flash_attention_tc");
 }
 

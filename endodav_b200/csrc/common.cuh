@@ -229,7 +229,6 @@ struct Epi {
   float sig_sign;  // ACT_SIGMOID: sigmoid(sig_sign * x)
   int kind;        // tcgen05 epilogue specialisation (gemm_tc.cuh EF_* mask) or -1: set by the launcher
   long long* tim;  // optional in-kernel timeline of gemm_tc_kernel (edv_op_linear_timeline), else null
-  int dbg;         // timeline experiments only (EDV_GEMM_DBG): 1 skip the epilogue work, 2 skip the A loads (results are garbage)
 };
 
 // maps GEMM row m -> output row for the column-independent mappings

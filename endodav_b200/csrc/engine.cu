@@ -1227,7 +1227,6 @@ int edv_op_linear_timeline(int dtype, const void* A, const void* W, const float*
   a.e = epi_zero();
   a.e.out = C; a.e.ldo = N; a.e.bias = bias; a.e.act = act;
   a.e.tim = timeline_dev;
-  if (const char* env = getenv("EDV_GEMM_DBG")) a.e.dbg = atoi(env);
   gemm(L, dtype, EDV_ENGINE_TC, a);
   return finish(L);
 }

@@ -180,10 +180,6 @@ __global__ void __launch_bounds__(GB_THREADS, 1) gemm_bres_kernel(const __grid_c
         for (int kb = 0; kb < kblocks; ++kb, ++kc) {
           const int s = kc % stages;
           mbar_wait(&empty_bar[s], ((kc / stages) & 1) ^ 1);
-          if (e.dbg & 2) {
-            mbar_arrive(&full_bar[s]);
-            continue;
-          }
           mbar_expect_tx(&full_bar[s], GB_A_STAGE);
           tma_load_2d(sA + (size_t)s * GB_A_STAGE, &tmA, &full_bar[s], kb * 64, tm * GT_BM);
         }
@@ -243,12 +239,6 @@ __global__ void __launch_bounds__(GB_THREADS, 1) gemm_bres_kernel(const __grid_c
       if (stamp) tm_[10 + 4 * it] = clock64();
       const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16) + b * BN + wg * CW;
       const int row0 = tm * GT_BM, col0 = tile_n * BN + wg * CW;
-      if (e.dbg & 1) {
-        fence_before_sync();
-        mbar_arrive(&tempty_bar[b]);
-        if (stamp) tm_[11 + 4 * it] = clock64();
-        continue;
-      }
       switch (kind) {
         case EF_BIAS: gb_epilogue<T, BN, EF_BIAS>(&tmC, trow, row0, col0, r, wg, stg_wg, bias_s, &tempty_bar[b]); break;
         case EF_BIAS | EF_GELU: gb_epilogue<T, BN, EF_BIAS | EF_GELU>(&tmC, trow, row0, col0, r, wg, stg_wg, bias_s, &tempty_bar[b]); break;

@@ -25,7 +25,7 @@
 //   warp 17 (virtual 1)   TMEM allocator + MMA issuer (warp-uniform loop, elected lane)
 //   warps 0..15           four epilogue warpgroups
 #pragma once
-#include "gemm_tc2.cuh"
+#include "gemm_tc.cuh"
 
 namespace tc {
 

@@ -1,25 +1,19 @@
-// Host launchers of the tcgen05 GEMM family (gemm_tc.cuh, gemm_tc2.cuh, conv_halo.cuh).  Included by
+// Host launchers of the tcgen05 GEMM family (gemm_tc.cuh, gemm_bres.cuh, gemm_ln.cuh, conv_halo.cuh).  Included by
 // the gemm_tc_*.cu translation units, each of which explicitly instantiates one (dtype, lin|conv) slice.
 #pragma once
 #include "ops.h"
 #include "gemm_tc.cuh"
-#include "gemm_tc2.cuh"
 #include "gemm_bres.cuh"
 #include "gemm_ln.cuh"
 #include "conv_halo.cuh"
 
 namespace edv {
 
-// EDV_GEMM_TMA_OUT=0 falls back to the row-segment epilogue everywhere (A/B measurements)
-inline bool gemm_tma_out_enabled() {
-  static const bool v = [] { const char* e = getenv("EDV_GEMM_TMA_OUT"); return !(e && e[0] == '0'); }();
-  return v;
-}
 // the TMA-store epilogue handles 16-bit row-major outputs with bias / GELU / ReLU only
 inline bool gemm_tma_out_ok(const GemmArgs& a) {
   using namespace tc;
   const int k = a.e.kind;
-  if (!gemm_tma_out_enabled() || a.conv || k < 0) return false;
+  if (a.conv || k < 0) return false;
   if (k != 0 && k != EF_BIAS && k != (EF_BIAS | EF_GELU) && k != (EF_BIAS | EF_RELU)) return false;
   if (a.e.map != MAP_LINEAR || a.e.out_f32 || !a.e.out) return false;
   if ((a.e.ldo * 2) % 16 != 0 || ((uintptr_t)a.e.out & 15) != 0) return false;
@@ -114,54 +108,6 @@ inline bool conv_halo_ok(const GemmArgs& a) {
          (a.e.act == ACT_NONE || a.e.act == ACT_RELU || a.e.act == ACT_SIGMOID) && a.e.map == MAP_LINEAR;
 }
 
-// 2-SM (cta_group::2) GEMM for the big token GEMMs (gemm_tc2.cuh)
-template <typename T, int BN> void launch_gemm_tc2(Launch& L, int dtype, const GemmArgs& a) {
-  using namespace tc;
-  CUtensorMap tmA, tmB;
-  {
-    uint64_t dims[2] = {(uint64_t)a.K, (uint64_t)a.M};
-    uint64_t str[1] = {(uint64_t)a.lda * 2};
-    uint32_t box[2] = {64u, (uint32_t)GT_BM};
-    if (!make_tmap(L, &tmA, dtype, a.A, 2, dims, str, box, 128)) return;
-  }
-  {
-    uint64_t dims[2] = {(uint64_t)a.K, (uint64_t)a.N};
-    uint64_t str[1] = {(uint64_t)a.K * 2};
-    uint32_t box[2] = {64u, (uint32_t)(BN / 2)};
-    if (!make_tmap(L, &tmB, dtype, a.W, 2, dims, str, box, 128)) return;
-  }
-  const size_t stg_bytes = 16 * (size_t)GT_STG_WORDS * 4 + 16 * 128 * 4;
-  const int stage_bytes = gt2_stage_bytes<BN>();
-  int stages = (int)((220 * 1024 - stg_bytes - 2048) / stage_bytes);
-  if (stages > 8) stages = 8;
-  const size_t smem = (size_t)stages * stage_bytes + 1024 + (2 * stages + 4) * 8 + 16 + stg_bytes;
-  auto kern = gemm_tc2_kernel<T, BN>;
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024);
-    attr_done = true;
-  }
-  const int n_tiles = a.N / BN;
-  const long long total = (long long)((a.M + 255) / 256) * n_tiles;
-  int pairs = (int)std::min<long long>(total, num_sms() / 2);
-  note_gemm(L, a, 2);
-  kern<<<2 * pairs, GT_THREADS, smem, L.stream>>>(tmA, tmB, a.e, a.M, a.N, a.K, stages, n_tiles, (int)total);
-  L.check("gemm_tc2");
-}
-
-constexpr int GEMM_2SM_DEFAULT_MIN_M_DECL = 0;
-// EDV_GEMM_2SM=<min M> routes linear GEMMs with at least that many rows to the 2-SM kernel (0 = off)
-inline int gemm_2sm_min_m() {
-  static int v = -1;
-  if (v < 0) {
-    const char* env = getenv("EDV_GEMM_2SM");
-    v = env ? atoi(env) : GEMM_2SM_DEFAULT_MIN_M_DECL;
-    if (v < 0) v = 0;
-  }
-  return v;
-}
-
-
 inline int gemm_tc_pick_bk(const GemmArgs& a) { return (a.conv ? (a.C % 64 != 0) : (a.K % 64 != 0)) ? 32 : 64; }
 
 inline int gemm_tc_pick_bn(const GemmArgs& a, int bk) {
@@ -198,10 +144,6 @@ template <typename T, bool CONV> void launch_gemm_tc_any(Launch& L, int dtype, c
 
 #ifdef EDV_GEMM_TU_LIN
 // B-resident GEMM (gemm_bres.cuh): short K, 16-bit output through the TMA-store epilogue
-inline bool gemm_bres_enabled() {
-  static const bool v = [] { const char* e = getenv("EDV_GEMM_BRES"); return !(e && e[0] == '0'); }();
-  return v;
-}
 constexpr size_t GB_SMEM_MAX = 232448 - 1024;   // 227 KB opt-in limit minus the alignment slack
 
 template <typename T, int BN> bool launch_gemm_bres(Launch& L, int dtype, const GemmArgs& a) {
@@ -294,13 +236,9 @@ void launch_gemm_ln(Launch& L, int dtype, const void* A, const void* W, const fl
   L.check("gemm_ln");
 }
 
-#ifdef EDV_GEMM_LN_DEFS
-inline bool gemm_ln_enabled() {
-  static const bool v = [] { const char* e = getenv("EDV_GEMM_LN"); return !(e && e[0] == '0'); }();
-  return v;
-}
+#ifdef EDV_GEMM_TU_LN
 bool gemm_ln_supported(int dtype, int N, int K) {
-  return gemm_ln_enabled() && dtype != EDV_F32 && N == tc::GL_N && K % 64 == 0 && K >= 64;
+  return dtype != EDV_F32 && N == tc::GL_N && K % 64 == 0 && K >= 64;
 }
 void gemm_ln(Launch& L, int dtype, const void* A, const void* W, const float* bias, float* x, void* xn, const float* gamma,
              const float* beta, float eps, int M, int N, int K, int do_ln, long long* tim) {
@@ -313,15 +251,10 @@ void gemm_ln(Launch& L, int dtype, const void* A, const void* W, const float* bi
 
 // linear GEMMs (2-D A operand)
 template <typename T> void launch_gemm_tc_lin(Launch& L, int dtype, const GemmArgs& a) {
-  if (gemm_bres_enabled() && gemm_tma_out_ok(a) && a.K % 64 == 0 && a.K <= 384 && a.lda == a.K && a.M >= 2048) {
+  if (gemm_tma_out_ok(a) && a.K % 64 == 0 && a.K <= 384 && a.lda == a.K && a.M >= 2048) {
     if (a.N % 192 == 0) { if (launch_gemm_bres<T, 192>(L, dtype, a)) return; }
     else if (a.N % 128 == 0) { if (launch_gemm_bres<T, 128>(L, dtype, a)) return; }
     else if (a.N % 64 == 0) { if (launch_gemm_bres<T, 64>(L, dtype, a)) return; }
-  }
-  if (gemm_2sm_min_m() > 0 && a.M >= gemm_2sm_min_m() && a.K % 64 == 0 && a.lda == a.K && a.e.act != ACT_GEGLU &&
-      a.e.act != ACT_HEAD) {
-    if (a.N % 256 == 0) return launch_gemm_tc2<T, 256>(L, dtype, a);
-    if (a.N % 192 == 0) return launch_gemm_tc2<T, 192>(L, dtype, a);
   }
   launch_gemm_tc_any<T, false>(L, dtype, a);
 }

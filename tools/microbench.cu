@@ -388,6 +388,35 @@ template <int OP> void run_pipe(const char* what, float* d_f, long long* d_out, 
 
 
 // ---- the exponential phase of the flash-attention softmax, as an instruction mix ---------------------------------
+__device__ __forceinline__ void fma2(float& d0, float& d1, float a0, float a1, float b0, float b1, float c0, float c1) {
+  uint64_t ra, rb, rc, rd;
+  asm("mov.b64 %0, {%1, %2};" : "=l"(ra) : "f"(a0), "f"(a1));
+  asm("mov.b64 %0, {%1, %2};" : "=l"(rb) : "f"(b0), "f"(b1));
+  asm("mov.b64 %0, {%1, %2};" : "=l"(rc) : "f"(c0), "f"(c1));
+  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(rd) : "l"(ra), "l"(rb), "l"(rc));
+  asm("mov.b64 {%0, %1}, %2;" : "=f"(d0), "=f"(d1) : "l"(rd));
+}
+// 2^x for a PAIR on the FMA / ALU pipes (no MUFU), packed fp32x2: x = n + f (round to nearest), degree-3 minimax
+// polynomial for 2^f on [-0.5, 0.5] (max relative error 1.1e-4 < the 16-bit rounding of P: 4.9e-4 fp16,
+// 3.9e-3 bf16), exponent inserted with one integer multiply-add.
+__device__ __forceinline__ void ex2_poly2(float& p0, float& p1, float x0, float x1) {
+  x0 = fmaxf(x0, -125.f);
+  x1 = fmaxf(x1, -125.f);
+  float t0 = x0, t1 = x1;
+  add2(t0, t1, 12582912.f, 12582912.f);            // 1.5 * 2^23: n lands in the low mantissa bits
+  float n0 = t0, n1 = t1;
+  add2(n0, n1, -12582912.f, -12582912.f);
+  float f0, f1;
+  fma2_bcast(f0, f1, n0, n1, -1.0f, 0.f);          // -n
+  add2(f0, f1, x0, x1);                            // f = x - n
+  float q0, q1;
+  fma2_bcast(q0, q1, f0, f1, 0.05550410866f, 0.2402265069f);
+  fma2(q0, q1, q0, q1, f0, f1, 0.6931471806f, 0.6931471806f);
+  fma2(q0, q1, q0, q1, f0, f1, 1.0f, 1.0f);
+  p0 = __int_as_float(__float_as_int(q0) + (__float_as_int(t0) << 23));
+  p1 = __int_as_float(__float_as_int(q1) + (__float_as_int(t1) << 23));
+}
+
 // Each thread owns NP pairs of scores in registers and runs, per "key block":  x = s * log2e - m (FFMA2), p = ex2(x)
 // (2 MUFU), row sum (FADD2), 16-bit pack (F2FP) -- attention_tc.cuh's loop.  MODE bit 0: drop the pack, bit 1: drop the
 // row sum, bit 2: every 4th pair through the FMA-pipe polynomial.  Reports cycles per MUFU warp-instruction per SMSP

@@ -38,8 +38,8 @@ if which == "attn":
     out = eng.op_attention(qkv, 32, 1370, 6).float()
     t = qkv[:1370 * 2].float().reshape(2, 1370, 3, 6, 64).permute(2, 0, 3, 1, 4)
     r = ((t[0] @ t[1].transpose(-1, -2)).softmax(-1) @ t[2]).transpose(1, 2).reshape(2 * 1370, 384)
-    print("attn EDV_FA_POLY=%s: %.1f us  (%.1f TFLOP/s)  max err vs fp32 %.3g" % (
-        os.environ.get("EDV_FA_POLY", "default"), us, 4 * 32 * 6 * 1370 * 1370 * 64 / us / 1e6, float((out[:2740] - r).abs().max())))
+    print("attn: %.1f us  (%.1f TFLOP/s)  max err vs fp32 %.3g" % (
+        us, 4 * 32 * 6 * 1370 * 1370 * 64 / us / 1e6, float((out[:2740] - r).abs().max())))
 elif which in ("qkv", "fc1", "fc2", "proj"):
     N, K, act = {"qkv": (1152, 384, 0), "fc1": (1536, 384, 1), "fc2": (384, 1536, 0), "proj": (384, 384, 0)}[which]
     A, W, b = rnd(M, K), rnd(N, K, scale=K ** -0.5), torch.zeros(N).cuda()
@@ -47,8 +47,7 @@ elif which in ("qkv", "fc1", "fc2", "proj"):
     got = eng.op_linear(A[:512], W, b, act).float()
     ref = torch.nn.functional.linear(A[:512].float(), W.float())
     ref = torch.nn.functional.gelu(ref) if act else ref
-    print("%s EDV_GEMM_2SM=%s: %.1f us (%.0f TFLOP/s) max err %.3g" % (which, os.environ.get("EDV_GEMM_2SM", "0"), us,
-                                                                      2.0 * M * N * K / us / 1e6, float((got - ref).abs().max())))
+    print("%s: %.1f us (%.0f TFLOP/s) max err %.3g" % (which, us, 2.0 * M * N * K / us / 1e6, float((got - ref).abs().max())))
 elif which == "ln":
     x = torch.randn(M, 384, generator=g).cuda()
     gam, bet = torch.ones(384).cuda(), torch.zeros(384).cuda()
