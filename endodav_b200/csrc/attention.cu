@@ -12,8 +12,8 @@ void attention(Launch& L, int dtype, int engine, const void* qkv, void* out, int
   // QK^T + PV: 4*S*S*64 per (frame, head); q,k,v read once, o written once
   L.note(4.0 * F * heads * (double)S * S * 64, 4.0 * F * S * heads * 64 * dtype_size(dtype));
   if (dtype != EDV_F32 && engine == EDV_ENGINE_TC) {
-    if (dtype == EDV_BF16) tc::launch_attention_tc<bf16>(L, dtype, qkv, out, F, S, heads, &make_tmap, timeline);
-    else tc::launch_attention_tc<f16>(L, dtype, qkv, out, F, S, heads, &make_tmap, timeline);
+    if (dtype == EDV_BF16) tc::launch_attention_tc<bf16>(L, dtype, qkv, out, F, S, heads, timeline);
+    else tc::launch_attention_tc<f16>(L, dtype, qkv, out, F, S, heads, timeline);
     return;
   }
   dim3 grid((S + 127) / 128, heads, F);
@@ -35,12 +35,8 @@ void launch_temporal(Launch& L, const void* qkv, void* out, int B, int Tn, int h
   while (hg > 1 && 32 * hg * pb > ta_max_threads<HD>()) hg >>= 1;
   if (pb > hw) pb = hw;
   const size_t smem = (size_t)pb * hg * per + (size_t)Tn * 16 + 16;
-  auto kern = temporal_attention_kernel<T, HD>;
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    attr_done = true;
-  }
+  constexpr auto kern = temporal_attention_kernel<T, HD>;
+  smem_opt_in<kern>(200 * 1024);
   dim3 grid((hw + pb - 1) / pb, B, heads / hg);
   L.note(4.0 * B * hw * heads * (double)Tn * Tn * HD, 4.0 * B * Tn * hw * C * sizeof(T));
   kern<<<grid, 32 * hg * pb, smem, L.stream>>>((const T*)qkv, (T*)out, Tn, hw, C, pb, hg, (const float2*)rope);   // fp32 CUDA-core path: no PDL hooks, plain launch
@@ -49,13 +45,9 @@ void launch_temporal(Launch& L, const void* qkv, void* out, int B, int Tn, int h
 
 template <typename T, int HD, int PB>
 void launch_temporal_mma_pb(Launch& L, const void* qkv, void* out, int B, int Tn, int hw, const float* rope) {
-  auto kern = tmma::temporal_attention_mma_kernel<T, HD, PB>;
+  constexpr auto kern = tmma::temporal_attention_mma_kernel<T, HD, PB>;
   const size_t smem = PB * tmma::ta_smem_per_pos<HD>();
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    attr_done = true;
-  }
+  smem_opt_in<kern>((int)smem);
   dim3 grid((hw + PB - 1) / PB, B);
   const int C = 8 * HD;
   L.note(4.0 * B * hw * 8 * (double)Tn * Tn * HD, 4.0 * B * Tn * hw * C * sizeof(T));

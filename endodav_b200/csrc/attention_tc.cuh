@@ -32,7 +32,7 @@
 // TMEM columns (512): S_A [0,128) S_B [128,256) O_A [256,320) O_B [320,384) P_A [384,448) P_B [448,512)
 #pragma once
 #include "attention_simt.cuh"
-#include "launch.h"
+#include "ops.h"
 
 #include "tc_common.cuh"
 
@@ -433,21 +433,12 @@ __global__ void __launch_bounds__(FA_THREADS, 1)
 }
 
 template <typename T>
-void launch_attention_tc(edv::Launch& L, int dtype, const void* qkv, void* out, int F, int S, int heads,
-                         bool (*make_map)(edv::Launch&, CUtensorMap*, int, const void*, int, const uint64_t*,
-                                          const uint64_t*, const uint32_t*, int), long long* timeline = nullptr) {
-  const int D = heads * FA_HD;
+void launch_attention_tc(edv::Launch& L, int dtype, const void* qkv, void* out, int F, int S, int heads, long long* timeline = nullptr) {
+  const uint64_t D = heads * FA_HD;
   CUtensorMap tm;
-  uint64_t dims[2] = {(uint64_t)3 * D, (uint64_t)F * S};
-  uint64_t str[1] = {(uint64_t)3 * D * 2};
-  uint32_t box[2] = {(uint32_t)FA_HD, (uint32_t)FA_BM};
-  if (!make_map(L, &tm, dtype, qkv, 2, dims, str, box, 128)) return;
-  auto kern = flash_attention_tc_kernel<T>;
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FA_SMEM);
-    attr_done = true;
-  }
+  if (!edv::make_tmap_2d(L, &tm, dtype, qkv, 3 * D, (uint64_t)F * S, 3 * D * 2, FA_HD, FA_BM, 128)) return;
+  constexpr auto kern = flash_attention_tc_kernel<T>;
+  edv::smem_opt_in<kern>((int)FA_SMEM);
   const int nx = (S + 2 * FA_BM - 1) / (2 * FA_BM);
   const long long total = (long long)nx * heads * F;
   if (total > 0x7fffffffLL) return L.fail(EDV_ERR_ARG, "flash_attention_tc: too many work items");

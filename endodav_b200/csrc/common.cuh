@@ -307,3 +307,21 @@ namespace tc {
 enum { EF_BIAS = 1, EF_GELU = 2, EF_RELU = 4, EF_RES1_F32 = 8, EF_RES1_T = 16, EF_RES2_T = 32, EF_OUT_F32 = 64, EF_OUT_RELU = 128, EF_ROWBIAS = 256,
        EF_TMA_OUT = 512 /* 16-bit output written through shared memory + TMA store (gt_epilogue_tma) */ };
 }
+// The kinds that get their own instantiation, as X-macro lists: the host (ops.cuh epi_kind, gemm_tc_inst.cuh
+// gemm_tma_out_ok) accepts exactly the kinds that the device switches (gemm_tc.cuh, gemm_bres.cuh) dispatch.
+// Row-segment epilogue (gt_epi_rows); any other epilogue runs its generic F = -1 version.
+#define EDV_EPI_ROW_KINDS(X)                                                                  \
+  X(EF_BIAS)                                                  /* qkv, projects, out_conv, output_conv1 */ \
+  X(EF_BIAS | EF_GELU)                                        /* fc1 */                      \
+  X(EF_BIAS | EF_RES1_F32 | EF_OUT_F32)                       /* attn.proj, fc2, temporal to_out: x += ... */ \
+  X(EF_BIAS | EF_OUT_F32)                                     /* temporal proj_in */         \
+  X(EF_BIAS | EF_RES1_F32)                                    /* temporal ff.net.2 */        \
+  X(EF_BIAS | EF_RES1_T)                                      /* temporal proj_out, RCU conv2 */ \
+  X(EF_BIAS | EF_RES1_T | EF_OUT_RELU)                                                       \
+  X(EF_BIAS | EF_RES1_T | EF_RES2_T)                                                         \
+  X(EF_BIAS | EF_RES1_T | EF_RES2_T | EF_OUT_RELU)                                           \
+  X(EF_BIAS | EF_RELU)                                        /* RCU conv1 */                \
+  X(EF_OUT_RELU)                                              /* layer*_rn */                \
+  X(0)                                                        /* temporal q|k|v (no bias) */
+// TMA-store epilogue (gt_epilogue_tma): 16-bit row-major output with bias / GELU / ReLU only
+#define EDV_EPI_TMA_KINDS(X) X(EF_BIAS) X(EF_BIAS | EF_GELU) X(EF_BIAS | EF_RELU) X(0)

@@ -14,8 +14,8 @@
 //   warp 1       TMEM allocator + MMA issuer (warp-uniform loop, elected lane; two accumulator buffers)
 //   warps 4..19  four epilogue warpgroups, ALL of them on every tile (columns [wg * BN/4, +BN/4)): thread = row,
 //                16-column steps: tcgen05.ld -> bias / GELU / ReLU -> 16-bit -> swizzled shared-memory sub-tile -> TMA
-//                store (gt_epilogue_tma in gemm_tc.cuh; ONE 4 KB staging sub-tile per warpgroup here: shared memory is
-//                full -- 144 KB W + 64 KB A ring + 16 KB staging)
+//                store: gemm_tc's TMA-store epilogue (gt_epilogue_tma) with ONE 4 KB staging sub-tile per warpgroup, as
+//                shared memory is full -- 144 KB W + 64 KB A ring + 16 KB staging
 #pragma once
 #include "gemm_tc.cuh"
 
@@ -26,72 +26,6 @@ constexpr int GB_A_STAGE = GT_BM * 128;   // one 128 x 64 16-bit k-block of A
 constexpr int GB_PF_TILES = 2;            // A tiles prefetched into L2 ahead of the ring
 
 template <int BN> constexpr uint32_t gb_tmem_cols() { return 2 * BN <= 256 ? 256 : 512; }
-
-// One 16-column step at a time through a single staging sub-tile (the store of step s-1 must have read it first).
-template <typename T, int BN, int F>
-__device__ __forceinline__ void gb_epilogue(const CUtensorMap* tmC, uint32_t trow, int row0, int col0, int r, int wg,
-                                            unsigned char* stg_wg, const float* bias_s, uint64_t* tempty) {
-  constexpr int CW = BN / 4;
-  constexpr int NSUB = CW / 16;
-  static_assert(CW % 16 == 0 && NSUB >= 1, "BN must be a multiple of 64");
-  uint32_t raw[2][16];
-  tmem_ld16_nowait(trow, raw[0]);
-  const int sw = (r >> 2) & 1;                                // SWIZZLE_32B: 16-byte chunk index ^= address bit 7
-#pragma unroll
-  for (int s = 0; s < NSUB; ++s) {
-    tmem_ld_wait_all();
-    if (s + 1 < NSUB) tmem_ld16_nowait(trow + 16 * (s + 1), raw[(s + 1) & 1]);
-    float v[16];
-#pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(raw[s & 1][i]);
-    if (F & EF_BIAS) {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const float4 b = *reinterpret_cast<const float4*>(bias_s + 16 * s + 4 * i);   // warp-wide broadcast
-        add2_f32(v[4 * i], v[4 * i + 1], b.x, b.y);
-        add2_f32(v[4 * i + 2], v[4 * i + 3], b.z, b.w);
-      }
-    }
-    if (F & EF_GELU) {
-#pragma unroll
-      for (int i = 0; i < 8; ++i) gelu_poly2(v[2 * i], v[2 * i + 1], v[2 * i], v[2 * i + 1]);
-    }
-    if (F & EF_RELU) {
-#pragma unroll
-      for (int i = 0; i < 16; ++i) v[i] = fmaxf(v[i], 0.f);
-    }
-    uint4 p[2];
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-      p[i].x = pack2(from_f<T>(v[8 * i + 0]), from_f<T>(v[8 * i + 1]));
-      p[i].y = pack2(from_f<T>(v[8 * i + 2]), from_f<T>(v[8 * i + 3]));
-      p[i].z = pack2(from_f<T>(v[8 * i + 4]), from_f<T>(v[8 * i + 5]));
-      p[i].w = pack2(from_f<T>(v[8 * i + 6]), from_f<T>(v[8 * i + 7]));
-    }
-    if (s + 1 == NSUB) {
-      // every tcgen05.ld of this thread has completed: hand the accumulator back before the store bookkeeping
-      fence_before_sync();
-      mbar_arrive(tempty);
-    }
-    if ((r >> 5) == 0) {
-      if (elect_one_sync()) tma_store_wait_read<0>();         // the previous store has read the staging sub-tile
-      __syncwarp();
-    }
-    wg_bar_sync(1 + wg);
-    unsigned char* row = stg_wg + r * 32;
-    *reinterpret_cast<uint4*>(row + ((0 ^ sw) << 4)) = p[0];
-    *reinterpret_cast<uint4*>(row + ((1 ^ sw) << 4)) = p[1];
-    fence_proxy_async();
-    wg_bar_sync(1 + wg);
-    if ((r >> 5) == 0) {
-      if (elect_one_sync()) {
-        tma_store_2d(tmC, stg_wg, col0 + 16 * s, row0);
-        tma_store_commit();
-      }
-      __syncwarp();
-    }
-  }
-}
 
 template <typename T, int BN>
 __global__ void __launch_bounds__(GB_THREADS, 1) gemm_bres_kernel(const __grid_constant__ CUtensorMap tmA,
@@ -187,36 +121,15 @@ __global__ void __launch_bounds__(GB_THREADS, 1) gemm_bres_kernel(const __grid_c
       }
     }
   } else if (warp == 1) {
-    constexpr uint32_t idesc = make_idesc<T>(GT_BM, BN, 0);
     const uint32_t leader = elect_one_sync();
     const uint32_t sa_addr = smem_u32(sA), sb_addr = smem_u32(sB);
+    const auto ab = [&](int s, int kb) { return make_uint2(sa_addr + s * GB_A_STAGE, sb_addr + kb * B_KB_BYTES); };
     mbar_wait(b_full, 0);
     fence_after_sync();
     uint32_t kc = 0, it = 0;
     for (int tm = grp; tm < m_tiles; tm += grp_size, ++it) {
       const uint32_t b = it & 1;
-      mbar_wait(&tempty_bar[b], ((it >> 1) & 1) ^ 1);
-      fence_after_sync();
-      if (tm_ && leader && it < 20) tm_[8 + 4 * it] = clock64();
-      const uint32_t acc = tmem_base + b * BN;
-      for (int kb = 0; kb < kblocks; ++kb, ++kc) {
-        const int s = kc % stages;
-        if (tm_ && leader && it == 4 && kb < 30) tm_[200 + kb] = clock64();   // [200+kb]: before the wait for k-block kb
-        mbar_wait(&full_bar[s], (kc / stages) & 1);
-        fence_after_sync();
-        if (tm_ && leader && it == 4 && kb < 30) tm_[130 + kb] = clock64();
-        const uint64_t adesc = make_smem_desc(sa_addr + s * GB_A_STAGE, 1024, 16, SWZ_128B);
-        const uint64_t bdesc = make_smem_desc(sb_addr + kb * B_KB_BYTES, 1024, 16, SWZ_128B);
-        if (leader) {
-#pragma unroll
-          for (int k = 0; k < 4; ++k) mma_ss(acc, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (kb | k) ? 1u : 0u);
-          mma_commit(&empty_bar[s]);
-        }
-        __syncwarp();
-      }
-      if (leader) mma_commit(&tfull_bar[b]);
-      if (tm_ && leader && it < 20) tm_[9 + 4 * it] = clock64();
-      __syncwarp();
+      mma_tile<T, BN, 64>(leader, tmem_base + b * BN, &tempty_bar[b], &tfull_bar[b], full_bar, empty_bar, stages, kblocks, kc, it, ab, tm_);
     }
   } else if (warp >= 4) {
     const int wg = (warp - 4) >> 2;
@@ -240,10 +153,10 @@ __global__ void __launch_bounds__(GB_THREADS, 1) gemm_bres_kernel(const __grid_c
       const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16) + b * BN + wg * CW;
       const int row0 = tm * GT_BM, col0 = tile_n * BN + wg * CW;
       switch (kind) {
-        case EF_BIAS: gb_epilogue<T, BN, EF_BIAS>(&tmC, trow, row0, col0, r, wg, stg_wg, bias_s, &tempty_bar[b]); break;
-        case EF_BIAS | EF_GELU: gb_epilogue<T, BN, EF_BIAS | EF_GELU>(&tmC, trow, row0, col0, r, wg, stg_wg, bias_s, &tempty_bar[b]); break;
-        case EF_BIAS | EF_RELU: gb_epilogue<T, BN, EF_BIAS | EF_RELU>(&tmC, trow, row0, col0, r, wg, stg_wg, bias_s, &tempty_bar[b]); break;
-        default: gb_epilogue<T, BN, 0>(&tmC, trow, row0, col0, r, wg, stg_wg, bias_s, &tempty_bar[b]); break;
+#define EDV_TMA_CASE(F_) case F_: gt_epilogue_tma<T, BN, F_, 1>(&tmC, trow, row0, col0, r, wg, stg_wg, bias_s, &tempty_bar[b], nullptr); break;
+        EDV_EPI_TMA_KINDS(EDV_TMA_CASE)
+#undef EDV_TMA_CASE
+        default: __builtin_unreachable();   // EF_TMA_OUT is set for these kinds only (gemm_tma_out_ok)
       }
       if (stamp) tm_[11 + 4 * it] = clock64();
     }

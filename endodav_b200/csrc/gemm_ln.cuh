@@ -18,7 +18,8 @@
 //   exchange (sum, M2) of the half row -> peer CTA (st.shared::cluster + remote mbarrier arrive); Chan's
 //           combination gives the full-row mean / variance with two-pass accuracy
 //   pass 3  (x - mean) * rstd * gamma + beta -> 16 bit -> TMA store of xn
-// thread = row, warpgroup wg = columns [48 wg, +48) of the half, 16-column steps (as gemm_tc.cuh's TMA-store epilogue).
+// thread = row, warpgroup wg = columns [48 wg, +48) of the half, 16-column steps; pass 3 stages and stores each step
+// with the steps of gemm_tc.cuh's TMA-store epilogue (pack16, stage_store16).
 //
 //   warp 16 (virtual 0)   TMA producer: A k-block (128 x 64) + this CTA's 192 rows of the W k-block, 3-stage ring,
 //                         A L2-prefetched a few k-blocks ahead
@@ -161,31 +162,17 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GL_THREADS, 1)
       }
     }
   } else if (warp == 1) {
-    constexpr uint32_t idesc = make_idesc<T>(GT_BM, GL_HN, 0);
     const uint32_t leader = elect_one_sync();
     const uint32_t ring_addr = smem_u32(ring);
+    const auto ab = [&](int s, int) {
+      const uint32_t sa = ring_addr + s * GL_STAGE_BYTES;
+      return make_uint2(sa, sa + GL_A_BYTES);
+    };
     uint32_t kc = 0, it = 0;
     for (int tile = pair; tile < m_tiles; tile += npairs, ++it) {
       const uint32_t b = it & 1;
-      mbar_wait(&tempty_bar[b], ((it >> 1) & 1) ^ 1);   // the epilogue has finished with this accumulator
-      fence_after_sync();
-      const uint32_t acc = tmem_base + b * GL_HN;
-      for (int kb = 0; kb < kblocks; ++kb, ++kc) {
-        const int s = kc % GL_STAGES;
-        mbar_wait(&full_bar[s], (kc / GL_STAGES) & 1);
-        fence_after_sync();
-        const uint32_t sa = ring_addr + s * GL_STAGE_BYTES;
-        const uint64_t adesc = make_smem_desc(sa, 1024, 16, SWZ_128B);
-        const uint64_t bdesc = make_smem_desc(sa + GL_A_BYTES, 1024, 16, SWZ_128B);
-        if (leader) {
-#pragma unroll
-          for (int k = 0; k < 4; ++k) mma_ss(acc, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (kb | k) ? 1u : 0u);
-          mma_commit(&empty_bar[s]);
-        }
-        __syncwarp();
-      }
-      if (leader) mma_commit(&tfull_bar[b]);
-      __syncwarp();
+      mma_tile<T, GL_HN, 64>(leader, tmem_base + b * GL_HN, &tempty_bar[b], &tfull_bar[b], full_bar, empty_bar, GL_STAGES, kblocks, kc, it, ab,
+                             nullptr);
     }
   } else if (warp >= 4) {
     // Epilogue, thread = row.  (Direct 128-bit global loads / stores in this row-owner pattern -- 64 contiguous bytes
@@ -199,7 +186,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GL_THREADS, 1)
     unsigned char* xn_wg = xns + wg * GT_OUT_SUB_BYTES;
     uint64_t* rfull = res_full + wg * 2;
     const int sw64 = (r >> 1) & 3;                              // SWIZZLE_64B (fp32 sub-tiles, 64-byte rows)
-    const int sw32 = (r >> 2) & 1;                              // SWIZZLE_32B (16-bit sub-tiles, 32-byte rows)
     const int col_wg = wg * GL_CW;                              // within this CTA's half
     const int gcol_wg = col_half + col_wg;                      // global column
     const uint32_t peer_mail = map_to_cta(mail, rank ^ 1);
@@ -329,37 +315,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GL_THREADS, 1)
           fence_before_sync();
           mbar_arrive(&tempty_bar[b]);                          // last TMEM read of this tile
         }
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+          const int c = col_wg + 16 * s + i;
+          v[i] = (v[i] - mean) * rstd * sgamma[c] + sbeta[c];
+        }
         uint4 p[2];
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          float o[8];
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            const int c = col_wg + 16 * s + 8 * h + i;
-            o[i] = (v[8 * h + i] - mean) * rstd * sgamma[c] + sbeta[c];
-          }
-          p[h].x = pack2(from_f<T>(o[0]), from_f<T>(o[1]));
-          p[h].y = pack2(from_f<T>(o[2]), from_f<T>(o[3]));
-          p[h].z = pack2(from_f<T>(o[4]), from_f<T>(o[5]));
-          p[h].w = pack2(from_f<T>(o[6]), from_f<T>(o[7]));
-        }
-        if (w0) {
-          if (elect_one_sync()) tma_store_wait_read<0>();       // the previous store has read the staging sub-tile
-          __syncwarp();
-        }
-        wg_bar_sync(1 + wg);
-        unsigned char* rowp = xn_wg + r * 32;
-        *reinterpret_cast<uint4*>(rowp + ((0 ^ sw32) << 4)) = p[0];
-        *reinterpret_cast<uint4*>(rowp + ((1 ^ sw32) << 4)) = p[1];
-        fence_proxy_async();
-        wg_bar_sync(1 + wg);
-        if (w0) {
-          if (elect_one_sync()) {
-            tma_store_2d(&tmXn, xn_wg, gcol_wg + 16 * s, row0);
-            tma_store_commit();
-          }
-          __syncwarp();
-        }
+        pack16<T>(v, p);
+        stage_store16(&tmXn, xn_wg, r, wg, p, gcol_wg + 16 * s, row0);
       }
       if (tm_ && it < 8) tm_[8 * it + 6] = clock64();
     }

@@ -278,18 +278,7 @@ __device__ __forceinline__ void gt_epilogue(const Epi& e, uint32_t trow, bool va
     if (BN < 64 && half != 0) return;
     switch (e.kind) {
 #define EDV_EPI_CASE(F_) case F_: gt_epi_rows<T, BN, F_>(e, trow, m32, o32, n0, stg, lane, half, bias_s); break;
-      EDV_EPI_CASE(EF_BIAS)                                              // qkv, projects, out_conv, output_conv1
-      EDV_EPI_CASE(EF_BIAS | EF_GELU)                                    // fc1
-      EDV_EPI_CASE(EF_BIAS | EF_RES1_F32 | EF_OUT_F32)                   // attn.proj, fc2, temporal to_out: x += ...
-      EDV_EPI_CASE(EF_BIAS | EF_OUT_F32)                                 // temporal proj_in
-      EDV_EPI_CASE(EF_BIAS | EF_RES1_F32)                                // temporal ff.net.2
-      EDV_EPI_CASE(EF_BIAS | EF_RES1_T)                                  // temporal proj_out, RCU conv2
-      EDV_EPI_CASE(EF_BIAS | EF_RES1_T | EF_OUT_RELU)
-      EDV_EPI_CASE(EF_BIAS | EF_RES1_T | EF_RES2_T)
-      EDV_EPI_CASE(EF_BIAS | EF_RES1_T | EF_RES2_T | EF_OUT_RELU)
-      EDV_EPI_CASE(EF_BIAS | EF_RELU)                                    // RCU conv1
-      EDV_EPI_CASE(EF_OUT_RELU)                                          // layer*_rn
-      EDV_EPI_CASE(0)                                                    // temporal q|k|v (no bias)
+      EDV_EPI_ROW_KINDS(EDV_EPI_CASE)
 #undef EDV_EPI_CASE
       default: gt_epi_rows<T, BN, -1>(e, trow, m32, o32, n0, stg, lane, half, bias_s); break;
     }
@@ -300,10 +289,10 @@ __device__ __forceinline__ void gt_epilogue(const Epi& e, uint32_t trow, bool va
 // The row-segment epilogue above costs ~6 000 cycles per 128 x 192 tile even with trivial math (in-kernel timeline,
 // tools/gemm_timeline.py: transposition through shared memory, row-index shuffles, 4-row store instructions), which
 // made qkv / fc1 epilogue-bound at 2 x their mainloop.  Here the accumulator stays in the row-owner domain:
-// thread = row, 32 columns per step: tcgen05.ld -> bias / GELU / ReLU -> pack to 16 bit -> four 16-byte shared-memory
-// stores at 64B-swizzled chunk positions (conflict-free) -> one elected thread issues a TMA store of the
-// 128 x 32 sub-tile (coalescing, M-tail clipping and address arithmetic are the TMA unit's job).  Two 8 KB staging
-// buffers per epilogue warpgroup; cp.async.bulk.wait_group.read gates their reuse.
+// thread = row, 16 columns per step: tcgen05.ld -> bias / GELU / ReLU -> pack to 16 bit -> two 16-byte shared-memory
+// stores at 32B-swizzled chunk positions (conflict-free) -> one elected thread issues a TMA store of the
+// 128 x 16 sub-tile (coalescing, M-tail clipping and address arithmetic are the TMA unit's job).  4 KB staging
+// sub-tiles per epilogue warpgroup; cp.async.bulk.wait_group.read gates their reuse.
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, const void* smem_src, int c0, int c1) {
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(reinterpret_cast<uint64_t>(m)),
                "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
@@ -333,25 +322,75 @@ __device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, uint32_t* r) {
 }
 __device__ __forceinline__ void tmem_ld_wait_all() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
+// The staging steps shared by the TMA-store epilogue and gemm_ln.cuh's pass 3.  r = row of the tile = thread of the
+// warpgroup; warp 0 of the warpgroup (r < 32) owns the bulk-store groups, its elected lane issues (warp-uniform branch:
+// no uniformisation loops around UTMASTG).
+template <typename T> __device__ __forceinline__ void pack16(const float* v, uint4* p) {
+#pragma unroll
+  for (int i = 0; i < 2; ++i) {
+    p[i].x = pack2(from_f<T>(v[8 * i + 0]), from_f<T>(v[8 * i + 1]));
+    p[i].y = pack2(from_f<T>(v[8 * i + 2]), from_f<T>(v[8 * i + 3]));
+    p[i].z = pack2(from_f<T>(v[8 * i + 4]), from_f<T>(v[8 * i + 5]));
+    p[i].w = pack2(from_f<T>(v[8 * i + 6]), from_f<T>(v[8 * i + 7]));
+  }
+}
+// this thread's row of a staging sub-tile; SWIZZLE_32B: 16-byte chunk index ^= address bit 7
+__device__ __forceinline__ void stage_row16(unsigned char* sub, int r, const uint4* p) {
+  const int sw = (r >> 2) & 1;
+  unsigned char* row = sub + r * 32;
+  *reinterpret_cast<uint4*>(row + ((0 ^ sw) << 4)) = p[0];
+  *reinterpret_cast<uint4*>(row + ((1 ^ sw) << 4)) = p[1];
+}
+// the stores issued so far have read their staging sub-tiles
+__device__ __forceinline__ void wg_staging_wait(int r) {
+  if ((r >> 5) == 0) {
+    if (elect_one_sync()) tma_store_wait_read<0>();
+    __syncwarp();
+  }
+}
+// TMA store of the NS sub-tiles staged at stg to columns [c0, c0 + 16 NS) of rows [row0, row0 + 128)
+template <int NS> __device__ __forceinline__ void wg_store_staged(const CUtensorMap* tm, unsigned char* stg, int r, int c0, int row0) {
+  if ((r >> 5) == 0) {
+    if (elect_one_sync()) {
+#pragma unroll
+      for (int s = 0; s < NS; ++s) tma_store_2d(tm, stg + s * GT_OUT_SUB_BYTES, c0 + 16 * s, row0);
+      tma_store_commit();
+    }
+    __syncwarp();
+  }
+}
+// one step through a single staging sub-tile: wait for the previous store to have read it, stage, store
+__device__ __forceinline__ void stage_store16(const CUtensorMap* tm, unsigned char* stg, int r, int wg, const uint4* p, int c0, int row0) {
+  wg_staging_wait(r);
+  wg_bar_sync(1 + wg);
+  stage_row16(stg, r, p);
+  fence_proxy_async();
+  wg_bar_sync(1 + wg);
+  wg_store_staged<1>(tm, stg, r, c0, row0);
+}
+
 // All FOUR epilogue warpgroups drain every tile, warpgroup wg columns [wg * BN/4, +BN/4) in 16-column steps
 // (the next tcgen05.ld is in flight while the current step is computed), so the epilogue of tile i takes a quarter
 // of a warpgroup-per-half schedule and runs under the mainloop of tile i+1 (other accumulator buffer).
-// trow: TMEM address of this thread's row at the warpgroup's first column; stg_wg: (BN/64) x 4 KB of staging.
-template <typename T, int BN, int F>
+// trow: TMEM address of this thread's row at the warpgroup's first column; stg_wg: NSTG x 4 KB of staging, either
+//   NSTG = BN/64 (gemm_tc): a sub-tile per step; one wait for the previous tile's stores, one barrier before the first
+//                write, all stores after the last step
+//   NSTG = 1     (gemm_bres, whose shared memory is full): every step waits for the previous step's store and stores
+// stamps (null, or gemm_tc's timeline slots [170..175]): [0] staging free, [1] first sub-tile computed, [2] barrier
+// passed, [3] last sub-tile staged, [4] proxy fence done, [5] all sub-tiles staged
+template <typename T, int BN, int F, int NSTG>
 __device__ __forceinline__ void gt_epilogue_tma(const CUtensorMap* tmC, uint32_t trow, int row0, int col0, int r, int wg,
-                                                unsigned char* stg_wg, const float* bias_s, bool issuer, uint64_t* tempty,
+                                                unsigned char* stg_wg, const float* bias_s, uint64_t* tempty,
                                                 long long* stamps) {
   constexpr int CW = BN / 4;
   constexpr int NSUB = CW / 16;
   static_assert(CW % 16 == 0 && NSUB >= 1, "TMA-store epilogue needs BN to be a multiple of 64");
+  static_assert(NSTG == NSUB || NSTG == 1, "staging: one sub-tile per step, or a single one");
+  constexpr bool ALL = NSTG == NSUB;
   uint32_t raw[2][16];
   tmem_ld16_nowait(trow, raw[0]);
-  if ((r >> 5) == 0) {
-    if (elect_one_sync()) tma_store_wait_read<0>();           // the previous tile's stores have read the staging buffers
-    __syncwarp();
-  }
+  if (ALL) wg_staging_wait(r);                                // the previous tile's stores have read the staging
   if (stamps) stamps[0] = clock64();
-  const int sw = (r >> 2) & 1;                                // SWIZZLE_32B: 16-byte chunk index ^= address bit 7
 #pragma unroll
   for (int s = 0; s < NSUB; ++s) {
     tmem_ld_wait_all();
@@ -376,41 +415,71 @@ __device__ __forceinline__ void gt_epilogue_tma(const CUtensorMap* tmC, uint32_t
       for (int i = 0; i < 16; ++i) v[i] = fmaxf(v[i], 0.f);
     }
     uint4 p[2];
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-      p[i].x = pack2(from_f<T>(v[8 * i + 0]), from_f<T>(v[8 * i + 1]));
-      p[i].y = pack2(from_f<T>(v[8 * i + 2]), from_f<T>(v[8 * i + 3]));
-      p[i].z = pack2(from_f<T>(v[8 * i + 4]), from_f<T>(v[8 * i + 5]));
-      p[i].w = pack2(from_f<T>(v[8 * i + 6]), from_f<T>(v[8 * i + 7]));
+    pack16<T>(v, p);
+    if (ALL) {
+      if (s == 0) {
+        if (stamps) stamps[1] = clock64();
+        wg_bar_sync(1 + wg);                                  // staging free (warp 0 has passed its wait above)
+        if (stamps) stamps[2] = clock64();
+      }
+      stage_row16(stg_wg + s * GT_OUT_SUB_BYTES, r, p);
     }
-    if (s == 0) {
-      if (stamps) stamps[1] = clock64();
-      wg_bar_sync(1 + wg);                                    // staging free (the issuer has passed its wait above)
-      if (stamps) stamps[2] = clock64();
-    }
-    unsigned char* row = stg_wg + s * GT_OUT_SUB_BYTES + r * 32;
-    *reinterpret_cast<uint4*>(row + ((0 ^ sw) << 4)) = p[0];
-    *reinterpret_cast<uint4*>(row + ((1 ^ sw) << 4)) = p[1];
     if (s + 1 == NSUB) {
-      // every tcgen05.ld of this thread has completed: hand the accumulator back before the store bookkeeping
+      // every tcgen05.ld of this thread has completed: hand the accumulator back before the stores
       fence_before_sync();
       mbar_arrive(tempty);
     }
+    if (!ALL) stage_store16(tmC, stg_wg, r, wg, p, col0 + 16 * s, row0);
   }
-  if (stamps) stamps[3] = clock64();
-  fence_proxy_async();
-  if (stamps) stamps[4] = clock64();
-  wg_bar_sync(1 + wg);
-  if (stamps) stamps[5] = clock64();
-  if ((r >> 5) == 0) {
-    // warp-uniform branch (warp 0 of the warpgroup), elected lane issues: no uniformisation loops around UTMASTG
-    if (elect_one_sync()) {
+  if (ALL) {
+    if (stamps) stamps[3] = clock64();
+    fence_proxy_async();
+    if (stamps) stamps[4] = clock64();
+    wg_bar_sync(1 + wg);
+    if (stamps) stamps[5] = clock64();
+    wg_store_staged<NSUB>(tmC, stg_wg, r, col0, row0);
+  }
+}
+
+// MMA issuer of one tile: all 32 lanes of warp 1 wait on the barriers and build the descriptors, the elected `leader`
+// issues tcgen05.mma / tcgen05.commit (see elect_one_sync in tc_common.cuh).  Waits for the epilogue to have drained
+// accumulator `acc` (tempty), then per k-block waits for its ring stage, issues BK/16 MMAs (M = 128, N) and releases
+// the stage (empty_bar) once they have read it; finally hands the accumulator to the epilogue (tfull).  ab(s, kb)
+// returns the shared-memory addresses of the A and B tiles of k-block kb (ring stage s).  kc counts the k-blocks of
+// the whole kernel (ring position); it counts the tiles of this CTA.  tm_: optional timeline (slot table of
+// gemm_tc_kernel).
+template <typename T, int N, int BK, typename AB>
+__device__ __forceinline__ void mma_tile(uint32_t leader, uint32_t acc, uint64_t* tempty, uint64_t* tfull, uint64_t* full_bar,
+                                         uint64_t* empty_bar, int stages, int kblocks, uint32_t& kc, uint32_t it, AB ab,
+                                         long long* tm_) {
+  constexpr uint32_t idesc = make_idesc<T>(GT_BM, N, 0);
+  constexpr uint32_t SBO = 8 * BK * 2;                      // 8-row swizzle atom of BK * 2-byte rows
+  constexpr uint32_t SWZ = (BK == 64) ? SWZ_128B : SWZ_64B;
+  mbar_wait(tempty, ((it >> 1) & 1) ^ 1);
+  fence_after_sync();
+  if (tm_ && leader && it < 20) tm_[8 + 4 * it] = clock64();
+  for (int kb = 0; kb < kblocks; ++kb, ++kc) {
+    const int s = kc % stages;
+    if (tm_ && leader && it == 4 && kb < 30) tm_[200 + kb] = clock64();   // [200+kb]: before the wait for k-block kb
+    mbar_wait(&full_bar[s], (kc / stages) & 1);
+    fence_after_sync();
+    if (tm_ && leader && it == 4 && kb < 30) tm_[130 + kb] = clock64();
+    const uint2 op = ab(s, kb);
+    const uint64_t adesc = make_smem_desc(op.x, SBO, 16, SWZ);
+    const uint64_t bdesc = make_smem_desc(op.y, SBO, 16, SWZ);
+    if (leader) {
 #pragma unroll
-      for (int s = 0; s < NSUB; ++s) tma_store_2d(tmC, stg_wg + s * GT_OUT_SUB_BYTES, col0 + 16 * s, row0);
-      tma_store_commit();
+      for (int k = 0; k < BK / 16; ++k) {
+        // advance 16 elements (32 bytes) along K inside the swizzle atom: +2 in the >>4 address field
+        mma_ss(acc, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (kb | k) ? 1u : 0u);
+      }
+      mma_commit(&empty_bar[s]);  // stage reusable once these MMAs have read it
     }
     __syncwarp();
   }
+  if (leader) mma_commit(tfull);    // accumulator complete
+  if (tm_ && leader && it < 20) tm_[9 + 4 * it] = clock64();
+  __syncwarp();
 }
 
 template <typename T, int BN, int BK, bool CONV>
@@ -421,8 +490,6 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gemm_tc_kernel(const __grid_con
                                                                 int total_tiles) {
   pdl_launch();   // PDL: the next kernel of the stream may start its prologue (common.cuh)
   constexpr uint32_t ROW_BYTES = BK * 2;                    // 128 (BK=64) or 64 (BK=32)
-  constexpr uint32_t SWZ = (BK == 64) ? SWZ_128B : SWZ_64B;
-  constexpr uint32_t SBO = 8 * ROW_BYTES;                   // 8-row swizzle atom
   constexpr uint32_t A_BYTES = GT_BM * ROW_BYTES;
   constexpr uint32_t B_BYTES = BN * ROW_BYTES;
   constexpr uint32_t STAGE_BYTES = A_BYTES + B_BYTES;
@@ -513,39 +580,15 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gemm_tc_kernel(const __grid_con
       }
     }
   } else if (warp == 1) {
-    // warp-uniform issue loop: all 32 lanes wait on the barriers and build the descriptors, the elected lane
-    // issues tcgen05.mma / tcgen05.commit (see elect_one_sync in tc_common.cuh)
-    constexpr uint32_t idesc = make_idesc<T>(GT_BM, BN, 0);
     const uint32_t leader = elect_one_sync();
+    const auto ab = [&](int s, int) {
+      const uint32_t sa = smem_u32(smem + (size_t)s * STAGE_BYTES);
+      return make_uint2(sa, sa + A_BYTES);
+    };
     uint32_t kc = 0, it = 0;
     for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++it) {
       const uint32_t b = it & 1;
-      mbar_wait(&tempty_bar[b], ((it >> 1) & 1) ^ 1);   // epilogue has drained this accumulator
-      fence_after_sync();
-      if (tm_ && leader && it < 20) tm_[8 + 4 * it] = clock64();
-      const uint32_t acc = tmem_base + b * BN;
-      for (int kb = 0; kb < kblocks; ++kb, ++kc) {
-        const int s = kc % stages;
-        if (tm_ && leader && it == 4 && kb < 30) tm_[200 + kb] = clock64();   // [200+kb]: before the wait for k-block kb
-        mbar_wait(&full_bar[s], (kc / stages) & 1);
-        fence_after_sync();
-        if (tm_ && leader && it == 4 && kb < 30) tm_[130 + kb] = clock64();
-        const uint32_t sa = smem_u32(smem + (size_t)s * STAGE_BYTES);
-        const uint64_t adesc = make_smem_desc(sa, SBO, 16, SWZ);
-        const uint64_t bdesc = make_smem_desc(sa + A_BYTES, SBO, 16, SWZ);
-        if (leader) {
-#pragma unroll
-          for (int k = 0; k < BK / 16; ++k) {
-            // advance 16 elements (32 bytes) along K inside the swizzle atom: +2 in the >>4 address field
-            mma_ss(acc, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (kb | k) ? 1u : 0u);
-          }
-          mma_commit(&empty_bar[s]);  // stage reusable once these MMAs have read it
-        }
-        __syncwarp();
-      }
-      if (leader) mma_commit(&tfull_bar[b]);    // accumulator complete
-      if (tm_ && leader && it < 20) tm_[9 + 4 * it] = clock64();
-      __syncwarp();
+      mma_tile<T, BN, BK>(leader, tmem_base + b * BN, &tempty_bar[b], &tfull_bar[b], full_bar, empty_bar, stages, kblocks, kc, it, ab, tm_);
     }
   } else if (warp >= 4) {
     // epilogue warpgroups 0..3: accumulator buffer g = wg & 1, column half = wg >> 1;
@@ -562,7 +605,6 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gemm_tc_kernel(const __grid_con
         // ---- TMA-store mode: warpgroup wg drains columns [wg * BN/4, +BN/4) of EVERY tile ----
         constexpr int CW = BN / 4;
         unsigned char* stg_wg = reinterpret_cast<unsigned char*>(stg_base) + wg * ((CW / 16) * GT_OUT_SUB_BYTES);
-        const bool issuer = (q == 0 && lane == 0);
         float* bias_s = bias_base + (warp - 4) * 128;
         const int kind = e.kind & ~EF_TMA_OUT;
         for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++it) {
@@ -582,10 +624,10 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gemm_tc_kernel(const __grid_con
           const int row0 = tile_m * GT_BM, col0 = tile_n * BN + wg * CW;
           long long* st = (stamp && it == 5) ? tm_ + 170 : nullptr;   // [170..175]: phases of tile 5 (see gt_epilogue_tma)
           switch (kind) {
-            case EF_BIAS: gt_epilogue_tma<T, BN, EF_BIAS>(&tmC, trow, row0, col0, r, wg, stg_wg, bias_s, issuer, &tempty_bar[b], st); break;
-            case EF_BIAS | EF_GELU: gt_epilogue_tma<T, BN, EF_BIAS | EF_GELU>(&tmC, trow, row0, col0, r, wg, stg_wg, bias_s, issuer, &tempty_bar[b], st); break;
-            case EF_BIAS | EF_RELU: gt_epilogue_tma<T, BN, EF_BIAS | EF_RELU>(&tmC, trow, row0, col0, r, wg, stg_wg, bias_s, issuer, &tempty_bar[b], st); break;
-            default: gt_epilogue_tma<T, BN, 0>(&tmC, trow, row0, col0, r, wg, stg_wg, bias_s, issuer, &tempty_bar[b], st); break;
+#define EDV_TMA_CASE(F_) case F_: gt_epilogue_tma<T, BN, F_, BN / 64>(&tmC, trow, row0, col0, r, wg, stg_wg, bias_s, &tempty_bar[b], st); break;
+            EDV_EPI_TMA_KINDS(EDV_TMA_CASE)
+#undef EDV_TMA_CASE
+            default: __builtin_unreachable();   // EF_TMA_OUT is set for these kinds only (gemm_tma_out_ok)
           }
           if (stamp) tm_[11 + 4 * it] = clock64();
         }

@@ -9,12 +9,16 @@
 
 namespace edv {
 
-// the TMA-store epilogue handles 16-bit row-major outputs with bias / GELU / ReLU only
+// the TMA-store epilogue handles 16-bit row-major outputs of the EDV_EPI_TMA_KINDS only
 inline bool gemm_tma_out_ok(const GemmArgs& a) {
   using namespace tc;
-  const int k = a.e.kind;
-  if (a.conv || k < 0) return false;
-  if (k != 0 && k != EF_BIAS && k != (EF_BIAS | EF_GELU) && k != (EF_BIAS | EF_RELU)) return false;
+  if (a.conv) return false;
+  switch (a.e.kind) {
+#define EDV_KIND_LABEL(F_) case F_:
+    EDV_EPI_TMA_KINDS(EDV_KIND_LABEL) break;
+#undef EDV_KIND_LABEL
+    default: return false;
+  }
   if (a.e.map != MAP_LINEAR || a.e.out_f32 || !a.e.out) return false;
   if ((a.e.ldo * 2) % 16 != 0 || ((uintptr_t)a.e.out & 15) != 0) return false;
   return true;
@@ -39,26 +43,15 @@ void launch_gemm_tc_inst(Launch& L, int dtype, const GemmArgs& a) {
     if (!make_tmap(L, &tmA, dtype, a.A, 4, dims, str, box, swz)) return;
   } else {
     m_tiles = (a.M + GT_BM - 1) / GT_BM;
-    uint64_t dims[2] = {(uint64_t)a.K, (uint64_t)a.M};
-    uint64_t str[1] = {(uint64_t)a.lda * 2};
-    uint32_t box[2] = {(uint32_t)BK, (uint32_t)GT_BM};
-    if (!make_tmap(L, &tmA, dtype, a.A, 2, dims, str, box, swz)) return;
+    if (!make_tmap_2d(L, &tmA, dtype, a.A, a.K, a.M, a.lda * 2, BK, GT_BM, swz)) return;
   }
-  {
-    uint64_t dims[2] = {(uint64_t)a.K, (uint64_t)a.N};
-    uint64_t str[1] = {(uint64_t)a.K * 2};
-    uint32_t box[2] = {(uint32_t)BK, (uint32_t)BN};
-    if (!make_tmap(L, &tmB, dtype, a.W, 2, dims, str, box, swz)) return;
-  }
+  if (!make_tmap_2d(L, &tmB, dtype, a.W, a.K, a.N, a.K * 2, BK, BN, swz)) return;
   // TMA-store epilogue: output tensor map over C [M rows, N cols] (row pitch ldo), box 16 columns x 128 rows, 32B swizzle
   CUtensorMap tmC;
   memset(&tmC, 0, sizeof tmC);
   GemmArgs a2 = a;
   if (!CONV && BN % 64 == 0 && gemm_tma_out_ok(a)) {
-    uint64_t dims[2] = {(uint64_t)a.N, (uint64_t)a.M};
-    uint64_t str[1] = {(uint64_t)a.e.ldo * 2};
-    uint32_t box[2] = {16u, (uint32_t)GT_BM};
-    if (!make_tmap(L, &tmC, dtype, a.e.out, 2, dims, str, box, 32)) return;
+    if (!make_tmap_2d(L, &tmC, dtype, a.e.out, a.N, a.M, a.e.ldo * 2, 16, GT_BM, 32)) return;
     a2.e.kind |= tc::EF_TMA_OUT;
   }
   const int kblocks = a.K / BK;
@@ -68,12 +61,8 @@ void launch_gemm_tc_inst(Launch& L, int dtype, const GemmArgs& a) {
   if (stages > 8) stages = 8;
   if (stages < 2) stages = 2;
   const size_t smem = (size_t)stages * stage_bytes + 1024 /*align*/ + (2 * stages + 4) * 8 + 16 + stg_bytes;
-  auto kern = gemm_tc_kernel<T, BN, BK, CONV>;
-  static bool attr_done = false;  // per instantiation
-  if (!attr_done) {
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024);
-    attr_done = true;
-  }
+  constexpr auto kern = gemm_tc_kernel<T, BN, BK, CONV>;
+  smem_opt_in<kern>(226 * 1024);
   const int n_tiles = a.N / BN;
   const long long total = m_tiles * n_tiles;
   if (total > 0x7fffffffLL) return L.fail(EDV_ERR_ARG, "gemm_tc: too many tiles");
@@ -87,12 +76,8 @@ void launch_gemm_tc_inst(Launch& L, int dtype, const GemmArgs& a) {
 // 64-channel 3x3 convs with halo reuse (conv_halo.cuh)
 template <typename T, int BN> void launch_conv_halo(Launch& L, const GemmArgs& a) {
   using namespace tc;
-  auto kern = conv3x3_halo_kernel<T, 64, BN>;
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ch_smem_bytes<64, BN>());
-    attr_done = true;
-  }
+  constexpr auto kern = conv3x3_halo_kernel<T, 64, BN>;
+  smem_opt_in<kern>((int)ch_smem_bytes<64, BN>());
   const int tiles_x = (a.Wd + CH_TW - 1) / CH_TW, tiles_y = (a.H + CH_TH - 1) / CH_TH;
   const long long total = (long long)a.F * tiles_x * tiles_y;
   if (total > 0x7fffffffLL) return L.fail(EDV_ERR_ARG, "conv_halo: too many tiles");
@@ -155,30 +140,11 @@ template <typename T, int BN> bool launch_gemm_bres(Launch& L, int dtype, const 
   int stages = (int)((GB_SMEM_MAX - fixed) / GB_A_STAGE);
   if (stages > 8) stages = 8;
   CUtensorMap tmA, tmB, tmC;
-  {
-    uint64_t dims[2] = {(uint64_t)a.K, (uint64_t)a.M};
-    uint64_t str[1] = {(uint64_t)a.lda * 2};
-    uint32_t box[2] = {64u, (uint32_t)GT_BM};
-    if (!make_tmap(L, &tmA, dtype, a.A, 2, dims, str, box, 128)) return true;
-  }
-  {
-    uint64_t dims[2] = {(uint64_t)a.K, (uint64_t)a.N};
-    uint64_t str[1] = {(uint64_t)a.K * 2};
-    uint32_t box[2] = {64u, (uint32_t)BN};
-    if (!make_tmap(L, &tmB, dtype, a.W, 2, dims, str, box, 128)) return true;
-  }
-  {
-    uint64_t dims[2] = {(uint64_t)a.N, (uint64_t)a.M};
-    uint64_t str[1] = {(uint64_t)a.e.ldo * 2};
-    uint32_t box[2] = {16u, (uint32_t)GT_BM};
-    if (!make_tmap(L, &tmC, dtype, a.e.out, 2, dims, str, box, 32)) return true;
-  }
-  auto kern = gemm_bres_kernel<T, BN>;
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    attr_done = true;
-  }
+  if (!make_tmap_2d(L, &tmA, dtype, a.A, a.K, a.M, a.lda * 2, 64, GT_BM, 128)) return true;
+  if (!make_tmap_2d(L, &tmB, dtype, a.W, a.K, a.N, a.K * 2, 64, BN, 128)) return true;
+  if (!make_tmap_2d(L, &tmC, dtype, a.e.out, a.N, a.M, a.e.ldo * 2, 16, GT_BM, 32)) return true;
+  constexpr auto kern = gemm_bres_kernel<T, BN>;
+  smem_opt_in<kern>(232448);
   const int n_tiles = a.N / BN;
   const int m_tiles = (a.M + GT_BM - 1) / GT_BM;
   int grid = num_sms();
@@ -198,36 +164,12 @@ void launch_gemm_ln(Launch& L, int dtype, const void* A, const void* W, const fl
                     const float* beta, float eps, int M, int K, int do_ln, long long* tim) {
   using namespace tc;
   CUtensorMap tmA, tmB, tmX, tmXn;
-  {
-    uint64_t dims[2] = {(uint64_t)K, (uint64_t)M};
-    uint64_t str[1] = {(uint64_t)K * 2};
-    uint32_t box[2] = {64u, (uint32_t)GT_BM};
-    if (!make_tmap(L, &tmA, dtype, A, 2, dims, str, box, 128)) return;
-  }
-  {
-    uint64_t dims[2] = {(uint64_t)K, (uint64_t)GL_N};
-    uint64_t str[1] = {(uint64_t)K * 2};
-    uint32_t box[2] = {64u, (uint32_t)GL_HN};
-    if (!make_tmap(L, &tmB, dtype, W, 2, dims, str, box, 128)) return;
-  }
-  {
-    uint64_t dims[2] = {(uint64_t)GL_N, (uint64_t)M};
-    uint64_t str[1] = {(uint64_t)GL_N * 4};
-    uint32_t box[2] = {16u, (uint32_t)GT_BM};
-    if (!make_tmap(L, &tmX, EDV_F32, x, 2, dims, str, box, 64)) return;
-  }
-  {
-    uint64_t dims[2] = {(uint64_t)GL_N, (uint64_t)M};
-    uint64_t str[1] = {(uint64_t)GL_N * 2};
-    uint32_t box[2] = {16u, (uint32_t)GT_BM};
-    if (!make_tmap(L, &tmXn, dtype, do_ln ? xn : (const void*)x, 2, dims, str, box, 32)) return;
-  }
-  auto kern = gemm_ln_kernel<T>;
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GL_SMEM);
-    attr_done = true;
-  }
+  if (!make_tmap_2d(L, &tmA, dtype, A, K, M, K * 2, 64, GT_BM, 128)) return;
+  if (!make_tmap_2d(L, &tmB, dtype, W, K, GL_N, K * 2, 64, GL_HN, 128)) return;
+  if (!make_tmap_2d(L, &tmX, EDV_F32, x, GL_N, M, GL_N * 4, 16, GT_BM, 64)) return;
+  if (!make_tmap_2d(L, &tmXn, dtype, do_ln ? xn : (const void*)x, GL_N, M, GL_N * 2, 16, GT_BM, 32)) return;
+  constexpr auto kern = gemm_ln_kernel<T>;
+  smem_opt_in<kern>((int)GL_SMEM);
   const int m_tiles = (M + GT_BM - 1) / GT_BM;
   const int grid = 2 * std::min(m_tiles, num_sms() / 2);   // clusters of two CTAs, one 128-row tile per pair at a time
   // algorithmic work: 2 M N K; bytes: A + W + the fp32 stream read and written once + xn written once

@@ -9,12 +9,8 @@ template <typename T, int CIN>
 void launch_head_fused(Launch& L, const void* x, const void* w, const float* bias, const float* head_w, float* out, int F,
                        int H1, int W1, int OH, int OW, float sig_sign) {
   using namespace tc;
-  auto kern = head_fused_kernel<T, CIN>;
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hf_smem_bytes<CIN>());
-    attr_done = true;
-  }
+  constexpr auto kern = head_fused_kernel<T, CIN>;
+  smem_opt_in<kern>((int)hf_smem_bytes<CIN>());
   const int tiles_x = (OW + HF_TW - 1) / HF_TW, tiles_y = (OH + HF_TH - 1) / HF_TH;
   const long long total = (long long)F * tiles_x * tiles_y;
   if (total > 0x7fffffffLL) return L.fail(EDV_ERR_ARG, "head_fused: too many tiles");

@@ -35,6 +35,17 @@ inline void launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem,
   cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
 }
 
+// Allows kernel Kern up to `bytes` of dynamic shared memory; sets the attribute on the first call only, so eager
+// forwards pay no host time for it.  The kernel itself is the template argument: a flag in a helper templated on the
+// kernel's signature would be shared by all instances of a kernel template (e.g. every gemm_tc_kernel<T, BN, BK, CONV>).
+template <auto Kern> inline void smem_opt_in(int bytes) {
+  static bool done = false;
+  if (!done) {
+    cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    done = true;
+  }
+}
+
 // Optional per-launch timing: one CUDA event after every launch on the launching stream, so
 // the duration of launch i is event[i] - event[i-1] (the stream is serial).  Used by bench.py
 // for the live roofline numbers; off by default (no events are recorded).

@@ -35,12 +35,12 @@ inline int epi_kind(const Epi& e) {
   if (e.res2) f |= EF_RES2_T;
   if (e.out_f32) f |= EF_OUT_F32;
   if (e.out_relu) f |= EF_OUT_RELU;
-  const int known[] = {EF_BIAS, EF_BIAS | EF_GELU, EF_BIAS | EF_RES1_F32 | EF_OUT_F32, EF_BIAS | EF_OUT_F32, EF_BIAS | EF_RES1_F32,
-                       EF_BIAS | EF_RES1_T, EF_BIAS | EF_RES1_T | EF_OUT_RELU, EF_BIAS | EF_RES1_T | EF_RES2_T,
-                       EF_BIAS | EF_RES1_T | EF_RES2_T | EF_OUT_RELU, EF_BIAS | EF_RELU, EF_OUT_RELU, 0};
-  for (int k : known)
-    if (k == f) return f;
-  return -1;
+  switch (f) {
+#define EDV_KIND_LABEL(F_) case F_:
+    EDV_EPI_ROW_KINDS(EDV_KIND_LABEL) return f;
+#undef EDV_KIND_LABEL
+    default: return -1;
+  }
 }
 
 // dispatch on dtype / engine.  GEGLU and HEAD epilogues exist only in the tcgen05 kernel;

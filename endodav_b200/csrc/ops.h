@@ -73,6 +73,13 @@ inline bool make_tmap(Launch& L, CUtensorMap* m, int dtype, const void* base, in
   }
   return true;
 }
+// 2-D map over a row-major [outer][inner] tensor whose rows are pitch_bytes apart
+inline bool make_tmap_2d(Launch& L, CUtensorMap* m, int dtype, const void* base, uint64_t inner, uint64_t outer, uint64_t pitch_bytes,
+                         uint32_t box_inner, uint32_t box_outer, int swizzle_bytes) {
+  const uint64_t dims[2] = {inner, outer};
+  const uint32_t box[2] = {box_inner, box_outer};
+  return make_tmap(L, m, dtype, base, 2, dims, &pitch_bytes, box, swizzle_bytes);
+}
 
 // ---- GEMM -----------------------------------------------------------------------------------
 struct GemmArgs {

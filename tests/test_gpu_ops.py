@@ -55,12 +55,12 @@ def test_linear_fp32(M, N, K, act):
 @pytest.mark.parametrize("dtype", DT16)
 @pytest.mark.parametrize("engine", [eng.ENGINE_TC, eng.ENGINE_SIMT])
 @pytest.mark.parametrize("M,N,K", LIN_SHAPES)
-@pytest.mark.parametrize("act", [0, 1])
+@pytest.mark.parametrize("act", [0, 1, 2])
 def test_linear_16bit(dtype, engine, M, N, K, act):
     A, W, b = _rand((M, K), dtype, 1), _rand((N, K), dtype, 2, K ** -0.5), _rand((N,), torch.float32, 3)
     got = eng.op_linear(A, W, b, act, engine)
     ref = F.linear(A.double(), W.double(), b.double())
-    ref = F.gelu(ref) if act == 1 else ref
+    ref = F.gelu(ref) if act == 1 else F.relu(ref) if act == 2 else ref
     _close(got, ref.float(), dtype, "linear %s engine %d" % (dtype, engine))
 
 
