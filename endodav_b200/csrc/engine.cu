@@ -1201,16 +1201,54 @@ static int finish(Launch& L) {
   return L.status;
 }
 
-int edv_op_linear(int dtype, int engine, const void* A, const void* W, const float* bias, void* C, int M, int N, int K,
-                  int act, void* stream) {
+// One GEMM / conv with a caller-described epilogue through gemm(), the forward's own kernel selection; `kernel` receives
+// the instance that ran.
+int edv_op_gemm(int dtype, int engine, const edv_gemm_desc* d, char* kernel, int kernel_cap, void* stream) {
+  if (kernel && kernel_cap > 0) kernel[0] = 0;
+  if (!d || d->struct_bytes != (int)sizeof(edv_gemm_desc))
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_gemm: struct_bytes %d, library's edv_gemm_desc has %d", d ? d->struct_bytes : -1,
+                   (int)sizeof(edv_gemm_desc));
+  if (dtype < EDV_F32 || dtype > EDV_F16) return set_err(nullptr, EDV_ERR_ARG, "edv_op_gemm: bad dtype %d", dtype);
+  const bool tc = dtype != EDV_F32 && engine == EDV_ENGINE_TC;
+  // GEGLU and the disparity head exist only in the tcgen05 epilogue: the CUDA-core forward composes them from a plain GEMM
+  // plus geglu_pair_kernel / head_dot_kernel, and epi_apply would silently ignore them
+  if (!tc && (d->act == ACT_GEGLU || d->act == ACT_HEAD))
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_gemm: act %d needs the tensor-core engine", d->act);
+  if (d->act < ACT_NONE || d->act > ACT_SIGMOID || d->map < MAP_LINEAR || d->map > MAP_PIXSHUF)
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_gemm: bad act %d / map %d", d->act, d->map);
+  if (!d->out || !d->A || !d->W) return set_err(nullptr, EDV_ERR_ARG, "edv_op_gemm: null A, W or out");
+  if (d->M < 1 || d->N < 1 || d->K < 1) return set_err(nullptr, EDV_ERR_ARG, "edv_op_gemm: empty problem");
+  if (d->conv) {
+    if (d->stride != 1 && (tc || d->stride != 2)) return set_err(nullptr, EDV_ERR_ARG, "edv_op_gemm: conv stride %d", d->stride);
+    if (d->F < 1 || d->H < 1 || d->Wd < 1 || d->C < 1 || d->K != 9 * d->C ||
+        (long long)d->M != (long long)d->F * ((d->H - 1) / d->stride + 1) * ((d->Wd - 1) / d->stride + 1))
+      return set_err(nullptr, EDV_ERR_ARG, "edv_op_gemm: conv needs K = 9*C and M = F*OH*OW");
+  } else if (d->lda < d->K) {
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_gemm: lda < K");
+  }
+  // the vector-alignment contract of load_vec / store_vec (common.cuh): leading dimensions are multiples of 8 elements
+  // (the head epilogue writes one float per row and has no output pitch)
+  if ((!d->conv && d->lda % 8) || (d->act != ACT_HEAD && d->ldo % 8) || (d->res1 && d->ld_res1 % 8) || (d->res2 && d->ld_res2 % 8) ||
+      (d->rowbias && d->rb_ld % 8))
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_gemm: leading dimensions must be multiples of 8");
   Launch L;
   L.stream = (cudaStream_t)stream;
   GemmArgs a;
-  a.A = A; a.W = W; a.M = M; a.N = N; a.K = K; a.lda = K;
-  a.e = epi_zero();
-  a.e.out = C; a.e.ldo = N; a.e.bias = bias; a.e.act = act;
-  if (act != ACT_NONE && act != ACT_GELU && act != ACT_RELU) return EDV_ERR_ARG;
+  a.A = d->A; a.W = d->W; a.M = d->M; a.N = d->N; a.K = d->K; a.lda = d->lda;
+  a.conv = d->conv != 0; a.F = d->F; a.H = d->H; a.Wd = d->Wd; a.C = d->C; a.stride = d->stride;
+  Epi& e = a.e;
+  e = epi_zero();
+  e.out = d->out; e.out_relu = d->out_relu; e.bias = d->bias; e.rowbias = d->rowbias;
+  e.res1 = d->res1; e.res2 = d->res2; e.head_w = d->head_w;
+  e.ldo = d->ldo; e.ld_res1 = d->ld_res1; e.ld_res2 = d->ld_res2; e.rb_ld = d->rb_ld;
+  e.rb_div = d->rb_div; e.rb_mod = d->rb_mod;
+  e.out_f32 = d->out_f32; e.res1_f32 = d->res1_f32; e.res2_f32 = d->res2_f32;
+  e.act = d->act; e.map = d->map; e.map_p = d->map_p;
+  e.ps_k = d->ps_k; e.ps_h = d->ps_h; e.ps_w = d->ps_w; e.ps_c = d->ps_c;
+  e.head_b = 0.f;   // the head's 1x1 bias is head_w[32], as in the forward
+  e.sig_sign = d->sig_sign;
   gemm(L, dtype, engine, a);
+  if (kernel && kernel_cap > 0) snprintf(kernel, kernel_cap, "%s", L.kernel.c_str());
   return finish(L);
 }
 
@@ -1239,19 +1277,6 @@ int edv_op_linear_residual_ln(int dtype, const void* A, const void* W, const flo
   const int do_ln = (gamma && beta && xn_out) ? 1 : 0;
   if (timeline_dev && cudaMemsetAsync(timeline_dev, 0, 64 * sizeof(long long), L.stream) != cudaSuccess) return EDV_ERR_CUDA;
   gemm_ln(L, dtype, A, W, bias, x_inout, xn_out, gamma, beta, eps, M, N, K, do_ln, timeline_dev);
-  return finish(L);
-}
-
-int edv_op_conv3x3(int dtype, int engine, const void* X, const void* Wt, const float* bias, void* Y, int F, int H,
-                   int W, int Cin, int Cout, int relu_out, void* stream) {
-  Launch L;
-  L.stream = (cudaStream_t)stream;
-  GemmArgs a;
-  a.A = X; a.W = Wt; a.M = F * H * W; a.N = Cout; a.K = 9 * Cin;
-  a.e = epi_zero();
-  a.e.out = Y; a.e.ldo = Cout; a.e.bias = bias; a.e.act = relu_out ? ACT_RELU : ACT_NONE;
-  a.conv = true; a.F = F; a.H = H; a.Wd = W; a.C = Cin; a.stride = 1;
-  gemm(L, dtype, engine, a);
   return finish(L);
 }
 

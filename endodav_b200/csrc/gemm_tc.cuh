@@ -658,9 +658,11 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gemm_tc_kernel(const __grid_con
         valid = m < M;
         orow = epi_row(e, m);
       }
-      // stage this warp's bias slice (columns [half*BN/2, +BN/2) of the tile) while the mainloop runs
+      // stage this warp's bias slice (columns [half*BN/2, +BN/2) of the tile) while the mainloop runs.  At BN = 32
+      // warpgroup half 0 drains all columns and half 1 returns without them: staging there would read bias[N, N + 32)
+      // on the last n-tile.
       float* bias_s = nullptr;
-      if (e.bias && e.act != ACT_GEGLU && e.act != ACT_HEAD) {
+      if (e.bias && e.act != ACT_GEGLU && e.act != ACT_HEAD && (BN >= 64 || half == 0)) {
         constexpr int CH0 = (BN >= 64) ? BN / 2 : BN;
         bias_s = bias_base + (warp - 4) * 128;
         __syncwarp();

@@ -69,6 +69,8 @@ void launch_gemm_tc_inst(Launch& L, int dtype, const GemmArgs& a) {
   const int grid = (int)std::min<long long>(total, num_sms());
   (void)kblocks;
   note_gemm(L, a, 2);
+  L.kernel = std::string(CONV ? "gemm_tc_conv<" : "gemm_tc<") + "BN=" + std::to_string(BN) + ",BK=" + std::to_string(BK) + ",kind=" +
+             kind_label(a.e.kind) + (CONV ? ">" : (a2.e.kind != a.e.kind ? ",tma=1>" : ",tma=0>"));
   edv::launch_k(kern, dim3(grid), dim3(GT_THREADS), smem, L.stream, tmA, tmB, tmC, a2.e, a.M, a.N, a.K, stages, ct, n_tiles, (int)total);
   L.check("gemm_tc");
 }
@@ -83,6 +85,7 @@ template <typename T, int BN> void launch_conv_halo(Launch& L, const GemmArgs& a
   if (total > 0x7fffffffLL) return L.fail(EDV_ERR_ARG, "conv_halo: too many tiles");
   const int grid = (int)std::min<long long>(total, num_sms());
   note_gemm(L, a, 2);
+  L.kernel = "conv_halo<BN=" + std::to_string(BN) + ",kind=" + kind_label(a.e.kind) + ">";
   edv::launch_k(kern, dim3(grid), dim3(CH_THREADS), ch_smem_bytes<64, BN>(), L.stream, (const T*)a.A, (const T*)a.W, a.e, a.F, a.H, a.Wd, tiles_x,
                                                                tiles_y, (int)total);
   L.check("conv_halo");
@@ -154,6 +157,7 @@ template <typename T, int BN> bool launch_gemm_bres(Launch& L, int dtype, const 
   GemmArgs a2 = a;
   a2.e.kind |= EF_TMA_OUT;
   note_gemm(L, a, 2);
+  L.kernel = "gemm_bres<BN=" + std::to_string(BN) + ">";
   edv::launch_k(kern, dim3(grid), dim3(GB_THREADS), smem, L.stream, tmA, tmB, tmC, a2.e, a.M, a.K, stages, n_tiles, m_tiles);
   L.check("gemm_bres");
   return true;

@@ -82,6 +82,7 @@ struct Launch {
   std::string err;
   Profiler* prof = nullptr;
   std::string tag;       // which call site of the forward graph the next launches belong to
+  std::string kernel;    // the GEMM kernel instance launched last, e.g. "gemm_tc<BN=32,BK=64,kind=0x9,tma=0>" (edv_op_gemm)
   double nflops = 0, nbytes = 0;  // algorithmic work of the next launch (set by the launcher)
 
   void note(double flops, double bytes) {

@@ -9,6 +9,7 @@ namespace edv {
 
 template <typename T> void launch_gemm_simt(Launch& L, const GemmArgs& a) {
   note_gemm(L, a, sizeof(T));
+  L.kernel = "gemm_simt";
   dim3 grid((unsigned)((a.M + SG_BM - 1) / SG_BM), (a.N + SG_BN - 1) / SG_BN);
   ConvGeom g{};
   if (a.conv) {

@@ -101,6 +101,14 @@ inline Epi epi_zero() {
   return e;
 }
 
+// Epi::kind as launchers report it: the EF_* mask in hex, or -1 (generic epilogue)
+inline std::string kind_label(int kind) {
+  char b[16];
+  if (kind < 0) snprintf(b, sizeof b, "-1");
+  else snprintf(b, sizeof b, "0x%x", (unsigned)kind);
+  return b;
+}
+
 inline void note_gemm(Launch& L, const GemmArgs& a, size_t es) {
   // algorithmic work: 2*M*N*K; bytes: A (conv: the activation once) + W + C once
   const double a_elems = a.conv ? (double)a.F * a.H * a.Wd * a.C : (double)a.M * a.K;

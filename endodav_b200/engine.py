@@ -16,11 +16,11 @@ DTYPES = {"fp32": EDV_F32, "f32": EDV_F32, "float32": EDV_F32, "bf16": EDV_BF16,
           "fp16": EDV_F16, "f16": EDV_F16, "float16": EDV_F16}
 TORCH_DTYPE = {EDV_F32: torch.float32, EDV_BF16: torch.bfloat16, EDV_F16: torch.float16}
 
-ABI_VERSION = 12   # must equal EDV_ABI_VERSION of include/endodav_b200.h (argtypes below are mirrored by hand)
+ABI_VERSION = 13   # must equal EDV_ABI_VERSION of include/endodav_b200.h (argtypes below are mirrored by hand)
 
 EXPORTS = [
     "edv_abi_version", "edv_create", "edv_destroy", "edv_last_error", "edv_set_weight", "edv_plan", "edv_forward", "edv_forward_u8",
-    "edv_output_shape", "edv_launch_count", "edv_set_debug", "edv_debug_tap", "edv_plan_buffer", "edv_set_graph_mode", "edv_graph_count", "edv_graph_status", "edv_op_linear", "edv_op_conv3x3",
+    "edv_output_shape", "edv_launch_count", "edv_set_debug", "edv_debug_tap", "edv_plan_buffer", "edv_set_graph_mode", "edv_graph_count", "edv_graph_status", "edv_op_gemm",
     "edv_op_attention", "edv_op_temporal_attention", "edv_op_layernorm", "edv_op_groupnorm", "edv_op_upsample",
     "edv_op_resize_f32", "edv_profile", "edv_profile_reset", "edv_profile_collect", "edv_profile_get",
     "edv_op_disp_head", "edv_op_cubic_resize_u8", "edv_op_stitch_window", "edv_op_stitch_plan",
@@ -36,6 +36,30 @@ class EdvConfig(ctypes.Structure):
         ("res_blocks", ctypes.c_int32), ("rope", ctypes.c_int32), ("dtype", ctypes.c_int32), ("engine", ctypes.c_int32),
         ("no_motion", ctypes.c_int32), ("no_normalize", ctypes.c_int32), ("use_clstoken", ctypes.c_int32), ("no_cls", ctypes.c_int32),
     ]
+
+
+class EdvGemmDesc(ctypes.Structure):
+    """Mirror of edv_gemm_desc (include/endodav_b200.h); the library rejects a struct_bytes other than its own sizeof."""
+    _fields_ = [
+        ("struct_bytes", ctypes.c_int32),
+        ("A", ctypes.c_void_p), ("W", ctypes.c_void_p),
+        ("M", ctypes.c_int32), ("N", ctypes.c_int32), ("K", ctypes.c_int32), ("lda", ctypes.c_int64),
+        ("conv", ctypes.c_int32), ("F", ctypes.c_int32), ("H", ctypes.c_int32), ("Wd", ctypes.c_int32), ("C", ctypes.c_int32),
+        ("stride", ctypes.c_int32),
+        ("out", ctypes.c_void_p), ("out_relu", ctypes.c_void_p), ("bias", ctypes.c_void_p), ("rowbias", ctypes.c_void_p),
+        ("res1", ctypes.c_void_p), ("res2", ctypes.c_void_p), ("head_w", ctypes.c_void_p),
+        ("ldo", ctypes.c_int64), ("ld_res1", ctypes.c_int64), ("ld_res2", ctypes.c_int64), ("rb_ld", ctypes.c_int64),
+        ("rb_div", ctypes.c_int32), ("rb_mod", ctypes.c_int32),
+        ("out_f32", ctypes.c_int32), ("res1_f32", ctypes.c_int32), ("res2_f32", ctypes.c_int32),
+        ("act", ctypes.c_int32), ("map", ctypes.c_int32), ("map_p", ctypes.c_int32),
+        ("ps_k", ctypes.c_int32), ("ps_h", ctypes.c_int32), ("ps_w", ctypes.c_int32), ("ps_c", ctypes.c_int32),
+        ("sig_sign", ctypes.c_float),
+    ]
+
+
+# epilogue codes of csrc/common.cuh (Epi::act, Epi::map)
+ACT_NONE, ACT_GELU, ACT_RELU, ACT_GEGLU, ACT_HEAD, ACT_SIGMOID = 0, 1, 2, 3, 4, 5
+MAP_LINEAR, MAP_TOKENS, MAP_PIXSHUF = 0, 1, 2
 
 
 class EndoDAVError(RuntimeError):
@@ -85,8 +109,7 @@ def load_library():
     lib.edv_profile_get.argtypes = [vp, ci, ctypes.c_char_p, ci, ctypes.POINTER(ctypes.c_double),
                                     ctypes.POINTER(ctypes.c_longlong), ctypes.POINTER(ctypes.c_double),
                                     ctypes.POINTER(ctypes.c_double)]
-    lib.edv_op_linear.argtypes = [ci, ci, vp, vp, vp, vp, ci, ci, ci, ci, vp]
-    lib.edv_op_conv3x3.argtypes = [ci, ci, vp, vp, vp, vp, ci, ci, ci, ci, ci, ci, vp]
+    lib.edv_op_gemm.argtypes = [ci, ci, ctypes.POINTER(EdvGemmDesc), ctypes.c_char_p, ci, vp]
     lib.edv_op_attention.argtypes = [ci, ci, vp, vp, ci, ci, ci, vp]
     lib.edv_op_linear_residual_ln.argtypes = [ci, vp, vp, vp, vp, vp, vp, ctypes.c_float, vp, ci, ci, ci, vp, vp]
     lib.edv_op_linear_timeline.argtypes = [ci, vp, vp, vp, vp, ci, ci, ci, ci, vp, vp]
@@ -271,12 +294,63 @@ def _dt(t):
     return {torch.float32: EDV_F32, torch.bfloat16: EDV_BF16, torch.float16: EDV_F16}[t.dtype]
 
 
-def op_linear(A, W, bias=None, act=0, engine=ENGINE_TC):
-    lib = load_library()
-    M, K = A.shape
+def gemm_desc(A, W, out, M=None, lda=None, conv=None, bias=None, rowbias=None, res1=None, res2=None, out_relu=None,
+              head_w=None, ldo=None, ld_res1=None, ld_res2=None, rb_ld=0, rb_div=1, rb_mod=1, act=ACT_NONE, map=MAP_LINEAR,
+              map_p=0, ps=(0, 0, 0, 0), sig_sign=0.0):
+    """-> EdvGemmDesc for out = epilogue(A W^T).  A [M, K] (row pitch lda) or, with conv = (F, H, W, C, stride), an NHWC
+    activation for a 3x3 pad-1 convolution (K = 9 C); W [N, K].  Leading dimensions default to N; ld_res1 / ld_res2 to ldo.
+    out / res1 / res2 are float32 tensors (out_f32 / res*_f32) or in A's dtype; ps = (k, grid h, grid w, channels)."""
     N = W.shape[0]
-    C = torch.empty(M, N, dtype=A.dtype, device=A.device)
-    _check(lib.edv_op_linear(_dt(A), engine, _ptr(A), _ptr(W), _ptr(bias), _ptr(C), M, N, K, act, _stream()), None, "edv_op_linear")
+    d = EdvGemmDesc()
+    d.struct_bytes = ctypes.sizeof(EdvGemmDesc)
+    d.A, d.W, d.N, d.K = A.data_ptr(), W.data_ptr(), N, W.shape[1]
+    if conv is not None:
+        d.conv = 1
+        d.F, d.H, d.Wd, d.C, d.stride = conv
+        d.M = M if M is not None else d.F * ((d.H - 1) // d.stride + 1) * ((d.Wd - 1) // d.stride + 1)
+        d.lda = d.K
+    else:
+        d.M = M if M is not None else A.shape[0]
+        d.lda = lda if lda is not None else A.shape[1]
+        d.stride = 1
+    d.out, d.out_relu = _ptr(out).value, _ptr(out_relu).value
+    d.bias, d.rowbias, d.head_w = _ptr(bias).value, _ptr(rowbias).value, _ptr(head_w).value
+    d.res1, d.res2 = _ptr(res1).value, _ptr(res2).value
+    d.ldo = ldo if ldo is not None else N
+    d.ld_res1 = ld_res1 if ld_res1 is not None else d.ldo
+    d.ld_res2 = ld_res2 if ld_res2 is not None else d.ldo
+    d.rb_ld, d.rb_div, d.rb_mod = rb_ld, rb_div, rb_mod
+    d.out_f32 = int(out is not None and out.dtype == torch.float32)
+    d.res1_f32 = int(res1 is not None and res1.dtype == torch.float32)
+    d.res2_f32 = int(res2 is not None and res2.dtype == torch.float32)
+    d.act, d.map, d.map_p = act, map, map_p
+    d.ps_k, d.ps_h, d.ps_w, d.ps_c = ps
+    d.sig_sign = sig_sign
+    return d
+
+
+def op_gemm_status(dtype, engine, desc):
+    """-> (edv_status, name of the kernel instance that ran, e.g. "gemm_tc<BN=32,BK=64,kind=0x9,tma=0>")."""
+    lib = load_library()
+    name = ctypes.create_string_buffer(128)
+    # without a device there is no stream; the library then rejects the call or fails at the launch
+    stream = _stream() if torch.cuda.is_available() else ctypes.c_void_p(0)
+    rc = lib.edv_op_gemm(dtype, engine, ctypes.byref(desc), name, 128, stream)
+    return rc, name.value.decode()
+
+
+def op_gemm(A, W, out, engine=ENGINE_TC, **epi):
+    """out (and epi["out_relu"]) = the fused epilogue of A W^T (gemm_desc), through the forward's own GEMM dispatcher;
+    returns the kernel instance that ran."""
+    rc, kernel = op_gemm_status(_dt(A), engine, gemm_desc(A, W, out, **epi))
+    _check(rc, None, "edv_op_gemm")
+    return kernel
+
+
+def op_linear(A, W, bias=None, act=0, engine=ENGINE_TC):
+    M = A.shape[0]
+    C = torch.empty(M, W.shape[0], dtype=A.dtype, device=A.device)
+    op_gemm(A, W, C, engine, bias=bias, act=act)
     return C
 
 
@@ -305,12 +379,9 @@ def op_linear_timeline(A, W, bias=None, act=0):
 
 
 def op_conv3x3(X, Wt, bias=None, relu_out=False, engine=ENGINE_TC):
-    lib = load_library()
     F, H, W, Cin = X.shape
-    Cout = Wt.shape[0]
-    Y = torch.empty(F, H, W, Cout, dtype=X.dtype, device=X.device)
-    _check(lib.edv_op_conv3x3(_dt(X), engine, _ptr(X), _ptr(Wt), _ptr(bias), _ptr(Y), F, H, W, Cin, Cout, int(relu_out), _stream()),
-           None, "edv_op_conv3x3")
+    Y = torch.empty(F, H, W, Wt.shape[0], dtype=X.dtype, device=X.device)
+    op_gemm(X, Wt, Y, engine, conv=(F, H, W, Cin, 1), bias=bias, act=ACT_RELU if relu_out else ACT_NONE)
     return Y
 
 

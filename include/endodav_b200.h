@@ -30,7 +30,7 @@ typedef struct edv_ctx edv_ctx;
 /* Bumped whenever an entry point's argument list or a struct layout changes.  The ctypes host
  * (endodav_b200/engine.py) mirrors the signatures by hand, so it refuses a library whose
  * edv_abi_version() differs from its own constant instead of calling it with a stale layout. */
-#define EDV_ABI_VERSION 12
+#define EDV_ABI_VERSION 13
 int edv_abi_version(void);
 
 enum edv_status {
@@ -150,14 +150,46 @@ int edv_plan_buffer(edv_ctx* ctx, int index, char* name, int name_cap, size_t* o
 
 /* --- per-kernel entry points (unit parity tests + ncu) ---------------------------------- */
 
-/* C[M,N] = A[M,K] * W[N,K]^T (+bias) with optional activation; A,W,C in `dtype`
- * (fp32 accumulate).  act: 0 none, 1 GELU(erf), 2 ReLU.  engine as in edv_config.
- * Replaces: every nn.Linear / 1x1 conv on the path (attention.py:58,67; mlp.py:34-37; ...). */
-int edv_op_linear(int dtype, int engine, const void* A, const void* W, const float* bias, void* C, int M, int N, int K,
-                  int act, void* stream);
+/* One GEMM / 3x3 convolution through the forward's own dispatcher and kernels, with any epilogue the forward uses:
+ *   out = epilogue(A[M,K] * W[N,K]^T)   (A, W in `dtype`, fp32 accumulate; engine as in edv_config)
+ * The fields after the conv geometry are those of the library's epilogue description (csrc/common.cuh: Epi), in the
+ * order it applies them: + bias[n], + rowbias[(m / rb_div) % rb_mod][n] (row pitch rb_ld), GELU (act 1), row map
+ * (map 1 tokens: out row m + m / map_p + 1; map 2 pixel shuffle: column (ky*ps_k + kx)*ps_c + c of grid cell m ->
+ * pixel (ps_k y + ky, ps_k x + kx) of a [ps_h ps_k, ps_w ps_k] map), + res1, + res2, ReLU (act 2) or
+ * sigmoid(sig_sign x) (act 5), store to out and relu(value) to out_relu.  act 3 (GEGLU: column pairs of 64 value | 64
+ * gate per 128, out has N/2 columns) and act 4 (disparity head, N = 32: relu(relu(v + bias) . head_w[0..31] +
+ * head_w[32]) or its sigmoid(sig_sign .), one float per row) exist on the tensor-core engine only.
+ * *_f32 = 1: that tensor is float32, else `dtype`.  Leading dimensions are in elements and multiples of 8.
+ * conv = 1: A is an NHWC activation [F,H,Wd,C], padding 1, K = 9*C in (ky,kx,c) order, M = F*OH*OW; stride 2 runs on
+ * the CUDA-core engine only.  struct_bytes must equal sizeof(edv_gemm_desc).
+ * `kernel` (may be NULL) receives the kernel instance that ran, e.g. "gemm_tc<BN=32,BK=64,kind=0x9,tma=0>".
+ * Replaces: every nn.Linear / 1x1 / 3x3 conv on the path (attention.py:58,67; mlp.py:34-37; dpt.py:100-117; ...). */
+typedef struct edv_gemm_desc {
+  int32_t struct_bytes;
+  const void* A;
+  const void* W;
+  int32_t M, N, K;
+  int64_t lda;
+  int32_t conv, F, H, Wd, C, stride;
+  void* out;
+  void* out_relu;
+  const float* bias;
+  const float* rowbias;
+  const void* res1;
+  const void* res2;
+  const float* head_w;
+  int64_t ldo, ld_res1, ld_res2, rb_ld;
+  int32_t rb_div, rb_mod;
+  int32_t out_f32, res1_f32, res2_f32;
+  int32_t act, map, map_p;
+  int32_t ps_k, ps_h, ps_w, ps_c;
+  float sig_sign;
+} edv_gemm_desc;
+int edv_op_gemm(int dtype, int engine, const edv_gemm_desc* d, char* kernel, int kernel_cap, void* stream);
 
-/* edv_op_linear on the tcgen05 kernel (16-bit dtypes) that also records the kernel's own timeline: 4 CTAs x 256 clock64
- * stamps (per-tile accumulator-free / issued / complete / stored times, slot table in csrc/gemm_tc.cuh). */
+/* C[M,N] = A[M,K] W[N,K]^T (+bias), act 0 none / 1 GELU / 2 ReLU, on the tcgen05 kernel (16-bit dtypes), recording the
+ * kernel's own timeline: 4 CTAs x 256 clock64 stamps (per-tile accumulator-free / issued / complete / stored times,
+ * slot table in csrc/gemm_tc.cuh). */
 int edv_op_linear_timeline(int dtype, const void* A, const void* W, const float* bias, void* C, int M, int N, int K, int act,
                            long long* timeline_dev, void* stream);
 
@@ -168,12 +200,6 @@ int edv_op_linear_timeline(int dtype, const void* A, const void* W, const float*
  * the next norm (layers/block.py:110-116,143-145; LayerScale is folded into W / bias by pack.py). */
 int edv_op_linear_residual_ln(int dtype, const void* A, const void* W, const float* bias, float* x_inout, const float* gamma,
                               const float* beta, float eps, void* xn_out, int M, int N, int K, long long* timeline_dev, void* stream);
-
-/* 3x3 convolution, padding 1, stride 1, NHWC: X[F,H,W,Cin] * Wt[Cout, 9*Cin] (+bias),
- * pre_relu applies ReLU to X first (ResidualConvUnit, util/blocks.py:78-84).
- * Replaces: scratch.layer*_rn, resConfUnit convs, output_conv1 (dpt.py:100-117). */
-int edv_op_conv3x3(int dtype, int engine, const void* X, const void* Wt, const float* bias, void* Y, int F, int H,
-                   int W, int Cin, int Cout, int relu_out, void* stream);
 
 /* Spatial multi-head attention over token-major qkv [F*S, 3*heads*64] (q pre-scaled) ->
  * out [F*S, heads*64].  Replaces: Attention.forward's softmax(qk^T)v (attention.py:60-66). */

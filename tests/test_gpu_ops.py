@@ -231,7 +231,7 @@ def test_disp_head_fused(dtype, Fr, h, w, oh, ow, C, sig):
 
 def test_linear_kernels_agree_bitwise():
     """The tcgen05 linear kernels that shape selects between must agree bit for bit on the same operands (same fp32
-    accumulation order per output element; act = none):
+    accumulation order per output element), for act = none and ReLU:
       A [20000, 384], W [1152, 384]   M >= 2048      -> B-resident gemm_bres, TMA-store epilogue
       A[:2000]                        M < 2048       -> streaming gemm_tc at BN = 192, TMA-store epilogue
       A[:2000], W[:1120]              N % 64 != 0    -> streaming gemm_tc at BN = 32, row-segment epilogue"""
@@ -239,11 +239,15 @@ def test_linear_kernels_agree_bitwise():
     A = torch.randn(20000, 384, generator=g).half().cuda()
     W = (torch.randn(1152, 384, generator=g) * 0.05).half().cuda()
     b = torch.randn(1152, generator=g).cuda()
-    bres = eng.op_linear(A, W, b, 0)
-    tc192 = eng.op_linear(A[:2000], W, b, 0)
-    tc32 = eng.op_linear(A[:2000], W[:1120], b[:1120], 0)
-    assert torch.equal(bres[:2000], tc192)
-    assert torch.equal(tc192[:, :1120], tc32)
+    for act, kind in ((0, "0x1"), (2, "0x5")):
+        bres = torch.empty(20000, 1152, dtype=torch.half, device=DEV)
+        tc192 = torch.empty(2000, 1152, dtype=torch.half, device=DEV)
+        tc32 = torch.empty(2000, 1120, dtype=torch.half, device=DEV)
+        assert eng.op_gemm(A, W, bres, bias=b, act=act) == "gemm_bres<BN=192>"
+        assert eng.op_gemm(A[:2000], W, tc192, bias=b, act=act) == "gemm_tc<BN=192,BK=64,kind=%s,tma=1>" % kind
+        assert eng.op_gemm(A[:2000], W[:1120], tc32, bias=b[:1120], act=act) == "gemm_tc<BN=32,BK=64,kind=%s,tma=0>" % kind
+        assert torch.equal(bres[:2000], tc192)
+        assert torch.equal(tc192[:, :1120], tc32)
 
 
 # ---- GPU-side preprocessing of the long-video driver ------------------------------------------------
