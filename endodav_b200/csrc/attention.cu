@@ -39,6 +39,7 @@ void launch_temporal(Launch& L, const void* qkv, void* out, int B, int Tn, int h
   smem_opt_in<kern>(200 * 1024);
   dim3 grid((hw + pb - 1) / pb, B, heads / hg);
   L.note(4.0 * B * hw * heads * (double)Tn * Tn * HD, 4.0 * B * Tn * hw * C * sizeof(T));
+  L.kernel = "temporal_attention_simt<HD=" + std::to_string(HD) + ",PB=" + std::to_string(pb) + ",HG=" + std::to_string(hg) + ">";
   kern<<<grid, 32 * hg * pb, smem, L.stream>>>((const T*)qkv, (T*)out, Tn, hw, C, pb, hg, (const float2*)rope);   // fp32 CUDA-core path: no PDL hooks, plain launch
   L.check("temporal_attention");
 }
@@ -51,6 +52,7 @@ void launch_temporal_mma_pb(Launch& L, const void* qkv, void* out, int B, int Tn
   dim3 grid((hw + PB - 1) / PB, B);
   const int C = 8 * HD;
   L.note(4.0 * B * hw * 8 * (double)Tn * Tn * HD, 4.0 * B * Tn * hw * C * sizeof(T));
+  L.kernel = "temporal_attention_mma<HD=" + std::to_string(HD) + ",PB=" + std::to_string(PB) + ">";
   edv::launch_k(kern, dim3(grid), dim3(tmma::TA_WARPS * 32), smem, L.stream, (const T*)qkv, (T*)out, Tn, hw, (const float2*)rope);
   L.check("temporal_attention");
 }

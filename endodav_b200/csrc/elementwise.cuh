@@ -482,13 +482,6 @@ __global__ void im2col3x3_kernel(const T* __restrict__ x, T* __restrict__ out, i
   store_vec<T, 8>(out + (p * 9 + tap) * C + c, v);
 }
 
-// copy T -> float32 (debug taps)
-template <typename T>
-__global__ void to_f32_kernel(const T* __restrict__ x, float* __restrict__ y, long long n) {
-  long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) y[i] = to_f<T>(x[i]);
-}
-
 // strided channel copy NHWC [.., Cs] -> [.., Cd] (first min(Cs,Cd) channels), debug taps of padded maps
 template <typename T>
 __global__ void copy_channels_f32_kernel(const T* __restrict__ x, float* __restrict__ y, long long rows, int Cs, int Cd) {

@@ -294,11 +294,7 @@ struct Fwd {
     } else {
       void* tmp = buf((set + "gg2").c_str());
       linear(lnb, Mm, C, n + "geglu.w", 8 * C, ep(tmp, 8 * C, wf(n + "geglu.b", 8 * C)));
-      if (L.ok()) {
-        long long tot = Mm * 4 * C;
-        EDV_DISPATCH_T(dt, { geglu_pair_kernel<T><<<nblk(tot, 256), 256, 0, L.stream>>>((const T*)tmp, (T*)gg, Mm, 4 * C); });
-        L.check("geglu");
-      }
+      geglu_pair(L, dt, tmp, gg, Mm, 4 * C);
     }
     {
       Epi e = ep(hsT, C, wf(n + "ff2.b", C));
@@ -381,14 +377,7 @@ struct Fwd {
       Epi e = ep(t32, 32, wf(c2 + ".b", 32));
       e.act = ACT_RELU;
       conv3(up, p.BT, OH, OW, Fh, c2 + ".w", 32, e);
-      if (L.ok()) {
-        long long Mh = (long long)p.BT * OH * OW;
-        EDV_DISPATCH_T(dt, {
-          head_dot_kernel<T><<<nblk(Mh, 256), 256, 0, L.stream>>>((const T*)t32, hw_, out, Mh, 32, sig_sign == 0.f, sig_sign,
-                                                                sig_sign != 0.f);
-        });
-        L.check("head_dot");
-      }
+      head_dot(L, dt, t32, hw_, out, (long long)p.BT * OH * OW, 32, sig_sign);
     }
   }
 
@@ -401,15 +390,8 @@ struct Fwd {
     void* A0 = buf("A0");
     float* x = (float*)buf("x");
     {
-      long long tot = p.Mp * KPATCH;
-      unsigned blocks = nblk(tot / 8, 256);
-      L.note(0, (double)p.BT * 3 * p.H * p.W * (u8 ? 1 : 4) + (double)tot * es);
-      EDV_DISPATCH_T(dt, {
-        const int nrm = g.no_normalize ? 0 : 1;  // endodac with pre_norm=False feeds raw [0,1] pixels (endodac.py:208-211)
-        if (u8) preprocess_patches_kernel<T, true><<<blocks, 256, 0, L.stream>>>(frames, (T*)A0, p.BT, p.H, p.W, p.h, p.w, KPATCH, nrm);
-        else preprocess_patches_kernel<T, false><<<blocks, 256, 0, L.stream>>>(frames, (T*)A0, p.BT, p.H, p.W, p.h, p.w, KPATCH, nrm);
-      });
-      L.check("preprocess");
+      // endodac with pre_norm=False feeds raw [0,1] pixels (endodac.py:208-211)
+      preprocess_patches(L, dt, frames, u8, A0, p.BT, p.H, p.W, p.h, p.w, KPATCH, g.no_normalize ? 0 : 1);
       const float* cls = g.no_cls ? nullptr : wf("cls_row", D);
       if (cls && L.ok()) {
         edv::launch_k(cls_row_kernel, dim3(nblk((long long)p.BT * D, 256)), dim3(256), 0, L.stream, x, cls, p.BT, p.N, D);
@@ -553,11 +535,7 @@ struct Fwd {
       const long long Mo = (long long)p.BT * p.ph2 * p.pw2;
       if (tc()) {
         void* col = buf("col");
-        if (L.ok()) {
-          long long tot = Mo * 9 * (p.Cp[3] / 8);
-          EDV_DISPATCH_T(dt, { edv::launch_k(im2col3x3_kernel<T>, dim3(nblk(tot, 256)), dim3(256), 0, L.stream, (const T*)L4p, (T*)col, p.BT, p.ph, p.pw, p.Cp[3], p.ph2, p.pw2, 2); });
-          L.check("im2col");
-        }
+        im2col3x3(L, dt, L4p, col, p.BT, p.ph, p.pw, p.Cp[3], p.ph2, p.pw2, 2);
         linear(col, Mo, 9 * p.Cp[3], "resize3.w", p.Cp[3], ep(L4, p.Cp[3], wf("resize3.b", p.Cp[3])));
       } else {
         GemmArgs a;
@@ -624,26 +602,14 @@ struct Fwd {
     void* t1 = buf("rb.t1");
     void* t2 = buf("rb.t2");
     void* t3 = buf("rb.t3");
-    if (!L.ok()) return;
-    EDV_DISPATCH_T(dt, {
-      tokens_to_patches_kernel<T><<<nblk(p.Mp * (D / 4), 256), 256, 0, L.stream>>>(x, (T*)pt, p.Mp, p.P, D, c->cfg.no_cls ? 0 : 1);
-    });
-    L.check("tokens_to_patches");
+    const int cls = c->cfg.no_cls ? 0 : 1;
+    tokens_to_patches(L, dt, x, pt, p.Mp, p.P, D, cls);
     linear(pt, p.Mp, D, n + "res.c1.w", bcp, ep(t1, bcp, nullptr));
-    if (L.ok()) {
-      EDV_DISPATCH_T(dt, { rowln_act_kernel<T><<<nblk(p.Mp * 32, 256), 256, 0, L.stream>>>((const T*)t1, wf(n + "res.n1.w", bcp), wf(n + "res.n1.b", bcp), (T*)t2, p.Mp, bcp, bc, 1e-6f, 1); });
-      L.check("res ln1");
-    }
+    rowln_act(L, dt, t1, wf(n + "res.n1.w", bcp), wf(n + "res.n1.b", bcp), t2, p.Mp, bcp, bc, 1e-6f, 1, "res ln1");
     conv3(t2, p.BT, p.ph, p.pw, bcp, n + "res.c2.w", bcp, ep(t1, bcp, nullptr));
-    if (L.ok()) {
-      EDV_DISPATCH_T(dt, { rowln_act_kernel<T><<<nblk(p.Mp * 32, 256), 256, 0, L.stream>>>((const T*)t1, wf(n + "res.n2.w", bcp), wf(n + "res.n2.b", bcp), (T*)t2, p.Mp, bcp, bc, 1e-6f, 1); });
-      L.check("res ln2");
-    }
+    rowln_act(L, dt, t1, wf(n + "res.n2.w", bcp), wf(n + "res.n2.b", bcp), t2, p.Mp, bcp, bc, 1e-6f, 1, "res ln2");
     linear(t2, p.Mp, bcp, n + "res.c3.w", D, ep(t3, D, nullptr));
-    if (L.ok()) {
-      EDV_DISPATCH_T(dt, { resblock_add_kernel<T><<<nblk(p.Mp * 32, 256), 256, 0, L.stream>>>(x, (const T*)t3, wf(n + "res.n3.w", D), wf(n + "res.n3.b", D), p.Mp, p.P, D, 1e-6f, c->cfg.no_cls ? 0 : 1); });
-      L.check("res add");
-    }
+    resblock_add(L, dt, x, t3, wf(n + "res.n3.w", D), wf(n + "res.n3.b", D), p.Mp, p.P, D, 1e-6f, cls);
   }
 };
 
@@ -1196,6 +1162,8 @@ int edv_profile_get(edv_ctx* ctx, int index, char* name, int name_cap, double* m
 }
 
 // ---- per-kernel entry points ----------------------------------------------------------------
+static bool aligned16(const void* p) { return ((uintptr_t)p & 15) == 0; }   // NULL passes: nullable pointers are checked apart
+
 static int finish(Launch& L) {
   if (!L.ok()) g_create_error = L.err;
   return L.status;
@@ -1298,10 +1266,18 @@ int edv_op_attention_timeline(int dtype, const void* qkv, void* out, int F, int 
   return finish(L);
 }
 
-int edv_op_temporal_attention(int dtype, const void* qkv, void* out, int B, int T, int hw, int C, void* stream) {
+int edv_op_temporal_attention(int dtype, const void* qkv, void* out, int B, int T, int hw, int C, const float* rope, char* kernel,
+                              int kernel_cap, void* stream) {
+  if (kernel && kernel_cap > 0) kernel[0] = 0;
+  if (dtype < EDV_F32 || dtype > EDV_F16) return set_err(nullptr, EDV_ERR_ARG, "edv_op_temporal_attention: bad dtype %d", dtype);
+  if (!qkv || !out) return set_err(nullptr, EDV_ERR_ARG, "edv_op_temporal_attention: null qkv or out");
+  if (B < 1 || hw < 1) return set_err(nullptr, EDV_ERR_ARG, "edv_op_temporal_attention: empty problem");
+  if (!aligned16(qkv) || !aligned16(out) || !aligned16(rope))
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_temporal_attention: qkv, out and rope must be 16-byte aligned");
   Launch L;
   L.stream = (cudaStream_t)stream;
-  temporal_attention(L, dtype, qkv, out, B, T, hw, C);
+  temporal_attention(L, dtype, qkv, out, B, T, hw, C, rope);
+  if (kernel && kernel_cap > 0) snprintf(kernel, kernel_cap, "%s", L.kernel.c_str());
   return finish(L);
 }
 
@@ -1324,11 +1300,101 @@ int edv_op_cubic_resize_u8(const uint8_t* src, float* dst, int N, int H, int W, 
   return finish(L);
 }
 
-int edv_op_layernorm(int dtype, const float* X, const float* gamma, const float* beta, void* Y, int M, int D,
-                     float eps, void* stream) {
+int edv_op_layernorm(int dtype, const float* X, const float* gamma, const float* beta, void* Y, int M, int D, float eps, int grp,
+                     int skip, const float* add, int add_div, int add_mod, void* stream) {
+  if (dtype < EDV_F32 || dtype > EDV_F16) return set_err(nullptr, EDV_ERR_ARG, "edv_op_layernorm: bad dtype %d", dtype);
+  if (!X || !gamma || !beta || !Y) return set_err(nullptr, EDV_ERR_ARG, "edv_op_layernorm: null argument");
+  if (M < 1) return set_err(nullptr, EDV_ERR_ARG, "edv_op_layernorm: empty problem");
+  if (grp < 0 || (grp == 0 && skip != 0) || (grp > 0 && (skip >= grp || -skip > grp)))
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_layernorm: skip %d outside (-grp, grp) for grp %d", skip, grp);
+  if (add && (add_div < 1 || add_mod < 1)) return set_err(nullptr, EDV_ERR_ARG, "edv_op_layernorm: add_div and add_mod must be >= 1");
+  if (!aligned16(X) || !aligned16(gamma) || !aligned16(beta) || !aligned16(add))
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_layernorm: X, gamma, beta and add must be 16-byte aligned");
   Launch L;
   L.stream = (cudaStream_t)stream;
-  layernorm(L, dtype, X, gamma, beta, Y, M, D, eps);
+  layernorm(L, dtype, X, gamma, beta, Y, M, D, eps, grp, skip, add, add ? add_div : 1, add ? add_mod : 1);
+  return finish(L);
+}
+
+int edv_op_preprocess_patches(int dtype, const void* src, int u8, void* out, int F, int H, int W, int h, int w, int normalize,
+                              void* stream) {
+  if (dtype < EDV_F32 || dtype > EDV_F16) return set_err(nullptr, EDV_ERR_ARG, "edv_op_preprocess_patches: bad dtype %d", dtype);
+  if (!src || !out) return set_err(nullptr, EDV_ERR_ARG, "edv_op_preprocess_patches: null src or out");
+  if (F < 1 || H < 1 || W < 1 || h < 14 || w < 14 || h % 14 || w % 14)
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_preprocess_patches: frames must be non-empty and h, w multiples of 14");
+  if (u8 && (H != h || W != w)) return set_err(nullptr, EDV_ERR_ARG, "edv_op_preprocess_patches: uint8 frames must be at network resolution");
+  if (!aligned16(out)) return set_err(nullptr, EDV_ERR_ARG, "edv_op_preprocess_patches: out must be 16-byte aligned");
+  Launch L;
+  L.stream = (cudaStream_t)stream;
+  preprocess_patches(L, dtype, src, u8 != 0, out, F, H, W, h, w, KPATCH, normalize ? 1 : 0);
+  return finish(L);
+}
+
+int edv_op_tokens_to_patches(int dtype, const float* x, void* out, long long Mp, int P, int D, int cls, void* stream) {
+  if (dtype < EDV_F32 || dtype > EDV_F16) return set_err(nullptr, EDV_ERR_ARG, "edv_op_tokens_to_patches: bad dtype %d", dtype);
+  if (!x || !out) return set_err(nullptr, EDV_ERR_ARG, "edv_op_tokens_to_patches: null x or out");
+  if (Mp < 1 || P < 1 || Mp % P || D < 4 || D % 4 || (cls != 0 && cls != 1))
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_tokens_to_patches: needs Mp a multiple of P, D %% 4 == 0, cls 0 or 1");
+  if (!aligned16(x) || !aligned16(out)) return set_err(nullptr, EDV_ERR_ARG, "edv_op_tokens_to_patches: x and out must be 16-byte aligned");
+  Launch L;
+  L.stream = (cudaStream_t)stream;
+  tokens_to_patches(L, dtype, x, out, Mp, P, D, cls);
+  return finish(L);
+}
+
+int edv_op_rowln_act(int dtype, const void* x, const float* gamma, const float* beta, void* y, long long M, int C, int Cr, float eps,
+                     int gelu, void* stream) {
+  if (dtype < EDV_F32 || dtype > EDV_F16) return set_err(nullptr, EDV_ERR_ARG, "edv_op_rowln_act: bad dtype %d", dtype);
+  if (!x || !gamma || !beta || !y) return set_err(nullptr, EDV_ERR_ARG, "edv_op_rowln_act: null argument");
+  if (M < 1 || Cr < 1 || Cr > C) return set_err(nullptr, EDV_ERR_ARG, "edv_op_rowln_act: needs M >= 1 and 1 <= Cr <= C");
+  Launch L;
+  L.stream = (cudaStream_t)stream;
+  rowln_act(L, dtype, x, gamma, beta, y, M, C, Cr, eps, gelu ? 1 : 0);
+  return finish(L);
+}
+
+int edv_op_resblock_add(int dtype, float* x, const void* r, const float* gamma, const float* beta, long long Mp, int P, int D, float eps,
+                        int cls, void* stream) {
+  if (dtype < EDV_F32 || dtype > EDV_F16) return set_err(nullptr, EDV_ERR_ARG, "edv_op_resblock_add: bad dtype %d", dtype);
+  if (!x || !r || !gamma || !beta) return set_err(nullptr, EDV_ERR_ARG, "edv_op_resblock_add: null argument");
+  if (Mp < 1 || P < 1 || Mp % P || D < 1 || (cls != 0 && cls != 1))
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_resblock_add: needs Mp a multiple of P, D >= 1, cls 0 or 1");
+  Launch L;
+  L.stream = (cudaStream_t)stream;
+  resblock_add(L, dtype, x, r, gamma, beta, Mp, P, D, eps, cls);
+  return finish(L);
+}
+
+int edv_op_im2col3x3(int dtype, const void* x, void* out, int F, int H, int W, int C, int stride, void* stream) {
+  if (dtype < EDV_F32 || dtype > EDV_F16) return set_err(nullptr, EDV_ERR_ARG, "edv_op_im2col3x3: bad dtype %d", dtype);
+  if (!x || !out) return set_err(nullptr, EDV_ERR_ARG, "edv_op_im2col3x3: null x or out");
+  if (F < 1 || H < 1 || W < 1 || C < 8 || C % 8 || stride < 1 || stride > 2)
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_im2col3x3: needs a non-empty map, C %% 8 == 0 and stride 1 or 2");
+  if (!aligned16(x) || !aligned16(out)) return set_err(nullptr, EDV_ERR_ARG, "edv_op_im2col3x3: x and out must be 16-byte aligned");
+  Launch L;
+  L.stream = (cudaStream_t)stream;
+  im2col3x3(L, dtype, x, out, F, H, W, C, (H - 1) / stride + 1, (W - 1) / stride + 1, stride);
+  return finish(L);
+}
+
+int edv_op_geglu_pair(int dtype, const void* hg, void* out, long long M, int C4, void* stream) {
+  if (dtype < EDV_F32 || dtype > EDV_F16) return set_err(nullptr, EDV_ERR_ARG, "edv_op_geglu_pair: bad dtype %d", dtype);
+  if (!hg || !out) return set_err(nullptr, EDV_ERR_ARG, "edv_op_geglu_pair: null hg or out");
+  if (M < 1 || C4 < 64 || C4 % 64) return set_err(nullptr, EDV_ERR_ARG, "edv_op_geglu_pair: needs M >= 1 and C4 a multiple of 64");
+  Launch L;
+  L.stream = (cudaStream_t)stream;
+  geglu_pair(L, dtype, hg, out, M, C4);
+  return finish(L);
+}
+
+int edv_op_head_dot(int dtype, const void* x, const float* w, float* out, long long M, int C, float sig_sign, void* stream) {
+  if (dtype < EDV_F32 || dtype > EDV_F16) return set_err(nullptr, EDV_ERR_ARG, "edv_op_head_dot: bad dtype %d", dtype);
+  if (!x || !w || !out) return set_err(nullptr, EDV_ERR_ARG, "edv_op_head_dot: null x, w or out");
+  if (M < 1 || C < 8 || C % 8) return set_err(nullptr, EDV_ERR_ARG, "edv_op_head_dot: needs M >= 1 and C a multiple of 8");
+  if (!aligned16(x)) return set_err(nullptr, EDV_ERR_ARG, "edv_op_head_dot: x must be 16-byte aligned");
+  Launch L;
+  L.stream = (cudaStream_t)stream;
+  head_dot(L, dtype, x, w, out, M, C, sig_sign);
   return finish(L);
 }
 

@@ -82,7 +82,8 @@ struct Launch {
   std::string err;
   Profiler* prof = nullptr;
   std::string tag;       // which call site of the forward graph the next launches belong to
-  std::string kernel;    // the GEMM kernel instance launched last, e.g. "gemm_tc<BN=32,BK=64,kind=0x9,tma=0>" (edv_op_gemm)
+  std::string kernel;    // the GEMM or temporal-attention instance launched last, e.g. "gemm_tc<BN=32,BK=64,kind=0x9,tma=0>",
+                         // "temporal_attention_mma<HD=24,PB=2>" (edv_op_gemm, edv_op_temporal_attention)
   double nflops = 0, nbytes = 0;  // algorithmic work of the next launch (set by the launcher)
 
   void note(double flops, double bytes) {

@@ -131,4 +131,65 @@ inline void resize_f32(Launch& L, const float* x, float* y, int F, int h, int w,
   L.check("resize_f32");
 }
 
+// K1: frames (float32 [F,3,H,W] or, u8, uint8 [F,H,W,3] at network resolution) -> out [F*(h/14)*(w/14), Kp]
+inline void preprocess_patches(Launch& L, int dtype, const void* src, bool u8, void* out, int F, int H, int W, int h, int w,
+                               int Kp, int normalize) {
+  if (!L.ok()) return;
+  const long long tot = (long long)F * (h / 14) * (w / 14) * Kp;
+  const unsigned blocks = nblk(tot / 8, 256);
+  L.note(0, (double)F * 3 * H * W * (u8 ? 1 : 4) + (double)tot * dtype_size(dtype));
+  EDV_DISPATCH_T(dtype, {
+    if (u8) preprocess_patches_kernel<T, true><<<blocks, 256, 0, L.stream>>>(src, (T*)out, F, H, W, h, w, Kp, normalize);
+    else preprocess_patches_kernel<T, false><<<blocks, 256, 0, L.stream>>>(src, (T*)out, F, H, W, h, w, Kp, normalize);
+  });
+  L.check("preprocess");
+}
+
+// patch rows of the fp32 residual stream x [Mp/P frames][P + cls][D] -> out [Mp, D] in `dtype`
+inline void tokens_to_patches(Launch& L, int dtype, const float* x, void* out, long long Mp, int P, int D, int cls) {
+  if (!L.ok()) return;
+  EDV_DISPATCH_T(dtype, { tokens_to_patches_kernel<T><<<nblk(Mp * (D / 4), 256), 256, 0, L.stream>>>(x, (T*)out, Mp, P, D, cls); });
+  L.check("tokens_to_patches");
+}
+
+// y [M, C] = act(LN over the first Cr of the C channels of x), padding columns Cr..C-1 written as 0
+inline void rowln_act(Launch& L, int dtype, const void* x, const float* gamma, const float* beta, void* y, long long M, int C,
+                      int Cr, float eps, int gelu, const char* what = "rowln_act") {
+  if (!L.ok()) return;
+  EDV_DISPATCH_T(dtype, { rowln_act_kernel<T><<<nblk(M * 32, 256), 256, 0, L.stream>>>((const T*)x, gamma, beta, (T*)y, M, C, Cr, eps, gelu); });
+  L.check(what);
+}
+
+// x (fp32 residual stream, in place): patch row p of every frame += LN(r[p]); cls rows untouched
+inline void resblock_add(Launch& L, int dtype, float* x, const void* r, const float* gamma, const float* beta, long long Mp, int P,
+                         int D, float eps, int cls) {
+  if (!L.ok()) return;
+  EDV_DISPATCH_T(dtype, { resblock_add_kernel<T><<<nblk(Mp * 32, 256), 256, 0, L.stream>>>(x, (const T*)r, gamma, beta, Mp, P, D, eps, cls); });
+  L.check("res add");
+}
+
+// 3x3 pad-1 im2col of NHWC x [F,H,W,C] -> out [F*OH*OW, 9*C] in (ky,kx,c) order
+inline void im2col3x3(Launch& L, int dtype, const void* x, void* out, int F, int H, int W, int C, int OH, int OW, int stride) {
+  if (!L.ok()) return;
+  const long long tot = (long long)F * OH * OW * 9 * (C / 8);
+  EDV_DISPATCH_T(dtype, { edv::launch_k(im2col3x3_kernel<T>, dim3(nblk(tot, 256)), dim3(256), 0, L.stream, (const T*)x, (T*)out, F, H, W, C, OH, OW, stride); });
+  L.check("im2col");
+}
+
+// out [M, C4] = value * gelu(gate) of hg [M, 2*C4] in pack.py's [64 value | 64 gate] column pairs (CUDA-core GEGLU)
+inline void geglu_pair(Launch& L, int dtype, const void* hg, void* out, long long M, int C4) {
+  if (!L.ok()) return;
+  EDV_DISPATCH_T(dtype, { geglu_pair_kernel<T><<<nblk(M * C4, 256), 256, 0, L.stream>>>((const T*)hg, (T*)out, M, C4); });
+  L.check("geglu");
+}
+
+// out[m] = x[m] . w[0..C-1] + w[C], then ReLU (sig_sign == 0) or sigmoid(sig_sign * .) (CUDA-core disparity head)
+inline void head_dot(Launch& L, int dtype, const void* x, const float* w, float* out, long long M, int C, float sig_sign) {
+  if (!L.ok()) return;
+  EDV_DISPATCH_T(dtype, {
+    head_dot_kernel<T><<<nblk(M, 256), 256, 0, L.stream>>>((const T*)x, w, out, M, C, sig_sign == 0.f, sig_sign, sig_sign != 0.f);
+  });
+  L.check("head_dot");
+}
+
 }  // namespace edv

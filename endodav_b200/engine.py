@@ -16,7 +16,7 @@ DTYPES = {"fp32": EDV_F32, "f32": EDV_F32, "float32": EDV_F32, "bf16": EDV_BF16,
           "fp16": EDV_F16, "f16": EDV_F16, "float16": EDV_F16}
 TORCH_DTYPE = {EDV_F32: torch.float32, EDV_BF16: torch.bfloat16, EDV_F16: torch.float16}
 
-ABI_VERSION = 13   # must equal EDV_ABI_VERSION of include/endodav_b200.h (argtypes below are mirrored by hand)
+ABI_VERSION = 14   # must equal EDV_ABI_VERSION of include/endodav_b200.h (argtypes below are mirrored by hand)
 
 EXPORTS = [
     "edv_abi_version", "edv_create", "edv_destroy", "edv_last_error", "edv_set_weight", "edv_plan", "edv_forward", "edv_forward_u8",
@@ -25,6 +25,8 @@ EXPORTS = [
     "edv_op_resize_f32", "edv_profile", "edv_profile_reset", "edv_profile_collect", "edv_profile_get",
     "edv_op_disp_head", "edv_op_cubic_resize_u8", "edv_op_stitch_window", "edv_op_stitch_plan",
     "edv_op_disp_to_depth", "edv_op_compute_errors", "edv_op_attention_timeline", "edv_op_linear_timeline", "edv_op_linear_residual_ln",
+    "edv_op_preprocess_patches", "edv_op_tokens_to_patches", "edv_op_rowln_act", "edv_op_resblock_add", "edv_op_im2col3x3",
+    "edv_op_geglu_pair", "edv_op_head_dot",
 ]
 
 
@@ -114,7 +116,7 @@ def load_library():
     lib.edv_op_linear_residual_ln.argtypes = [ci, vp, vp, vp, vp, vp, vp, ctypes.c_float, vp, ci, ci, ci, vp, vp]
     lib.edv_op_linear_timeline.argtypes = [ci, vp, vp, vp, vp, ci, ci, ci, ci, vp, vp]
     lib.edv_op_attention_timeline.argtypes = [ci, vp, vp, ci, ci, ci, vp, vp]
-    lib.edv_op_temporal_attention.argtypes = [ci, vp, vp, ci, ci, ci, ci, vp]
+    lib.edv_op_temporal_attention.argtypes = [ci, vp, vp, ci, ci, ci, ci, vp, ctypes.c_char_p, ci, vp]
     lib.edv_op_disp_head.argtypes = [ci, vp, vp, vp, vp, vp, ci, ci, ci, ci, ci, ci, ctypes.c_float, vp]
     lib.edv_op_cubic_resize_u8.argtypes = [vp, vp, ci, ci, ci, ci, ci, vp]
     lib.edv_op_stitch_window.argtypes = [vp, ci, ci, ci, vp, vp, ci, vp, vp, vp]
@@ -122,7 +124,15 @@ def load_library():
     lib.edv_op_disp_to_depth.argtypes = [vp, vp, vp, ctypes.c_longlong, ctypes.c_double, ctypes.c_double, vp]
     lib.edv_op_compute_errors.argtypes = [vp, vp, vp, ci, ctypes.c_longlong, ctypes.c_float, ctypes.c_float, ctypes.c_float,
                                           ctypes.c_float, ctypes.c_float, vp, vp]
-    lib.edv_op_layernorm.argtypes = [ci, vp, vp, vp, vp, ci, ci, ctypes.c_float, vp]
+    lib.edv_op_layernorm.argtypes = [ci, vp, vp, vp, vp, ci, ci, ctypes.c_float, ci, ci, vp, ci, ci, vp]
+    ll, cf = ctypes.c_longlong, ctypes.c_float
+    lib.edv_op_preprocess_patches.argtypes = [ci, vp, ci, vp, ci, ci, ci, ci, ci, ci, vp]
+    lib.edv_op_tokens_to_patches.argtypes = [ci, vp, vp, ll, ci, ci, ci, vp]
+    lib.edv_op_rowln_act.argtypes = [ci, vp, vp, vp, vp, ll, ci, ci, cf, ci, vp]
+    lib.edv_op_resblock_add.argtypes = [ci, vp, vp, vp, vp, ll, ci, ci, cf, ci, vp]
+    lib.edv_op_im2col3x3.argtypes = [ci, vp, vp, ci, ci, ci, ci, ci, vp]
+    lib.edv_op_geglu_pair.argtypes = [ci, vp, vp, ll, ci, vp]
+    lib.edv_op_head_dot.argtypes = [ci, vp, vp, vp, ll, ci, cf, vp]
     lib.edv_op_groupnorm.argtypes = [ci, vp, vp, vp, vp, ci, ci, ci, ctypes.c_float, vp]
     lib.edv_op_upsample.argtypes = [ci, vp, vp, ci, ci, ci, ci, ci, ci, vp]
     lib.edv_op_resize_f32.argtypes = [vp, vp, ci, ci, ci, ci, ci, vp]
@@ -402,11 +412,20 @@ def op_attention_timeline(qkv, F, S, heads):
     return out, tl
 
 
-def op_temporal_attention(qkv, B, T, hw, C):
+def op_temporal_attention_kernel(qkv, B, T, hw, C, rope=None, out=None):
+    """-> (out [B*T*hw, C], name of the kernel instance that ran).  rope: float32 [T, C] = [T][C/2] (cos, sin) pairs
+    (pack.py), or None."""
     lib = load_library()
-    out = torch.empty(B * T * hw, C, dtype=qkv.dtype, device=qkv.device)
-    _check(lib.edv_op_temporal_attention(_dt(qkv), _ptr(qkv), _ptr(out), B, T, hw, C, _stream()), None, "edv_op_temporal_attention")
-    return out
+    if out is None:
+        out = torch.empty(B * T * hw, C, dtype=qkv.dtype, device=qkv.device)
+    name = ctypes.create_string_buffer(128)
+    _check(lib.edv_op_temporal_attention(_dt(qkv), _ptr(qkv), _ptr(out), B, T, hw, C, _ptr(rope), name, 128, _stream()), None,
+           "edv_op_temporal_attention")
+    return out, name.value.decode()
+
+
+def op_temporal_attention(qkv, B, T, hw, C, rope=None):
+    return op_temporal_attention_kernel(qkv, B, T, hw, C, rope)[0]
 
 
 def op_disp_head(X, Wt, bias, head_w, oh, ow, sig_sign=0.0):
@@ -430,13 +449,71 @@ def op_cubic_resize_u8(frames_u8, h, w, out=None):
     return out
 
 
-def op_layernorm(X, gamma, beta, eps, out_dtype):
+def op_layernorm(X, gamma, beta, eps, out_dtype, grp=0, skip=0, add=None, add_div=1, add_mod=1, out=None):
+    """LayerNorm of the rows of X (float32 [rows, D]) into out_dtype, with the row selection grp / skip and the additive
+    per-frame table add of edv_op_layernorm.  out: optional [>= M, D] buffer (its first M rows are written)."""
     lib = load_library()
-    M, D = X.shape
-    Y = torch.empty(M, D, dtype=out_dtype, device=X.device)
-    _check(lib.edv_op_layernorm(_dt(Y), _ptr(X), _ptr(gamma), _ptr(beta), _ptr(Y), M, D, ctypes.c_float(eps), _stream()), None,
-           "edv_op_layernorm")
+    rows, D = X.shape
+    M = rows if grp == 0 else (rows // grp) * (grp - skip if skip >= 0 else -skip)
+    Y = out if out is not None else torch.empty(M, D, dtype=out_dtype, device=X.device)
+    _check(lib.edv_op_layernorm(_dt(Y), _ptr(X), _ptr(gamma), _ptr(beta), _ptr(Y), M, D, ctypes.c_float(eps), grp, skip, _ptr(add),
+                                add_div, add_mod, _stream()), None, "edv_op_layernorm")
     return Y
+
+
+def op_preprocess_patches(frames, h, w, out, normalize=True):
+    """frames float32 [F,3,H,W] or uint8 [F,H,W,3] (at h x w) -> out [F*(h/14)*(w/14), 640] (out's dtype)."""
+    lib = load_library()
+    u8 = frames.dtype == torch.uint8
+    Fr, H, W = (frames.shape[0], frames.shape[1], frames.shape[2]) if u8 else (frames.shape[0], frames.shape[2], frames.shape[3])
+    _check(lib.edv_op_preprocess_patches(_dt(out), _ptr(frames), int(u8), _ptr(out), Fr, H, W, h, w, int(normalize), _stream()), None,
+           "edv_op_preprocess_patches")
+    return out
+
+
+def op_tokens_to_patches(x, out, Mp, P, D, cls):
+    """out [Mp, D] (out's dtype) = the patch rows of the float32 token stream x [Mp/P, P + cls, D]."""
+    lib = load_library()
+    _check(lib.edv_op_tokens_to_patches(_dt(out), _ptr(x), _ptr(out), Mp, P, D, cls, _stream()), None, "edv_op_tokens_to_patches")
+    return out
+
+
+def op_rowln_act(x, gamma, beta, y, M, C, Cr, eps=1e-6, gelu=True):
+    """y [M, C] = GELU(LayerNorm over the first Cr channels of x [M, C]), padding columns 0 (x's dtype)."""
+    lib = load_library()
+    _check(lib.edv_op_rowln_act(_dt(x), _ptr(x), _ptr(gamma), _ptr(beta), _ptr(y), M, C, Cr, ctypes.c_float(eps), int(gelu), _stream()),
+           None, "edv_op_rowln_act")
+    return y
+
+
+def op_resblock_add(x, r, gamma, beta, Mp, P, D, cls, eps=1e-6):
+    """x (float32 token stream, in place): patch rows += LayerNorm(r [Mp, D]) (r's dtype)."""
+    lib = load_library()
+    _check(lib.edv_op_resblock_add(_dt(r), _ptr(x), _ptr(r), _ptr(gamma), _ptr(beta), Mp, P, D, ctypes.c_float(eps), cls, _stream()),
+           None, "edv_op_resblock_add")
+    return x
+
+
+def op_im2col3x3(x, out, stride=2):
+    """NHWC x [F,H,W,C] -> out [F*OH*OW, 9*C] (3x3, pad 1, (ky,kx,c) order)."""
+    lib = load_library()
+    Fr, H, W, C = x.shape
+    _check(lib.edv_op_im2col3x3(_dt(x), _ptr(x), _ptr(out), Fr, H, W, C, stride, _stream()), None, "edv_op_im2col3x3")
+    return out
+
+
+def op_geglu_pair(hg, out, M, C4):
+    """out [M, C4] = value * gelu(gate) of hg [M, 2*C4] in [64 value | 64 gate] column blocks (hg's dtype)."""
+    lib = load_library()
+    _check(lib.edv_op_geglu_pair(_dt(hg), _ptr(hg), _ptr(out), M, C4, _stream()), None, "edv_op_geglu_pair")
+    return out
+
+
+def op_head_dot(x, w, out, M, C, sig_sign=0.0):
+    """out [M] float32 = x [M, C] . w[:C] + w[C], then ReLU (sig_sign 0) or sigmoid(sig_sign * .)."""
+    lib = load_library()
+    _check(lib.edv_op_head_dot(_dt(x), _ptr(x), _ptr(w), _ptr(out), M, C, ctypes.c_float(sig_sign), _stream()), None, "edv_op_head_dot")
+    return out
 
 
 def op_groupnorm(X, gamma, beta, eps):

@@ -30,7 +30,7 @@ typedef struct edv_ctx edv_ctx;
 /* Bumped whenever an entry point's argument list or a struct layout changes.  The ctypes host
  * (endodav_b200/engine.py) mirrors the signatures by hand, so it refuses a library whose
  * edv_abi_version() differs from its own constant instead of calling it with a stale layout. */
-#define EDV_ABI_VERSION 13
+#define EDV_ABI_VERSION 14
 int edv_abi_version(void);
 
 enum edv_status {
@@ -213,9 +213,13 @@ int edv_op_attention_timeline(int dtype, const void* qkv, void* out, int F, int 
 
 /* Temporal attention over the frame axis: qkv [B*T*hw, 3C] (q pre-scaled by hd^-0.5) ->
  * out [B*T*hw, C]; 8 heads; one softmax per (clip, position, head) over T<=32 frames.
+ * rope (may be NULL: no rotation): [T][C/2] (cos, sin) float pairs as pack.py writes them; channel pair i of q and k at
+ * frame f is rotated by rope[f][i] before the scores (pe='rope').  `kernel` (may be NULL) receives the instance that ran,
+ * e.g. "temporal_attention_mma<HD=24,PB=2>" (16-bit) or "temporal_attention_simt<HD=24,PB=4,HG=8>" (float32).
  * Replaces: TemporalAttention/CrossAttention._attention (motion_module.py:232-295;
- * motion_module/attention.py:182-211). */
-int edv_op_temporal_attention(int dtype, const void* qkv, void* out, int B, int T, int hw, int C, void* stream);
+ * motion_module/attention.py:182-211, 403-429). */
+int edv_op_temporal_attention(int dtype, const void* qkv, void* out, int B, int T, int hw, int C, const float* rope, char* kernel,
+                              int kernel_cap, void* stream);
 
 /* Fused disparity-head tail on an NHWC map X[F,H1,W1,Cin] (16-bit, Cin in {32,128}):
  * bilinear resize (align_corners=True) to (OH,OW) -> 3x3 conv Wt[32, 9*Cin] + bias -> ReLU ->
@@ -229,9 +233,51 @@ int edv_op_disp_head(int dtype, const void* X, const void* Wt, const float* bias
  * centres, replicated border).  Replaces endodav.py:195 + util/transform.py:109-113,139-158. */
 int edv_op_cubic_resize_u8(const uint8_t* src, float* dst, int N, int H, int W, int h, int w, void* stream);
 
-/* LayerNorm over the last dim: X[M,D] float32 -> Y[M,D] `dtype`. */
-int edv_op_layernorm(int dtype, const float* X, const float* gamma, const float* beta, void* Y, int M, int D,
-                     float eps, void* stream);
+/* LayerNorm over the last dim: X float32 -> Y[M,D] `dtype` (M output rows), then + add[(m / add_div) % add_mod][0..D-1]
+ * when add is not NULL (the temporal modules' sinusoidal PE of row m's frame: add_div = hw, add_mod = T).
+ * grp = 0: X is [M,D] (skip must be 0).  grp > 0: X holds groups of grp rows (one frame of tokens) and
+ *   skip > 0 drops the first `skip` rows of every group from the compact output (the final norm on the taps without the
+ *   cls row: output row m reads X row (m / (grp - skip)) * grp + skip + m % (grp - skip));
+ *   skip < 0 keeps only the first -skip rows of every group (the cls row alone for the use_clstoken readout, skip = -1). */
+int edv_op_layernorm(int dtype, const float* X, const float* gamma, const float* beta, void* Y, int M, int D, float eps, int grp,
+                     int skip, const float* add, int add_div, int add_mod, void* stream);
+
+/* The forward's glue kernels, each through the launcher the forward calls (launch geometry included).  Every call
+ * rejects with EDV_ERR_ARG a shape its kernel cannot handle; vector-accessed pointers must be 16-byte aligned. */
+
+/* Patch embedding input: src float32 [F,3,H,W] in [0,1] (u8 = 0; bilinearly resized, align_corners=True, to h x w) or
+ * uint8 [F,H,W,3] with H = h, W = w (u8 = 1: x / 255), ImageNet-normalised unless normalize = 0, unfolded into 14 x 14
+ * patches: out [F*(h/14)*(w/14), 640] `dtype`, column c*196 + ky*14 + kx, columns 588..639 zero.
+ * Replaces endodav.py:153,155 + patch_embed.py:75-77. */
+int edv_op_preprocess_patches(int dtype, const void* src, int u8, void* out, int F, int H, int W, int h, int w, int normalize,
+                              void* stream);
+
+/* Patch rows of the float32 residual stream x [Mp/P][P + cls][D] -> out [Mp, D] `dtype` (cls = 1: the frame's row 0 is
+ * skipped).  The input of ResBottleneckBlock (block.py:146-150).  D % 4 == 0. */
+int edv_op_tokens_to_patches(int dtype, const float* x, void* out, long long Mp, int P, int D, int cls, void* stream);
+
+/* Channels-first LayerNorm of ResBottleneckBlock on NHWC rows: y[M,C] = GELU (gelu = 1, exact erf) of the LayerNorm over
+ * the first Cr of the C channels of x[M,C] (`dtype`), columns Cr..C-1 of y written as 0 and those of x never read.
+ * Replaces layers/utils.py:171-179 + the block's act. */
+int edv_op_rowln_act(int dtype, const void* x, const float* gamma, const float* beta, void* y, long long M, int C, int Cr, float eps,
+                     int gelu, void* stream);
+
+/* x (float32 residual stream [Mp/P][P + cls][D], in place): patch row p of each frame += LayerNorm(r[p]) (r [Mp,D]
+ * `dtype`); cls rows are not touched.  The residual add of ResBottleneckBlock (block.py:146-150). */
+int edv_op_resblock_add(int dtype, float* x, const void* r, const float* gamma, const float* beta, long long Mp, int P, int D, float eps,
+                        int cls, void* stream);
+
+/* 3x3 pad-1 im2col of an NHWC map x [F,H,W,C] at `stride` (1 or 2): out [F*OH*OW, 9*C] in (ky,kx,c) order,
+ * OH = (H-1)/stride + 1.  C % 8 == 0.  The operand of resize_layers[3] (dpt.py:85-90) on the tensor-core path. */
+int edv_op_im2col3x3(int dtype, const void* x, void* out, int F, int H, int W, int C, int stride, void* stream);
+
+/* GEGLU on the CUDA-core path: out [M, C4] = value * gelu(gate) (exact erf) of hg [M, 2*C4] laid out by pack.py in
+ * column blocks of 128 = [64 value | 64 gate].  C4 % 64 == 0.  Replaces attention.py:382-384. */
+int edv_op_geglu_pair(int dtype, const void* hg, void* out, long long M, int C4, void* stream);
+
+/* Disparity-head 1x1 on the CUDA-core path: out[m] (float32) = x[m,0..C-1] . w[0..C-1] + w[C], then ReLU (sig_sign = 0)
+ * or sigmoid(sig_sign * .).  C % 8 == 0.  Replaces dpt.py:121-123; layers.py:211-217. */
+int edv_op_head_dot(int dtype, const void* x, const float* w, float* out, long long M, int C, float sig_sign, void* stream);
 
 /* GroupNorm(32 groups) over NHWC X[F,hw,C] (`dtype`) -> Y same layout.
  * Replaces: TemporalTransformer3DModel.norm (motion_module.py:84,110). */

@@ -89,6 +89,19 @@ def test_forward_fp32_matches_reference_golden(name):
 @pytest.mark.parametrize("dtype", ["bf16", "fp16"])
 @pytest.mark.parametrize("name", FWD)
 def test_forward_16bit_within_tolerance(name, dtype):
+    _check_16bit(name, dtype)
+
+
+@pytest.mark.parametrize("dtype", ["bf16", "fp16"])
+@pytest.mark.parametrize("name", ["fwd_vits_lora_res_convhead", "fwd_vits_rope"])
+def test_forward_16bit_cuda_core_engine_within_tolerance(name, dtype, monkeypatch):
+    """The same gates on the CUDA-core 16-bit engine (ENDODAV_ENGINE=simt), the only product path that runs
+    geglu_pair, head_dot and the unfused disparity head in 16 bits."""
+    monkeypatch.setenv("ENDODAV_ENGINE", "simt")
+    _check_16bit(name, dtype, "simt")
+
+
+def _check_16bit(name, dtype, engine="tc"):
     m, arrays = load_case(name)
     model, cfg, sd = _build(m["ctor"], m["weight_seed"], dtype)
     B, T, H, W = m["input"]
@@ -113,7 +126,7 @@ def test_forward_16bit_within_tolerance(name, dtype):
         g = subsample_like_golden(name, s, out[("disp", s)].cpu().numpy())
         r = arrays["disp%d" % s]
         assert _rel(g, r).max() <= gate["rel"], (name, dtype, s)
-    _report_16bit(name, dtype, float(rel.max()), absrel, a1, gate["rel"])
+    _report_16bit(name, dtype if engine == "tc" else dtype + "." + engine, float(rel.max()), absrel, a1, gate["rel"])
 
 
 def test_stage_taps_fp32_match_oracle():
@@ -246,27 +259,29 @@ def test_cuda_graph_replay_on_default_stream_is_bit_identical():
     x = weights.make_frames(B, T, H, W, m["frame_seed"]).cuda()
     h, w = m["ctor"]["image_shape"]
     eng = model._ensure_engine(h // 14, w // 14)
+    def pyramid(inp):   # all four levels: a replay hands them over with one copy_pyramid_kernel launch
+        o = model(inp)
+        return [o[("disp", s)].clone() for s in range(4)]
+
     eng.set_graph_mode(False)
-    eager = model(x)[("disp", 0)].clone()
+    eager = pyramid(x)
     assert eng.graph_count() == 0
     eng.set_graph_mode(True)
-    outs = []
-    for _ in range(4):
-        o = model(x)
-        outs.append(o[("disp", 0)].clone())
-        del o
+    outs = [pyramid(x) for _ in range(4)]
     assert eng.graph_count() >= 1, eng.graph_status()
     assert eng.graph_status() == "ok"
     for o in outs:
-        assert torch.equal(o, eager)
+        for s in range(4):
+            assert torch.equal(o[s], eager[s]), s
     x2 = weights.make_frames(B, T, H, W, m["frame_seed"] + 1).cuda()
     eng.set_graph_mode(False)
-    eager2 = model(x2)[("disp", 0)].clone()
+    eager2 = pyramid(x2)
     eng.set_graph_mode(True)
     model(x)
     x.copy_(x2)           # same pointer, new values
     for _ in range(3):
-        got2 = model(x)[("disp", 0)].clone()
+        got2 = pyramid(x)
     assert eng.graph_count() >= 1
-    assert torch.equal(got2, eager2)
-    assert not torch.equal(got2, eager)
+    for s in range(4):
+        assert torch.equal(got2[s], eager2[s]), s
+    assert not torch.equal(got2[0], eager[0])

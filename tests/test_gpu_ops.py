@@ -148,13 +148,73 @@ def _tattn_ref(qkv, B, T, hw, C):
     return o.permute(0, 3, 1, 2, 4).reshape(B * T * hw, C).float()
 
 
+def _rope_table(T, C):
+    """pack.py's RoPE table [T][C/2] (cos, sin) as float32 [T, C], followed by T NaN guard rows in the same allocation."""
+    freqs = 1.0 / (10000.0 ** (torch.arange(0, C, 2, dtype=torch.float64)[: C // 2] / C))
+    ang = torch.outer(torch.arange(T, dtype=torch.float64), freqs)
+    tab = torch.full((2 * T, C), float("nan"), dtype=torch.float32)
+    tab[:T] = torch.stack([ang.cos(), ang.sin()], -1).reshape(T, C).float()
+    return tab.to(DEV)
+
+
+def _rope_apply(qkv, B, T, hw, C, tab, dtype):
+    """q and k of every row rotated in float64 by the (float32) table row of its frame; the tensor-core kernel rounds
+    the rotated q and k to the 16-bit dtype, so the reference does too."""
+    t = qkv.double().reshape(B, T, hw, 3, C // 2, 2).clone()
+    cs = tab[:T].double().reshape(1, T, 1, C // 2, 2)
+    c, s = cs[..., 0], cs[..., 1]
+    for w in (0, 1):
+        a, b = t[:, :, :, w, :, 0].clone(), t[:, :, :, w, :, 1].clone()
+        t[:, :, :, w, :, 0] = a * c - b * s
+        t[:, :, :, w, :, 1] = a * s + b * c
+    t = t.reshape(B * T * hw, 3 * C)
+    if dtype != torch.float32:
+        t[:, : 2 * C] = t[:, : 2 * C].to(dtype).double()
+    return t
+
+
+def _ta_instance(dtype, T, hw, C):
+    """The instance attention.cu launches: tensor-core PB from ta_smem_per_pos (<= 96 KB per CTA), CUDA-core PB / HG
+    from the 64 KB staging budget of launch_temporal."""
+    hd = C // 8
+    if dtype != torch.float32:
+        per = 3 * 32 * (8 * hd + 8) * 2
+        pb = 4 if 4 * per <= 96 * 1024 and hw >= 4 else 2 if 2 * per <= 96 * 1024 and hw >= 2 else 1
+        return "temporal_attention_mma<HD=%d,PB=%d>" % (hd, pb)
+    per, hg, mt = T * hd * 12, 8, 256 if hd >= 64 else 512
+    while hg > 1 and hg * per > 64 * 1024:
+        hg >>= 1
+    pb = min(4, max(1, (64 * 1024) // (hg * per)))
+    while pb > 1 and 32 * hg * pb > mt:
+        pb -= 1
+    while hg > 1 and 32 * hg * pb > mt:
+        hg >>= 1
+    return "temporal_attention_simt<HD=%d,PB=%d,HG=%d>" % (hd, min(pb, hw), hg)
+
+
+# every head dim the forward plans (8, 24, 32, 48, 128) at T up to 32 (the second 16-query m-tile starts at T = 17), B = 2,
+# hw with a tail of the PB = 4 (HD 8) / PB = 2 (HD 24) instances
+TA_SHAPES = [pytest.param(B, T, hw, C, False, id="%d-%d-%d-%d" % (B, T, hw, C))
+             for B, T, hw, C in [(1, 32, 320, 192), (2, 8, 80, 384), (1, 32, 100, 64), (3, 5, 7, 64), (1, 1, 9, 192), (1, 16, 30, 256),
+                                 (1, 32, 12, 1024)]]
+TA_SHAPES += [pytest.param(2, T, hw, 8 * hd, rope, id="2-%d-%d-%d-%s" % (T, hw, 8 * hd, "rope" if rope else "ape"))
+              for hd, hw in ((8, 7), (24, 5), (32, 3), (48, 2), (128, 3)) for T in (1, 5, 16, 17, 32) for rope in (False, True)]
+
+
 @pytest.mark.parametrize("dtype", [torch.float32] + DT16)
-@pytest.mark.parametrize("B,T,hw,C", [(1, 32, 320, 192), (2, 8, 80, 384), (1, 32, 100, 64), (3, 5, 7, 64), (1, 1, 9, 192),
-                                       (1, 16, 30, 256), (1, 32, 12, 1024)])
-def test_temporal_attention(dtype, B, T, hw, C):
+@pytest.mark.parametrize("B,T,hw,C,rope", TA_SHAPES)
+def test_temporal_attention(dtype, B, T, hw, C, rope):
     qkv = _rand((B * T * hw, 3 * C), dtype, 11, 0.7)
-    got = eng.op_temporal_attention(qkv, B, T, hw, C)
-    _close(got, _tattn_ref(qkv, B, T, hw, C), dtype, "temporal attention %s" % dtype, slack=4.0)
+    tab = _rope_table(T, C) if rope else None
+    got, kernel = eng.op_temporal_attention_kernel(qkv, B, T, hw, C, tab)
+    assert kernel == _ta_instance(dtype, T, hw, C)
+    ref_in = _rope_apply(qkv, B, T, hw, C, tab, dtype) if rope else qkv
+    _close(got, _tattn_ref(ref_in, B, T, hw, C), dtype, "temporal attention %s" % dtype, slack=4.0)
+    if rope:
+        # the identity rotation (cos 1, sin 0) must leave q and k bit for bit as they are
+        ident = torch.zeros(T, C, dtype=torch.float32, device=DEV)
+        ident[:, 0::2] = 1.0
+        assert torch.equal(eng.op_temporal_attention_kernel(qkv, B, T, hw, C, ident)[0], eng.op_temporal_attention(qkv, B, T, hw, C))
 
 
 # ---- norms ------------------------------------------------------------------------------------
