@@ -11,11 +11,16 @@ void attention(Launch& L, int dtype, int engine, const void* qkv, void* out, int
   if (!L.ok()) return;
   // QK^T + PV: 4*S*S*64 per (frame, head); q,k,v read once, o written once
   L.note(4.0 * F * heads * (double)S * S * 64, 4.0 * F * S * heads * 64 * dtype_size(dtype));
+  const char* tname = dtype == EDV_F32 ? "f32" : dtype == EDV_BF16 ? "bf16" : "f16";
   if (dtype != EDV_F32 && engine == EDV_ENGINE_TC) {
+    L.kernel = std::string("flash_attention_tc<") + tname + ">";
     if (dtype == EDV_BF16) tc::launch_attention_tc<bf16>(L, dtype, qkv, out, F, S, heads, timeline);
     else tc::launch_attention_tc<f16>(L, dtype, qkv, out, F, S, heads, timeline);
     return;
   }
+  // CUDA-core kernel: every fp32 call (there is no fp32 tensor-core kernel, whatever the engine) and EDV_ENGINE_SIMT
+  if (heads > 65535 || F > 65535) return L.fail(EDV_ERR_ARG, "spatial_attention_simt: heads and F must be at most 65535 (grid y / z)");
+  L.kernel = std::string("spatial_attention_simt<") + tname + ">";
   dim3 grid((S + 127) / 128, heads, F);
   EDV_DISPATCH_T(dtype, { spatial_attention_simt_kernel<T><<<grid, 128, 0, L.stream>>>((const T*)qkv, (T*)out, S, heads); });
   L.check("spatial_attention_simt");

@@ -1248,10 +1248,19 @@ int edv_op_linear_residual_ln(int dtype, const void* A, const void* W, const flo
   return finish(L);
 }
 
-int edv_op_attention(int dtype, int engine, const void* qkv, void* out, int F, int S, int heads, void* stream) {
+int edv_op_attention(int dtype, int engine, const void* qkv, void* out, int F, int S, int heads, char* kernel, int kernel_cap,
+                     void* stream) {
+  if (kernel && kernel_cap > 0) kernel[0] = 0;
+  if (dtype < EDV_F32 || dtype > EDV_F16) return set_err(nullptr, EDV_ERR_ARG, "edv_op_attention: bad dtype %d", dtype);
+  if (engine != EDV_ENGINE_TC && engine != EDV_ENGINE_SIMT) return set_err(nullptr, EDV_ERR_ARG, "edv_op_attention: bad engine %d", engine);
+  if (!qkv || !out) return set_err(nullptr, EDV_ERR_ARG, "edv_op_attention: null qkv or out");
+  if (F < 1 || S < 1 || heads < 1) return set_err(nullptr, EDV_ERR_ARG, "edv_op_attention: F, S and heads must be at least 1");
+  // the tensor map's base address (TMA) and the 16-byte vector loads / stores of both kernels
+  if (!aligned16(qkv) || !aligned16(out)) return set_err(nullptr, EDV_ERR_ARG, "edv_op_attention: qkv and out must be 16-byte aligned");
   Launch L;
   L.stream = (cudaStream_t)stream;
   attention(L, dtype, engine, qkv, out, F, S, heads);
+  if (kernel && kernel_cap > 0) snprintf(kernel, kernel_cap, "%s", L.kernel.c_str());
   return finish(L);
 }
 

@@ -16,7 +16,7 @@ DTYPES = {"fp32": EDV_F32, "f32": EDV_F32, "float32": EDV_F32, "bf16": EDV_BF16,
           "fp16": EDV_F16, "f16": EDV_F16, "float16": EDV_F16}
 TORCH_DTYPE = {EDV_F32: torch.float32, EDV_BF16: torch.bfloat16, EDV_F16: torch.float16}
 
-ABI_VERSION = 14   # must equal EDV_ABI_VERSION of include/endodav_b200.h (argtypes below are mirrored by hand)
+ABI_VERSION = 15  # must equal EDV_ABI_VERSION of include/endodav_b200.h (argtypes below are mirrored by hand)
 
 EXPORTS = [
     "edv_abi_version", "edv_create", "edv_destroy", "edv_last_error", "edv_set_weight", "edv_plan", "edv_forward", "edv_forward_u8",
@@ -112,7 +112,7 @@ def load_library():
                                     ctypes.POINTER(ctypes.c_longlong), ctypes.POINTER(ctypes.c_double),
                                     ctypes.POINTER(ctypes.c_double)]
     lib.edv_op_gemm.argtypes = [ci, ci, ctypes.POINTER(EdvGemmDesc), ctypes.c_char_p, ci, vp]
-    lib.edv_op_attention.argtypes = [ci, ci, vp, vp, ci, ci, ci, vp]
+    lib.edv_op_attention.argtypes = [ci, ci, vp, vp, ci, ci, ci, ctypes.c_char_p, ci, vp]
     lib.edv_op_linear_residual_ln.argtypes = [ci, vp, vp, vp, vp, vp, vp, ctypes.c_float, vp, ci, ci, ci, vp, vp]
     lib.edv_op_linear_timeline.argtypes = [ci, vp, vp, vp, vp, ci, ci, ci, ci, vp, vp]
     lib.edv_op_attention_timeline.argtypes = [ci, vp, vp, ci, ci, ci, vp, vp]
@@ -395,11 +395,20 @@ def op_conv3x3(X, Wt, bias=None, relu_out=False, engine=ENGINE_TC):
     return Y
 
 
-def op_attention(qkv, F, S, heads, engine=ENGINE_TC):
+def op_attention_kernel(qkv, F, S, heads, engine=ENGINE_TC, out=None):
+    """-> (out [F*S, heads*64], name of the kernel instance that ran, e.g. "flash_attention_tc<bf16>").  out: optional
+    caller-owned buffer whose first F*S rows receive the result."""
     lib = load_library()
-    out = torch.empty(F * S, heads * 64, dtype=qkv.dtype, device=qkv.device)
-    _check(lib.edv_op_attention(_dt(qkv), engine, _ptr(qkv), _ptr(out), F, S, heads, _stream()), None, "edv_op_attention")
-    return out
+    if out is None:
+        out = torch.empty(F * S, heads * 64, dtype=qkv.dtype, device=qkv.device)
+    name = ctypes.create_string_buffer(128)
+    _check(lib.edv_op_attention(_dt(qkv), engine, _ptr(qkv), _ptr(out), F, S, heads, name, 128, _stream()), None,
+           "edv_op_attention")
+    return out, name.value.decode()
+
+
+def op_attention(qkv, F, S, heads, engine=ENGINE_TC):
+    return op_attention_kernel(qkv, F, S, heads, engine)[0]
 
 
 def op_attention_timeline(qkv, F, S, heads):

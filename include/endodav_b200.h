@@ -30,7 +30,7 @@ typedef struct edv_ctx edv_ctx;
 /* Bumped whenever an entry point's argument list or a struct layout changes.  The ctypes host
  * (endodav_b200/engine.py) mirrors the signatures by hand, so it refuses a library whose
  * edv_abi_version() differs from its own constant instead of calling it with a stale layout. */
-#define EDV_ABI_VERSION 14
+#define EDV_ABI_VERSION 15
 int edv_abi_version(void);
 
 enum edv_status {
@@ -202,8 +202,13 @@ int edv_op_linear_residual_ln(int dtype, const void* A, const void* W, const flo
                               const float* beta, float eps, void* xn_out, int M, int N, int K, long long* timeline_dev, void* stream);
 
 /* Spatial multi-head attention over token-major qkv [F*S, 3*heads*64] (q pre-scaled) ->
- * out [F*S, heads*64].  Replaces: Attention.forward's softmax(qk^T)v (attention.py:60-66). */
-int edv_op_attention(int dtype, int engine, const void* qkv, void* out, int F, int S, int heads, void* stream);
+ * out [F*S, heads*64].  16-bit with EDV_ENGINE_TC runs the tcgen05 kernel; float32 (under either engine) and
+ * EDV_ENGINE_SIMT run the CUDA-core kernel.  `kernel` (may be NULL) receives the instance that ran, e.g.
+ * "flash_attention_tc<bf16>" or "spatial_attention_simt<f32>".  EDV_ERR_ARG for a NULL or not 16-byte aligned qkv / out,
+ * F, S or heads below 1, an unknown dtype or engine, and heads or F above 65535 on the CUDA-core kernel.
+ * Replaces: Attention.forward's softmax(qk^T)v (attention.py:60-66). */
+int edv_op_attention(int dtype, int engine, const void* qkv, void* out, int F, int S, int heads, char* kernel, int kernel_cap,
+                     void* stream);
 
 /* edv_op_attention (tcgen05 kernel, 16-bit dtypes) that also records the kernel's own timeline: timeline_dev gets
  * 8 CTAs x 64 clock64 stamps (entry, setup, per-iteration softmax / MMA-issue times; slot table in

@@ -347,8 +347,15 @@ COVERED = {
     "resize_f32_kernel": ["test_gpu_ops::test_resize_f32"],
     "temporal_attention_mma_kernel": ["test_gpu_ops::test_temporal_attention"],
     "temporal_attention_kernel": ["test_gpu_ops::test_temporal_attention"],
-    "spatial_attention_simt_kernel": ["test_gpu_ops::test_attention_fp32", "test_gpu_ops::test_attention_16bit"],
-    "flash_attention_tc_kernel": ["test_gpu_ops::test_attention_16bit"],
+    "spatial_attention_simt_kernel": ["test_gpu_ops::test_attention_fp32", "test_gpu_ops::test_attention_16bit",
+                                      "test_gpu_attention::test_attention_forward_shapes", "test_gpu_attention::test_attention_tails",
+                                      "test_gpu_attention::test_attention_frames_are_independent",
+                                      "test_gpu_attention::test_attention_poisoned_neighbour",
+                                      "test_gpu_attention::test_attention_lazy_rescale"],
+    "flash_attention_tc_kernel": ["test_gpu_ops::test_attention_16bit", "test_gpu_attention::test_attention_forward_shapes",
+                                  "test_gpu_attention::test_attention_tails", "test_gpu_attention::test_attention_frames_are_independent",
+                                  "test_gpu_attention::test_attention_poisoned_neighbour",
+                                  "test_gpu_attention::test_attention_lazy_rescale"],
     "gemm_simt_kernel": ["test_gpu_ops::test_linear_fp32", "test_gpu_epilogues::test_epilogue_matches_reference"],
     "gemm_tc_kernel": ["test_gpu_ops::test_linear_16bit", "test_gpu_epilogues::test_epilogue_matches_reference"],
     "gemm_bres_kernel": ["test_gpu_ops::test_linear_kernels_agree_bitwise", "test_gpu_epilogues::test_epilogue_matches_reference"],
