@@ -428,7 +428,7 @@ __global__ void __launch_bounds__(256) upsample_nhwc_kernel(const T* __restrict_
 // single-channel float32 bilinear resize (align_corners=True): disparity pyramid
 // (dpt_pyramid.py:95-97) and the final per-window resize (endodav.py:205).
 __global__ void resize_f32_kernel(const float* __restrict__ x, float* __restrict__ y, int F, int h, int w, int oh,
-                                  int ow, int sigmoid) {
+                                  int ow) {
   pdl_launch();
   pdl_wait();
   const long long total = (long long)F * oh * ow;
@@ -447,7 +447,6 @@ __global__ void resize_f32_kernel(const float* __restrict__ x, float* __restrict
   const float* b = x + (long long)f * h * w;
   float v = (1.f - ly) * ((1.f - lx) * b[(long long)y0 * w + x0] + lx * b[(long long)y0 * w + x1]) +
             ly * ((1.f - lx) * b[(long long)y1 * w + x0] + lx * b[(long long)y1 * w + x1]);
-  if (sigmoid) v = 1.f / (1.f + expf(-v));
   y[i] = v;
 }
 

@@ -27,7 +27,9 @@ struct WeightRef {
   size_t bytes;
 };
 
+// One workspace buffer.  `name` is empty when the plan's configuration does not need the buffer.
 struct Buf {
+  std::string name;
   size_t off = 0;
   size_t bytes = 0;
   int elem = 0;   // element size in bytes (4: float32 regardless of the activation dtype; 8: float2 statistics)
@@ -43,6 +45,11 @@ struct MMPlan {
   int C = 0, h = 0, w = 0;
 };
 
+// scratch of one temporal module (Fwd::motion); gg2 only on the CUDA-core engine
+struct MMScratch {
+  Buf stats, gn, hs, ln, qkv, att, gg, hsT, gg2;
+};
+
 struct Plan {
   bool valid = false;
   int B = 0, T = 0, H = 0, W = 0, h = 0, w = 0;
@@ -51,10 +58,27 @@ struct Plan {
   int ph2 = 0, pw2 = 0;
   int Cp[4] = {0, 0, 0, 0};
   int out_h[4] = {0, 0, 0, 0}, out_w[4] = {0, 0, 0, 0};
-  MMPlan mm[4];
+  MMPlan mod[4];            // geometry of temporal module j
+  // the path choices that decide which optional buffers exist; the forward follows them
+  bool tc = false;          // tensor-core engine (else CUDA-core)
+  bool fused_head = false;  // the disparity head runs as one kernel (head_fused.cuh): no head.up map
   size_t total = 0;
-  std::map<std::string, Buf> bufs;
-  std::map<std::string, DebugTap> taps;
+  // workspace buffers (edv_plan gives their layout order)
+  Buf A0, x, xn, qkv, ao, hid;             // hid: the MLP's hidden activations ("h")
+  Buf tap[4], tapc[4], rorb[4], tapr[4];   // final-norm taps; tapc / rorb / tapr: use_clstoken readout
+  Buf rb_pt, rb_t1, rb_t2, rb_t3;          // residual bottleneck blocks
+  Buf L1, L2, L3, L4p, L4, col, L3m, L4m;
+  MMScratch mm, mmb;                       // mmb: module 0, which runs on the side stream beside module 1
+  Buf lr[4], lrr[4];                       // layer{1-4}_rn outputs and their relu copies
+  Buf ref_tmp, ref_s, ref_sr, ref_u, ref_v;
+  Buf p4, p4m, p3, p3m, p2, p1;
+  Buf head_o1, head_up, head_t32;
+  Buf disp[4];
+  struct {
+    DebugTap tokens0, block0, tap[4], layer[4], mm[2], path4_pre, path3, path1;
+  } dbg;                                   // debug taps (planned with edv_set_debug on)
+  std::vector<Buf> bufs;                   // every planned buffer, for edv_plan_buffer
+  std::vector<DebugTap> taps;              // every debug tap, for edv_debug_tap
 };
 
 inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
@@ -75,7 +99,7 @@ struct GraphEntry {
   int u8 = 0, out_h = 0, out_w = 0;
   cudaGraphExec_t exec = nullptr;
   int launches = 0;
-  unsigned long long last_use = 0;
+  unsigned long long last_use = 0;   // graph_clock of the last replay (LRU eviction of graphs)
   bool same(const GraphEntry& o) const {
     return frames == o.frames && resized == o.resized && workspace == o.workspace && u8 == o.u8 && out_h == o.out_h && out_w == o.out_w;
   }
@@ -88,7 +112,6 @@ struct edv_ctx {
   std::string err;
   int last_launches = 0;
   int debug = 0;
-  int Kp = 640;
   // CUDA-graph replay of the planned forward (EDV_GRAPH=0 disables): up to GRAPH_SLOTS pointer sets per plan
   static constexpr int GRAPH_SLOTS = 32;
   int graph_mode = 1;
@@ -156,7 +179,7 @@ struct Fwd {
     L.stream = s;
     L.prof = &ctx->prof;
     dt = ctx->cfg.dtype;
-    eng = ctx->cfg.dtype == EDV_F32 ? EDV_ENGINE_SIMT : ctx->cfg.engine;
+    eng = ctx->plan.tc ? EDV_ENGINE_TC : EDV_ENGINE_SIMT;
     es = dtype_size(dt);
     par = ctx->branch_mode && !ctx->prof.on && !ctx->debug && ctx->ensure_side();
   }
@@ -176,13 +199,12 @@ struct Fwd {
   }
   bool tc() const { return eng == EDV_ENGINE_TC; }
 
-  void* buf(const char* name) {
-    auto it = c->plan.bufs.find(name);
-    if (it == c->plan.bufs.end()) {
-      L.fail(EDV_ERR_STATE, std::string("internal: unknown buffer ") + name);
-      return ws;
+  void* at(const Buf& b) {
+    if (b.name.empty()) {
+      L.fail(EDV_ERR_STATE, "internal: the forward reached a workspace buffer that its plan did not create");
+      return nullptr;
     }
-    return ws + it->second.off;
+    return ws + b.off;
   }
   const void* w(const std::string& name, size_t min_bytes = 0) {
     auto it = c->weights.find(name);
@@ -242,32 +264,32 @@ struct Fwd {
     e.out = out; e.ldo = ldo; e.bias = bias;
     return e;
   }
-  void snapshot(const char* name, const void* src, bool src_f32, long long rows, int cols_src, int cols) {
+  // debug tap t <- the first t.cols channels of t.rows rows of src (row pitch ld_src elements)
+  void snapshot(const DebugTap& t, const void* src, int ld_src, bool src_f32) {
     if (!c->debug || !L.ok()) return;
-    auto it = c->plan.taps.find(name);
-    if (it == c->plan.taps.end()) return;
-    float* dst = (float*)(ws + it->second.buf.off);
-    long long n = rows * cols;
-    if (src_f32) copy_channels_f32_kernel<float><<<nblk(n, 256), 256, 0, L.stream>>>((const float*)src, dst, rows, cols_src, cols);
-    else EDV_DISPATCH_T(dt, { copy_channels_f32_kernel<T><<<nblk(n, 256), 256, 0, L.stream>>>((const T*)src, dst, rows, cols_src, cols); });
+    float* dst = (float*)at(t.buf);
+    if (!dst) return;
+    long long n = t.rows * t.cols;
+    if (src_f32) copy_channels_f32_kernel<float><<<nblk(n, 256), 256, 0, L.stream>>>((const float*)src, dst, t.rows, ld_src, t.cols);
+    else EDV_DISPATCH_T(dt, { copy_channels_f32_kernel<T><<<nblk(n, 256), 256, 0, L.stream>>>((const T*)src, dst, t.rows, ld_src, t.cols); });
     L.check("debug snapshot");
   }
 
   // TemporalModule (motion_module.py:60-65,102-126,164-177): X [BT*hw, C] NHWC -> Y same
-  // `set`: scratch buffer family ("mm." on the main stream, "mmb." for the module that runs beside it on the side stream)
-  void motion(int j, const void* X, void* Y, const std::string& set = "mm.") {
+  // `s`: scratch family (mm on the main stream, mmb for the module that runs beside it on the side stream)
+  void motion(int j, const void* X, void* Y, const MMScratch& s) {
     const Plan& p = c->plan;
-    const int C = p.mm[j].C, hw = p.mm[j].h * p.mm[j].w, T = p.T, B = p.B;
+    const int C = p.mod[j].C, hw = p.mod[j].h * p.mod[j].w, T = p.T, B = p.B;
     const long long Mm = (long long)p.BT * hw;
     const std::string n = "mm" + std::to_string(j) + ".";
-    void* gnb = buf((set + "gn").c_str());
-    float* hs = (float*)buf((set + "hs").c_str());
-    void* lnb = buf((set + "ln").c_str());
-    void* qkvb = buf((set + "qkv").c_str());
-    void* att = buf((set + "att").c_str());
-    void* gg = buf((set + "gg").c_str());
-    void* hsT = buf((set + "hsT").c_str());
-    groupnorm(L, dt, X, wf(n + "gn.w", C), wf(n + "gn.b", C), gnb, (float2*)buf((set + "stats").c_str()), p.BT, hw, C, 1e-6f);
+    void* gnb = at(s.gn);
+    float* hs = (float*)at(s.hs);
+    void* lnb = at(s.ln);
+    void* qkvb = at(s.qkv);
+    void* att = at(s.att);
+    void* gg = at(s.gg);
+    void* hsT = at(s.hsT);
+    groupnorm(L, dt, X, wf(n + "gn.w", C), wf(n + "gn.b", C), gnb, (float2*)at(s.stats), p.BT, hw, C, 1e-6f);
     {
       Epi e = ep(hs, C, wf(n + "pin.b", C));
       e.out_f32 = 1;
@@ -292,7 +314,7 @@ struct Fwd {
       e.act = ACT_GEGLU;
       linear(lnb, Mm, C, n + "geglu.w", 8 * C, e);
     } else {
-      void* tmp = buf((set + "gg2").c_str());
+      void* tmp = at(s.gg2);
       linear(lnb, Mm, C, n + "geglu.w", 8 * C, ep(tmp, 8 * C, wf(n + "geglu.b", 8 * C)));
       geglu_pair(L, dt, tmp, gg, Mm, 4 * C);
     }
@@ -331,11 +353,11 @@ struct Fwd {
     const Plan& p = c->plan;
     const int C = c->cfg.features;
     const std::string n = "ref" + std::to_string(k) + ".";
-    void* tmp = buf("ref.tmp");
-    void* s = buf("ref.s");
-    void* sr = buf("ref.sr");
-    void* u = buf("ref.u");
-    void* v = buf("ref.v");
+    void* tmp = at(p.ref_tmp);
+    void* s = at(p.ref_s);
+    void* sr = at(p.ref_sr);
+    void* u = at(p.ref_u);
+    void* v = at(p.ref_v);
     const void* in = x0;
     const void* inr = x0r;
     if (x1) {
@@ -355,17 +377,17 @@ struct Fwd {
                  int OH, int OW, float sig_sign, float* out) {
     const Plan& p = c->plan;
     const int F_ = c->cfg.features, Fh = F_ / 2;
-    void* o1 = buf("head.o1");
+    void* o1 = at(p.head_o1);
     conv3(X, p.BT, H, Wd, F_, c0 + ".w", Fh, ep(o1, Fh, wf(c0 + ".b", Fh)));
     const float* hw_ = wf(c4 + ".w", 33);
-    if (tc() && head_fused_supported(dt, Fh)) {
+    if (p.fused_head) {
       // K14: the upsampled map and the 32-channel conv output never touch HBM
       L.tag = tag_of(c2);
       head_fused(L, dt, o1, wt(c2 + ".w", (size_t)32 * 9 * Fh), wf(c2 + ".b", 32), hw_, out, p.BT, H, Wd, OH, OW, Fh, sig_sign);
       L.tag.clear();
       return;
     }
-    void* up = buf("head.up");
+    void* up = at(p.head_up);
     upsample(L, dt, o1, up, p.BT, H, Wd, OH, OW, Fh);
     if (tc()) {
       Epi e = ep(out, 1, wf(c2 + ".b", 32));
@@ -373,7 +395,7 @@ struct Fwd {
       e.head_b = 0.f;  // the kernel adds head_w[32]
       conv3(up, p.BT, OH, OW, Fh, c2 + ".w", 32, e);
     } else {
-      void* t32 = buf("head.t32");
+      void* t32 = at(p.head_t32);
       Epi e = ep(t32, 32, wf(c2 + ".b", 32));
       e.act = ACT_RELU;
       conv3(up, p.BT, OH, OW, Fh, c2 + ".w", 32, e);
@@ -387,8 +409,8 @@ struct Fwd {
     const int D = g.dim;
     L.begin();
     // ---- K1 + K2: preprocess, patch embedding (patch_embed.py:75-77; vision_transformer.py:219-227)
-    void* A0 = buf("A0");
-    float* x = (float*)buf("x");
+    void* A0 = at(p.A0);
+    float* x = (float*)at(p.x);
     {
       // endodac with pre_norm=False feeds raw [0,1] pixels (endodac.py:208-211)
       preprocess_patches(L, dt, frames, u8, A0, p.BT, p.H, p.W, p.h, p.w, KPATCH, g.no_normalize ? 0 : 1);
@@ -403,12 +425,12 @@ struct Fwd {
       e.rb_div = 1; e.rb_mod = p.P; e.rb_ld = D;
       linear(A0, p.Mp, KPATCH, "patch.w", D, e);
     }
-    snapshot("tokens0", x, true, p.M, D, D);
+    snapshot(p.dbg.tokens0, x, D, true);
     // ---- encoder blocks (block.py:110-151)
-    void* xn = buf("xn");
-    void* qkv = buf("qkv");
-    void* ao = buf("ao");
-    void* hb = buf("h");
+    void* xn = at(p.xn);
+    void* qkv = at(p.qkv);
+    void* ao = at(p.ao);
+    void* hb = at(p.hid);
     int tap_i = 0;
     // ViT-S (D = 384) on the tensor-core path: proj / fc2 run as row-owning GEMMs whose epilogue also emits the
     // LayerNorm'ed operand of the NEXT GEMM (gemm_ln.cuh), so only the very first norm1 and the four tap norms remain
@@ -454,34 +476,31 @@ struct Fwd {
         linear(hb, p.M, 4 * D, n + "fc2.w", D, e);
       }
       if (g.res_blocks & (1 << i)) res_block(n, x);
-      if (i == 0) snapshot("block0", x, true, p.M, D, D);
+      if (i == 0) snapshot(p.dbg.block0, x, D, true);
       if (tap_i < 4 && i == g.taps[tap_i]) {
-        char tn[16];
-        snprintf(tn, sizeof tn, "tap%d", tap_i);
+        void* tap = at(p.tap[tap_i]);
         // final norm on the tap + cls split (vision_transformer.py:318-321)
-        layernorm(L, dt, x, wf("norm.w", D), wf("norm.b", D), buf(tn), p.Mp, D, 1e-6f, g.no_cls ? 0 : p.N, g.no_cls ? 0 : 1);
-        snapshot(tn, buf(tn), false, p.Mp, D, D);
+        layernorm(L, dt, x, wf("norm.w", D), wf("norm.b", D), tap, p.Mp, D, 1e-6f, g.no_cls ? 0 : p.N, g.no_cls ? 0 : 1);
+        snapshot(p.dbg.tap[tap_i], tap, D, false);
         if (g.use_clstoken) {
           // readout projects (dpt.py:92-99; dpt_pyramid.py:54-57): tap' = GELU(Linear(2D, D)([token | class token])) =
           // GELU(token W1^T + rb[frame]) with the per-frame row bias rb = class token W2^T + b.  The class token is row 0
           // of the frame after the final norm (without a cls token: its first patch token, as in the reference).
-          char cn[16], rn_[16], on[16];
-          snprintf(cn, sizeof cn, "tapc%d", tap_i);
-          snprintf(rn_, sizeof rn_, "rorb%d", tap_i);
-          snprintf(on, sizeof on, "tapr%d", tap_i);
+          void* cls_tok = at(p.tapc[tap_i]);
+          float* rb = (float*)at(p.rorb[tap_i]);
           const std::string ro = "ro" + std::to_string(tap_i) + ".";
-          layernorm(L, dt, x, wf("norm.w", D), wf("norm.b", D), buf(cn), p.BT, D, 1e-6f, p.N, -1);
+          layernorm(L, dt, x, wf("norm.w", D), wf("norm.b", D), cls_tok, p.BT, D, 1e-6f, p.N, -1);
           {
-            Epi e = ep(buf(rn_), D, wf(ro + "b", D));
+            Epi e = ep(rb, D, wf(ro + "b", D));
             e.out_f32 = 1;
-            linear(buf(cn), p.BT, D, ro + "w2", D, e);
+            linear(cls_tok, p.BT, D, ro + "w2", D, e);
           }
           {
-            Epi e = ep(buf(on), D, nullptr);
-            e.rowbias = (const float*)buf(rn_);
+            Epi e = ep(at(p.tapr[tap_i]), D, nullptr);
+            e.rowbias = rb;
             e.rb_div = p.P; e.rb_mod = p.BT; e.rb_ld = D;
             e.act = ACT_GELU;
-            linear(buf(tn), p.Mp, D, ro + "w1", D, e);
+            linear(tap, p.Mp, D, ro + "w1", D, e);
           }
         }
         ++tap_i;
@@ -490,17 +509,18 @@ struct Fwd {
     if (tap_i != 4) L.fail(EDV_ERR_ARG, "taps must be increasing block indices < depth");
     // ---- DPT head (dpt_pyramid.py:51-113)
     const int F_ = g.features;
-    void* L1 = buf("L1");
-    void* L2 = buf("L2");
-    void* L3 = buf("L3");
-    void* L4p = buf("L4p");
-    void* L4 = buf("L4");
+    void* L1 = at(p.L1);
+    void* L2 = at(p.L2);
+    void* L3 = at(p.L3);
+    void* L4p = at(p.L4p);
+    void* L4 = at(p.L4);
     // endodac (models/endodac/endodac.py:93-127) is this head without the four temporal modules
     const bool mm_on = !g.no_motion;
-    void* L3m = mm_on ? buf("L3m") : L3;
-    void* L4m = mm_on ? buf("L4m") : L4;
-    void *l1r = buf("l1r"), *l2r = buf("l2r"), *l3r = buf("l3r"), *l4r = buf("l4r");
-    void *l1rr = buf("l1rr"), *l2rr = buf("l2rr"), *l3rr = buf("l3rr"), *l4rr = buf("l4rr");
+    void* L3m = mm_on ? at(p.L3m) : L3;
+    void* L4m = mm_on ? at(p.L4m) : L4;
+    void *l1r = at(p.lr[0]), *l2r = at(p.lr[1]), *l3r = at(p.lr[2]), *l4r = at(p.lr[3]);
+    void *l1rr = at(p.lrr[0]), *l2rr = at(p.lrr[1]), *l3rr = at(p.lrr[2]), *l4rr = at(p.lrr[3]);
+    const Buf* tap_out = g.use_clstoken ? p.tapr : p.tap;   // what the reassemble projections read
     // The decoder is a DAG: paths 1-3 (reassemble -> [temporal module 0] -> layer_rn) only meet the deep path at
     // their fusion blocks.  The deep path (path 4 -> refinenet4 -> module 2 -> refinenet3 -> module 3 -> ...) is a
     // chain of small, latency-bound launches on 19 x 19 / 37 x 37 maps that leaves most SMs idle, so paths 1-3 run
@@ -510,15 +530,15 @@ struct Fwd {
       // projects[0] (1x1) merged with resize_layers[0] (ConvT k4 s4): one GEMM + pixel shuffle
       Epi e = ep(L1, p.Cp[0], wf("proj0.b", 16 * p.Cp[0]));
       e.map = MAP_PIXSHUF; e.ps_k = 4; e.ps_h = p.ph; e.ps_w = p.pw; e.ps_c = p.Cp[0];
-      linear(buf(g.use_clstoken ? "tapr0" : "tap0"), p.Mp, D, "proj0.w", 16 * p.Cp[0], e);
+      linear(at(tap_out[0]), p.Mp, D, "proj0.w", 16 * p.Cp[0], e);
     }
     {
       Epi e = ep(L2, p.Cp[1], wf("proj1.b", 4 * p.Cp[1]));
       e.map = MAP_PIXSHUF; e.ps_k = 2; e.ps_h = p.ph; e.ps_w = p.pw; e.ps_c = p.Cp[1];
-      linear(buf(g.use_clstoken ? "tapr1" : "tap1"), p.Mp, D, "proj1.w", 4 * p.Cp[1], e);
+      linear(at(tap_out[1]), p.Mp, D, "proj1.w", 4 * p.Cp[1], e);
     }
-    linear(buf(g.use_clstoken ? "tapr2" : "tap2"), p.Mp, D, "proj2.w", p.Cp[2], ep(L3, p.Cp[2], wf("proj2.b", p.Cp[2])));
-    if (mm_on) motion(0, L3, L3m, par ? "mmb." : "mm.");
+    linear(at(tap_out[2]), p.Mp, D, "proj2.w", p.Cp[2], ep(L3, p.Cp[2], wf("proj2.b", p.Cp[2])));
+    if (mm_on) motion(0, L3, L3m, par ? p.mmb : p.mm);
     // scratch.layer{1-4}_rn (3x3, no bias) -> F channels, plus relu copies for the RCUs
     {
       Epi e = ep(l3r, F_, nullptr); e.out_relu = l3rr;
@@ -529,12 +549,12 @@ struct Fwd {
       conv3(L1, p.BT, 4 * p.ph, 4 * p.pw, p.Cp[0], "rn1.w", F_, e);
     }
     back_to_main();
-    linear(buf(g.use_clstoken ? "tapr3" : "tap3"), p.Mp, D, "proj3.w", p.Cp[3], ep(L4p, p.Cp[3], wf("proj3.b", p.Cp[3])));
+    linear(at(tap_out[3]), p.Mp, D, "proj3.w", p.Cp[3], ep(L4p, p.Cp[3], wf("proj3.b", p.Cp[3])));
     {
       // resize_layers[3]: 3x3 stride 2 pad 1 (dpt.py:85-90) = explicit im2col + GEMM
       const long long Mo = (long long)p.BT * p.ph2 * p.pw2;
       if (tc()) {
-        void* col = buf("col");
+        void* col = at(p.col);
         im2col3x3(L, dt, L4p, col, p.BT, p.ph, p.pw, p.Cp[3], p.ph2, p.pw2, 2);
         linear(col, Mo, 9 * p.Cp[3], "resize3.w", p.Cp[3], ep(L4, p.Cp[3], wf("resize3.b", p.Cp[3])));
       } else {
@@ -545,32 +565,32 @@ struct Fwd {
         if (L.ok()) gemm(L, dt, eng, a);
       }
     }
-    if (mm_on) motion(1, L4, L4m);
+    if (mm_on) motion(1, L4, L4m, p.mm);
     {
       Epi e = ep(l4r, F_, nullptr); e.out_relu = l4rr;
       conv3(L4m, p.BT, p.ph2, p.pw2, p.Cp[3], "rn4.w", F_, e);
     }
-    snapshot("layer1", L1, false, (long long)p.BT * 16 * p.P, p.Cp[0], g.out_channels[0]);
-    snapshot("layer2", L2, false, (long long)p.BT * 4 * p.P, p.Cp[1], g.out_channels[1]);
-    snapshot("layer3", L3, false, p.Mp, p.Cp[2], g.out_channels[2]);
-    snapshot("layer4", L4, false, (long long)p.BT * p.ph2 * p.pw2, p.Cp[3], g.out_channels[3]);
-    snapshot("mm0", L3m, false, p.Mp, p.Cp[2], g.out_channels[2]);
-    snapshot("mm1", L4m, false, (long long)p.BT * p.ph2 * p.pw2, p.Cp[3], g.out_channels[3]);
-    void *p4 = buf("p4"), *p3 = buf("p3"), *p2 = buf("p2"), *p1 = buf("p1");
-    void *p4m = mm_on ? buf("p4m") : p4, *p3m = mm_on ? buf("p3m") : p3;
+    snapshot(p.dbg.layer[0], L1, p.Cp[0], false);
+    snapshot(p.dbg.layer[1], L2, p.Cp[1], false);
+    snapshot(p.dbg.layer[2], L3, p.Cp[2], false);
+    snapshot(p.dbg.layer[3], L4, p.Cp[3], false);
+    snapshot(p.dbg.mm[0], L3m, p.Cp[2], false);
+    snapshot(p.dbg.mm[1], L4m, p.Cp[3], false);
+    void *p4 = at(p.p4), *p3 = at(p.p3), *p2 = at(p.p2), *p1 = at(p.p1);
+    void *p4m = mm_on ? at(p.p4m) : p4, *p3m = mm_on ? at(p.p3m) : p3;
     fusion(4, l4r, l4rr, nullptr, nullptr, p.ph2, p.pw2, p.ph, p.pw, p4);
-    snapshot("path4_pre", p4, false, p.Mp, F_, F_);
-    if (mm_on) motion(2, p4, p4m);
+    snapshot(p.dbg.path4_pre, p4, F_, false);
+    if (mm_on) motion(2, p4, p4m, p.mm);
     join_side();   // refinenet3 is the first consumer of the side stream's layer{1,2,3}_rn maps
     fusion(3, p4m, nullptr, l3r, l3rr, p.ph, p.pw, 2 * p.ph, 2 * p.pw, p3);
-    if (mm_on) motion(3, p3, p3m);
-    snapshot("path3", p3m, false, (long long)p.BT * 4 * p.P, F_, F_);
+    if (mm_on) motion(3, p3, p3m, p.mm);
+    snapshot(p.dbg.path3, p3m, F_, false);
     fusion(2, p3m, nullptr, l2r, l2rr, 2 * p.ph, 2 * p.pw, 4 * p.ph, 4 * p.pw, p2);
     fusion(1, p2, nullptr, l1r, l1rr, 4 * p.ph, 4 * p.pw, 8 * p.ph, 8 * p.pw, p1);
-    snapshot("path1", p1, false, (long long)p.BT * 64 * p.P, F_, F_);
+    snapshot(p.dbg.path1, p1, F_, false);
     // ---- disparity outputs
     float* d[4];
-    for (int s = 0; s < 4; ++s) d[s] = disp[s] ? disp[s] : (float*)buf(s == 0 ? "disp0" : s == 1 ? "disp1" : s == 2 ? "disp2" : "disp3");
+    for (int s = 0; s < 4; ++s) d[s] = disp[s] ? disp[s] : (float*)at(p.disp[s]);
     if (!g.conv_head) {
       disp_head("oc1", "oc2a", "oc2b", p1, 8 * p.ph, 8 * p.pw, p.out_h[0], p.out_w[0], 0.f, d[0]);
       for (int s = 1; s < 4; ++s) resize_f32(L, d[s - 1], d[s], p.BT, p.out_h[s - 1], p.out_w[s - 1], p.out_h[s], p.out_w[s]);
@@ -598,10 +618,10 @@ struct Fwd {
   void res_block(const std::string& n, float* x) {
     const Plan& p = c->plan;
     const int D = c->cfg.dim, bc = D / 8, bcp = round_up(bc, 64);
-    void* pt = buf("rb.pt");
-    void* t1 = buf("rb.t1");
-    void* t2 = buf("rb.t2");
-    void* t3 = buf("rb.t3");
+    void* pt = at(p.rb_pt);
+    void* t1 = at(p.rb_t1);
+    void* t2 = at(p.rb_t2);
+    void* t3 = at(p.rb_t3);
     const int cls = c->cfg.no_cls ? 0 : 1;
     tokens_to_patches(L, dt, x, pt, p.Mp, p.P, D, cls);
     linear(pt, p.Mp, D, n + "res.c1.w", bcp, ep(t1, bcp, nullptr));
@@ -706,12 +726,12 @@ int edv_plan(edv_ctx* ctx, int B, int T, int H, int W, int net_h, int net_w, siz
     if (g.dim % 8 != 0) return set_err(ctx, EDV_ERR_ARG, "edv_plan: residual blocks need dim %% 8 == 0");
   }
   const int F_ = g.features, Fh = F_ / 2;
-  p.mm[0] = MMPlan{p.Cp[2], p.ph, p.pw};
-  p.mm[1] = MMPlan{p.Cp[3], p.ph2, p.pw2};
-  p.mm[2] = MMPlan{F_, p.ph, p.pw};
-  p.mm[3] = MMPlan{F_, 2 * p.ph, 2 * p.pw};
+  p.mod[0] = MMPlan{p.Cp[2], p.ph, p.pw};
+  p.mod[1] = MMPlan{p.Cp[3], p.ph2, p.pw2};
+  p.mod[2] = MMPlan{F_, p.ph, p.pw};
+  p.mod[3] = MMPlan{F_, 2 * p.ph, 2 * p.pw};
   for (int j = 0; j < 4 && !g.no_motion; ++j) {
-    int hd = p.mm[j].C / 8;
+    int hd = p.mod[j].C / 8;
     if (!(hd == 8 || hd == 24 || hd == 32 || hd == 48 || hd == 128))
       return set_err(ctx, EDV_ERR_ARG, "edv_plan: temporal head dim %d unsupported (8,24,32,48,128)", hd);
   }
@@ -727,141 +747,118 @@ int edv_plan(edv_ctx* ctx, int B, int T, int H, int W, int net_h, int net_w, siz
   for (int s = 0; s < 4; ++s)
     if (p.out_h[s] < 1 || p.out_w[s] < 1) return set_err(ctx, EDV_ERR_ARG, "edv_plan: resolution too small for the 4-level pyramid");
 
-  const size_t es = dtype_size(g.dtype);
+  p.tc = g.dtype != EDV_F32 && g.engine != EDV_ENGINE_SIMT;
+  p.fused_head = p.tc && head_fused_supported(g.dtype, Fh);
+
+  // Workspace layout: each buffer is placed here, in this order, at a 1 KiB-aligned offset.
+  const int es = (int)dtype_size(g.dtype);
   size_t off = 0;
-  auto add = [&](const char* name, size_t bytes, int elem = 0) {
-    Buf b;
+  auto place = [&](Buf& b, std::string name, size_t count, int elem) {
+    b.name = std::move(name);
     b.off = off;
-    b.bytes = bytes;
-    b.elem = elem ? elem : (int)es;
-    p.bufs[name] = b;
-    off += (bytes + 1023) & ~(size_t)1023;
+    b.bytes = count * elem;
+    b.elem = elem;
+    off += (b.bytes + 1023) & ~(size_t)1023;
+  };
+  auto add = [&](Buf& b, std::string name, size_t count, int elem) {
+    place(b, std::move(name), count, elem);
+    p.bufs.push_back(b);
   };
   const int D = g.dim;
-  const bool simt = (g.dtype == EDV_F32) || g.engine == EDV_ENGINE_SIMT;
-  add("A0", (size_t)p.Mp * KPATCH * es);
-  add("x", (size_t)p.M * D * 4, 4);
-  add("xn", (size_t)p.M * D * es);
-  add("qkv", (size_t)p.M * 3 * D * es);
-  add("ao", (size_t)p.M * D * es);
-  add("h", (size_t)p.M * 4 * D * es);
+  add(p.A0, "A0", (size_t)p.Mp * KPATCH, es);
+  add(p.x, "x", (size_t)p.M * D, 4);
+  add(p.xn, "xn", (size_t)p.M * D, es);
+  add(p.qkv, "qkv", (size_t)p.M * 3 * D, es);
+  add(p.ao, "ao", (size_t)p.M * D, es);
+  add(p.hid, "h", (size_t)p.M * 4 * D, es);
   for (int i = 0; i < 4; ++i) {
-    char n[8];
-    snprintf(n, sizeof n, "tap%d", i);
-    add(n, (size_t)p.Mp * D * es);
+    const std::string n = std::to_string(i);
+    add(p.tap[i], "tap" + n, (size_t)p.Mp * D, es);
     if (g.use_clstoken) {
-      char m[16];
-      snprintf(m, sizeof m, "tapc%d", i);
-      add(m, (size_t)p.BT * D * es);
-      snprintf(m, sizeof m, "rorb%d", i);
-      add(m, (size_t)p.BT * D * 4, 4);
-      snprintf(m, sizeof m, "tapr%d", i);
-      add(m, (size_t)p.Mp * D * es);
+      add(p.tapc[i], "tapc" + n, (size_t)p.BT * D, es);
+      add(p.rorb[i], "rorb" + n, (size_t)p.BT * D, 4);
+      add(p.tapr[i], "tapr" + n, (size_t)p.Mp * D, es);
     }
   }
   if (g.res_blocks) {
     const int bcp = round_up(D / 8, 64);
-    add("rb.pt", (size_t)p.Mp * D * es);
-    add("rb.t1", (size_t)p.Mp * bcp * es);
-    add("rb.t2", (size_t)p.Mp * bcp * es);
-    add("rb.t3", (size_t)p.Mp * D * es);
+    add(p.rb_pt, "rb.pt", (size_t)p.Mp * D, es);
+    add(p.rb_t1, "rb.t1", (size_t)p.Mp * bcp, es);
+    add(p.rb_t2, "rb.t2", (size_t)p.Mp * bcp, es);
+    add(p.rb_t3, "rb.t3", (size_t)p.Mp * D, es);
   }
   const size_t px1 = (size_t)p.BT * 16 * p.P, px2 = (size_t)p.BT * 4 * p.P, px3 = (size_t)p.Mp, px4 = (size_t)p.BT * p.ph2 * p.pw2;
   const size_t px0 = (size_t)p.BT * 64 * p.P;  // 8ph x 8pw
-  add("L1", px1 * p.Cp[0] * es);
-  add("L2", px2 * p.Cp[1] * es);
-  add("L3", px3 * p.Cp[2] * es);
-  add("L4p", px3 * p.Cp[3] * es);
-  add("L4", px4 * p.Cp[3] * es);
-  if (!simt) add("col", px4 * 9 * p.Cp[3] * es);
+  const size_t px[4] = {px1, px2, px3, px4};   // layer{1-4}
+  add(p.L1, "L1", px1 * p.Cp[0], es);
+  add(p.L2, "L2", px2 * p.Cp[1], es);
+  add(p.L3, "L3", px3 * p.Cp[2], es);
+  add(p.L4p, "L4p", px3 * p.Cp[3], es);
+  add(p.L4, "L4", px4 * p.Cp[3], es);
+  if (p.tc) add(p.col, "col", px4 * 9 * p.Cp[3], es);
   if (!g.no_motion) {
-    add("L3m", px3 * p.Cp[2] * es);
-    add("L4m", px4 * p.Cp[3] * es);
+    add(p.L3m, "L3m", px3 * p.Cp[2], es);
+    add(p.L4m, "L4m", px4 * p.Cp[3], es);
+    // temporal-module scratch: mm sized for the largest of the four modules, mmb for module 0
+    size_t mmC = 0;
+    for (int j = 0; j < 4; ++j) mmC = std::max(mmC, (size_t)p.BT * p.mod[j].h * p.mod[j].w * p.mod[j].C);
+    const size_t r0 = (size_t)p.BT * p.mod[0].h * p.mod[0].w * p.mod[0].C;
+    auto add_mm = [&](MMScratch& s, const std::string& set, size_t n) {
+      add(s.stats, set + "stats", (size_t)p.BT * 32 * (1 + GN_MAX_SPLIT), (int)sizeof(float2));
+      add(s.gn, set + "gn", n, es);
+      add(s.hs, set + "hs", n, 4);
+      add(s.ln, set + "ln", n, es);
+      add(s.qkv, set + "qkv", 3 * n, es);
+      add(s.att, set + "att", n, es);
+      add(s.gg, set + "gg", 4 * n, es);
+      add(s.hsT, set + "hsT", n, es);
+    };
+    add_mm(p.mm, "mm.", mmC);
+    add_mm(p.mmb, "mmb.", r0);
+    if (!p.tc) {
+      add(p.mm.gg2, "mm.gg2", 8 * mmC, es);
+      add(p.mmb.gg2, "mmb.gg2", 8 * r0, es);
+    }
   }
-  // motion-module scratch, sized for the largest of the four modules
-  size_t mmC = 0, mm3 = 0, mm4 = 0, mm8 = 0;
-  for (int j = 0; j < 4; ++j) {
-    size_t rows = (size_t)p.BT * p.mm[j].h * p.mm[j].w, C = p.mm[j].C;
-    mmC = std::max(mmC, rows * C);
-    mm3 = std::max(mm3, rows * 3 * C);
-    mm4 = std::max(mm4, rows * 4 * C);
-    mm8 = std::max(mm8, rows * 8 * C);
+  for (int i = 0; i < 4; ++i) {
+    const std::string n = "l" + std::to_string(i + 1);
+    add(p.lr[i], n + "r", px[i] * F_, es);
+    add(p.lrr[i], n + "rr", px[i] * F_, es);
   }
-  if (!g.no_motion) {
-    add("mm.stats", (size_t)p.BT * 32 * (1 + GN_MAX_SPLIT) * sizeof(float2), 8);
-    add("mm.gn", mmC * es);
-    add("mm.hs", mmC * 4, 4);
-    add("mm.ln", mmC * es);
-    add("mm.qkv", mm3 * es);
-    add("mm.att", mmC * es);
-    add("mm.gg", mm4 * es);
-    add("mm.hsT", mmC * es);
-    // second scratch family for module 0, which runs on the side stream while module 1 runs on the main one
-    const size_t r0 = (size_t)p.BT * p.mm[0].h * p.mm[0].w * p.mm[0].C;
-    add("mmb.stats", (size_t)p.BT * 32 * (1 + GN_MAX_SPLIT) * sizeof(float2), 8);
-    add("mmb.gn", r0 * es);
-    add("mmb.hs", r0 * 4, 4);
-    add("mmb.ln", r0 * es);
-    add("mmb.qkv", 3 * r0 * es);
-    add("mmb.att", r0 * es);
-    add("mmb.gg", 4 * r0 * es);
-    add("mmb.hsT", r0 * es);
-  }
-  if (simt && !g.no_motion) {
-    add("mm.gg2", mm8 * es);
-    add("mmb.gg2", 8 * (size_t)p.BT * p.mm[0].h * p.mm[0].w * p.mm[0].C * es);
-  }
-  add("l1r", px1 * F_ * es); add("l1rr", px1 * F_ * es);
-  add("l2r", px2 * F_ * es); add("l2rr", px2 * F_ * es);
-  add("l3r", px3 * F_ * es); add("l3rr", px3 * F_ * es);
-  add("l4r", px4 * F_ * es); add("l4rr", px4 * F_ * es);
   // refinenet scratch at the largest input resolution (refinenet1 runs at 4ph x 4pw)
-  add("ref.tmp", px1 * F_ * es);
-  add("ref.s", px1 * F_ * es);
-  add("ref.sr", px1 * F_ * es);
-  add("ref.u", px1 * F_ * es);
-  add("ref.v", px1 * F_ * es);
-  add("p4", px3 * F_ * es); add("p4m", px3 * F_ * es);
-  add("p3", px2 * F_ * es); add("p3m", px2 * F_ * es);
-  add("p2", px1 * F_ * es);
-  add("p1", px0 * F_ * es);
+  add(p.ref_tmp, "ref.tmp", px1 * F_, es);
+  add(p.ref_s, "ref.s", px1 * F_, es);
+  add(p.ref_sr, "ref.sr", px1 * F_, es);
+  add(p.ref_u, "ref.u", px1 * F_, es);
+  add(p.ref_v, "ref.v", px1 * F_, es);
+  add(p.p4, "p4", px3 * F_, es);
+  add(p.p4m, "p4m", px3 * F_, es);
+  add(p.p3, "p3", px2 * F_, es);
+  add(p.p3m, "p3m", px2 * F_, es);
+  add(p.p2, "p2", px1 * F_, es);
+  add(p.p1, "p1", px0 * F_, es);
   // disparity head scratch: conv at up to 8ph x 8pw, upsample target up to out_h[0] x out_w[0]
   const size_t pxo = (size_t)p.BT * p.out_h[0] * p.out_w[0];
-  add("head.o1", px0 * Fh * es);
-  const bool fused_head = !simt && head_fused_supported(g.dtype, Fh);   // the upsampled map never exists in HBM then
-  if (!fused_head) add("head.up", pxo * Fh * es);
-  if (simt) add("head.t32", pxo * 32 * es);
-  for (int s = 0; s < 4; ++s) {
-    char n[8];
-    snprintf(n, sizeof n, "disp%d", s);
-    add(n, (size_t)p.BT * p.out_h[s] * p.out_w[s] * 4, 4);
-  }
+  add(p.head_o1, "head.o1", px0 * Fh, es);
+  if (!p.fused_head) add(p.head_up, "head.up", pxo * Fh, es);
+  if (!p.tc) add(p.head_t32, "head.t32", pxo * 32, es);
+  for (int s = 0; s < 4; ++s) add(p.disp[s], "disp" + std::to_string(s), (size_t)p.BT * p.out_h[s] * p.out_w[s], 4);
   if (ctx->debug) {
-    auto tap = [&](const char* name, long long rows, int cols) {
-      DebugTap t;
+    auto tap = [&](DebugTap& t, std::string name, long long rows, int cols) {
+      place(t.buf, std::move(name), (size_t)rows * cols, 4);
       t.rows = rows;
       t.cols = cols;
-      t.buf.off = off;
-      t.buf.bytes = (size_t)rows * cols * 4;
-      off += (t.buf.bytes + 1023) & ~(size_t)1023;
-      p.taps[name] = t;
+      p.taps.push_back(t);
     };
-    tap("tokens0", p.M, D);
-    tap("block0", p.M, D);
-    for (int i = 0; i < 4; ++i) {
-      char n[8];
-      snprintf(n, sizeof n, "tap%d", i);
-      tap(n, p.Mp, D);
-    }
-    tap("layer1", px1, g.out_channels[0]);
-    tap("layer2", px2, g.out_channels[1]);
-    tap("layer3", px3, g.out_channels[2]);
-    tap("layer4", px4, g.out_channels[3]);
-    tap("mm0", px3, g.out_channels[2]);
-    tap("mm1", px4, g.out_channels[3]);
-    tap("path4_pre", px3, F_);
-    tap("path3", px2, F_);
-    tap("path1", px0, F_);
+    tap(p.dbg.tokens0, "tokens0", p.M, D);
+    tap(p.dbg.block0, "block0", p.M, D);
+    for (int i = 0; i < 4; ++i) tap(p.dbg.tap[i], "tap" + std::to_string(i), p.Mp, D);
+    for (int i = 0; i < 4; ++i) tap(p.dbg.layer[i], "layer" + std::to_string(i + 1), px[i], g.out_channels[i]);
+    tap(p.dbg.mm[0], "mm0", px3, g.out_channels[2]);
+    tap(p.dbg.mm[1], "mm1", px4, g.out_channels[3]);
+    tap(p.dbg.path4_pre, "path4_pre", px3, F_);
+    tap(p.dbg.path3, "path3", px2, F_);
+    tap(p.dbg.path1, "path1", px0, F_);
   }
   p.total = off + 1024;
   p.valid = true;
@@ -890,7 +887,6 @@ __global__ void __launch_bounds__(256) copy_pyramid_kernel(PyramidCopy c) {
   }
 }
 static int copy_pyramid_out(edv_ctx* ctx, float* const disp[4], void* workspace_dev, cudaStream_t st) {
-  static const char* names[4] = {"disp0", "disp1", "disp2", "disp3"};
   PyramidCopy c;
   c.start[0] = 0;
   bool vec = true, any = false;
@@ -899,11 +895,9 @@ static int copy_pyramid_out(edv_ctx* ctx, float* const disp[4], void* workspace_
   for (int s = 0; s < 4; ++s) {
     c.src[s] = nullptr; c.dst[s] = nullptr; c.n4[s] = 0; bytes[s] = 0; src[s] = nullptr;
     if (disp[s]) {
-      auto it = ctx->plan.bufs.find(names[s]);
-      if (it == ctx->plan.bufs.end()) return set_err(ctx, EDV_ERR_STATE, "edv_forward: internal disparity buffer missing");
       const size_t n = (size_t)ctx->plan.BT * ctx->plan.out_h[s] * ctx->plan.out_w[s];
       bytes[s] = n * sizeof(float);
-      src[s] = (const unsigned char*)workspace_dev + it->second.off;
+      src[s] = (const unsigned char*)workspace_dev + ctx->plan.disp[s].off;
       if ((n & 3) || ((uintptr_t)disp[s] & 15) || ((uintptr_t)src[s] & 15)) vec = false;
       c.src[s] = (const float4*)src[s]; c.dst[s] = (float4*)disp[s]; c.n4[s] = n / 4;
       any = true;
@@ -924,6 +918,55 @@ static int copy_pyramid_out(edv_ctx* ctx, float* const disp[4], void* workspace_
   return EDV_OK;
 }
 
+// Capture the forward on the private capture stream into key.exec / key.launches.  False when that gave no graph
+// (graph_note says why): the caller then runs the forward eagerly.
+static bool capture(edv_ctx* ctx, GraphEntry& key, const void* frames, bool u8, float* resized_dev, int out_h, int out_w,
+                    void* workspace_dev) {
+  // Capture on a private stream and replay on the caller's: the capture itself executes nothing, and the caller's
+  // stream is usually torch's current stream = the legacy default stream, which cudaStreamBeginCapture refuses.
+  int prio_lo = 0, prio_hi = 0;
+  cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);   // the captured main chain outranks the side-stream branches
+  if (!ctx->cap_stream && cudaStreamCreateWithPriority(&ctx->cap_stream, cudaStreamNonBlocking, prio_hi) != cudaSuccess) {
+    ctx->graph_note = std::string("cudaStreamCreateWithPriority: ") + cudaGetErrorString(cudaGetLastError());
+    ctx->cap_stream = nullptr;
+    ctx->graph_mode = 0;
+    return false;
+  }
+  cudaStream_t cap = ctx->cap_stream;
+  cudaError_t be = cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal);
+  if (be != cudaSuccess) {
+    ctx->graph_note = std::string("cudaStreamBeginCapture: ") + cudaGetErrorString(be);
+    cudaGetLastError();
+    return false;
+  }
+  int rc;
+  {
+    float* none[4] = {nullptr, nullptr, nullptr, nullptr};
+    Fwd f(ctx, workspace_dev, cap);
+    rc = f.run(frames, u8, none, resized_dev, out_h, out_w);   // pyramid into the plan's own buffers (see GraphEntry)
+    key.launches = f.L.count;
+  }
+  cudaGraph_t graph = nullptr;
+  const cudaError_t ce = cudaStreamEndCapture(cap, &graph);
+  if (rc != EDV_OK || ce != cudaSuccess || !graph) {
+    if (graph) cudaGraphDestroy(graph);
+    ctx->graph_note = rc != EDV_OK ? std::string("forward failed under capture: ") + ctx->err : std::string("cudaStreamEndCapture: ") + cudaGetErrorString(ce);
+    cudaGetLastError();
+    ctx->graph_mode = 0;   // capture is not possible in this process: stay eager (and say why in edv_graph_status)
+    return false;
+  }
+  const cudaError_t ie = cudaGraphInstantiate(&key.exec, graph, 0);
+  cudaGraphDestroy(graph);
+  if (ie != cudaSuccess || !key.exec) {
+    ctx->graph_note = std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ie);
+    cudaGetLastError();
+    ctx->graph_mode = 0;
+    return false;
+  }
+  ctx->graph_note = "ok";
+  return true;
+}
+
 static int forward_common(edv_ctx* ctx, const void* frames, bool u8, float* const disp_dev[4], float* resized_dev,
                           int out_h, int out_w, void* workspace_dev, void* stream) {
   if (!ctx || !frames || !workspace_dev) return set_err(ctx, EDV_ERR_ARG, "edv_forward: null argument");
@@ -935,10 +978,18 @@ static int forward_common(edv_ctx* ctx, const void* frames, bool u8, float* cons
   float* none[4] = {nullptr, nullptr, nullptr, nullptr};
   float* const* disp = disp_dev ? disp_dev : none;
   cudaStream_t st = (cudaStream_t)stream;
+  auto eager = [&] {
+    Fwd f(ctx, workspace_dev, st);
+    return f.run(frames, u8, disp, resized_dev, out_h, out_w);
+  };
+  auto replay = [&](const GraphEntry& g) {
+    ctx->last_launches = g.launches;
+    if (cudaGraphLaunch(g.exec, st) != cudaSuccess) return set_err(ctx, EDV_ERR_CUDA, "edv_forward: cudaGraphLaunch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    return copy_pyramid_out(ctx, disp, workspace_dev, st);
+  };
   const bool graphable = ctx->graph_mode && !ctx->prof.on && !ctx->debug && ctx->plan_warm;
   if (!graphable) {
-    Fwd f(ctx, workspace_dev, st);
-    const int rc = f.run(frames, u8, disp, resized_dev, out_h, out_w);
+    const int rc = eager();
     if (rc == EDV_OK) ctx->plan_warm = true;
     return rc;
   }
@@ -946,89 +997,29 @@ static int forward_common(edv_ctx* ctx, const void* frames, bool u8, float* cons
   key.frames = frames; key.resized = resized_dev; key.workspace = workspace_dev;
   key.u8 = u8; key.out_h = resized_dev ? out_h : 0; key.out_w = resized_dev ? out_w : 0;
   ++ctx->graph_clock;
-  for (GraphEntry& g : ctx->graphs) {
-    if (!g.same(key)) continue;
-    g.last_use = ctx->graph_clock;
-    ctx->last_launches = g.launches;
-    if (cudaGraphLaunch(g.exec, st) != cudaSuccess) return set_err(ctx, EDV_ERR_CUDA, "edv_forward: cudaGraphLaunch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    return copy_pyramid_out(ctx, disp, workspace_dev, st);
-  }
+  for (GraphEntry& g : ctx->graphs)
+    if (g.same(key)) {
+      g.last_use = ctx->graph_clock;
+      return replay(g);
+    }
   // A capture costs about as much as a forward at the reference's resolution, so a pointer set is captured only the
   // SECOND time it comes by: a caller whose buffers never repeat (fresh tensors from a cold or fragmented allocator,
   // outputs pinned by record_stream) runs eagerly and pays nothing, a steady caller replays from its third call on.
-  {
-    bool met = false;
-    for (GraphEntry& g : ctx->seen)
-      if (g.same(key)) {
-        met = true;
-        g = ctx->seen.back();
-        ctx->seen.pop_back();
-        break;
-      }
-    if (!met) {
-      key.last_use = ctx->graph_clock;
-      if (ctx->seen.size() >= 4 * (size_t)edv_ctx::GRAPH_SLOTS) ctx->seen.erase(ctx->seen.begin());
-      ctx->seen.push_back(key);
-      Fwd f(ctx, workspace_dev, st);
-      return f.run(frames, u8, disp, resized_dev, out_h, out_w);
-    }
+  auto met = std::find_if(ctx->seen.begin(), ctx->seen.end(), [&](const GraphEntry& g) { return g.same(key); });
+  if (met == ctx->seen.end()) {
+    if (ctx->seen.size() >= 4 * (size_t)edv_ctx::GRAPH_SLOTS) ctx->seen.erase(ctx->seen.begin());
+    ctx->seen.push_back(key);
+    return eager();
   }
+  *met = ctx->seen.back();
+  ctx->seen.pop_back();
   cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
   if (cudaStreamIsCapturing(st, &cs) != cudaSuccess || cs != cudaStreamCaptureStatusNone) {
     // the caller is capturing this stream itself: just record our launches into its graph
     cudaGetLastError();
-    Fwd f(ctx, workspace_dev, st);
-    return f.run(frames, u8, disp, resized_dev, out_h, out_w);
+    return eager();
   }
-  // Capture on a private stream and replay on the caller's: the capture itself executes nothing, and the caller's
-  // stream is usually torch's current stream = the legacy default stream, which cudaStreamBeginCapture refuses.
-  int prio_lo = 0, prio_hi = 0;
-  cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);   // the captured main chain outranks the side-stream branches
-  if (!ctx->cap_stream && cudaStreamCreateWithPriority(&ctx->cap_stream, cudaStreamNonBlocking, prio_hi) != cudaSuccess) {
-    ctx->graph_note = std::string("cudaStreamCreateWithPriority: ") + cudaGetErrorString(cudaGetLastError());
-    ctx->cap_stream = nullptr;
-    ctx->graph_mode = 0;
-    Fwd f(ctx, workspace_dev, st);
-    return f.run(frames, u8, disp, resized_dev, out_h, out_w);
-  }
-  cudaStream_t cap = ctx->cap_stream;
-  cudaError_t be = cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal);
-  if (be != cudaSuccess) {
-    ctx->graph_note = std::string("cudaStreamBeginCapture: ") + cudaGetErrorString(be);
-    cudaGetLastError();
-    Fwd f(ctx, workspace_dev, st);
-    return f.run(frames, u8, disp, resized_dev, out_h, out_w);
-  }
-  int rc;
-  int launches = 0;
-  {
-    Fwd f(ctx, workspace_dev, cap);
-    rc = f.run(frames, u8, none, resized_dev, out_h, out_w);   // pyramid into the plan's own buffers (see GraphEntry)
-    launches = f.L.count;
-  }
-  cudaGraph_t graph = nullptr;
-  const cudaError_t ce = cudaStreamEndCapture(cap, &graph);
-  if (rc != EDV_OK || ce != cudaSuccess || !graph) {
-    if (graph) cudaGraphDestroy(graph);
-    ctx->graph_note = rc != EDV_OK ? std::string("forward failed under capture: ") + ctx->err : std::string("cudaStreamEndCapture: ") + cudaGetErrorString(ce);
-    cudaGetLastError();
-    ctx->graph_mode = 0;   // capture is not possible in this process: stay eager (and say why in edv_graph_status)
-    Fwd f(ctx, workspace_dev, st);
-    return f.run(frames, u8, disp, resized_dev, out_h, out_w);
-  }
-  cudaGraphExec_t exec = nullptr;
-  const cudaError_t ie = cudaGraphInstantiate(&exec, graph, 0);
-  cudaGraphDestroy(graph);
-  if (ie != cudaSuccess || !exec) {
-    ctx->graph_note = std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ie);
-    cudaGetLastError();
-    ctx->graph_mode = 0;
-    Fwd f(ctx, workspace_dev, st);
-    return f.run(frames, u8, disp, resized_dev, out_h, out_w);
-  }
-  ctx->graph_note = "ok";
-  key.exec = exec;
-  key.launches = launches;
+  if (!capture(ctx, key, frames, u8, resized_dev, out_h, out_w, workspace_dev)) return eager();
   key.last_use = ctx->graph_clock;
   if ((int)ctx->graphs.size() >= edv_ctx::GRAPH_SLOTS) {
     size_t lru = 0;
@@ -1039,9 +1030,7 @@ static int forward_common(edv_ctx* ctx, const void* frames, bool u8, float* cons
   } else {
     ctx->graphs.push_back(key);
   }
-  ctx->last_launches = launches;
-  if (cudaGraphLaunch(exec, st) != cudaSuccess) return set_err(ctx, EDV_ERR_CUDA, "edv_forward: cudaGraphLaunch failed: %s", cudaGetErrorString(cudaGetLastError()));
-  return copy_pyramid_out(ctx, disp, workspace_dev, st);
+  return replay(key);
 }
 
 // 1: replay captured CUDA graphs of the planned forward (default), 0: launch every kernel from the host.
@@ -1081,12 +1070,14 @@ int edv_launch_count(const edv_ctx* ctx) { return ctx ? ctx->last_launches : 0; 
 int edv_debug_tap(edv_ctx* ctx, const char* name, size_t* offset_bytes, long long* rows, int* cols) {
   if (!ctx || !name || !offset_bytes || !rows || !cols) return EDV_ERR_ARG;
   if (!ctx->debug || !ctx->plan.valid) return set_err(ctx, EDV_ERR_STATE, "edv_debug_tap: enable edv_set_debug before edv_plan");
-  auto it = ctx->plan.taps.find(name);
-  if (it == ctx->plan.taps.end()) return set_err(ctx, EDV_ERR_ARG, "edv_debug_tap: unknown tap '%s'", name);
-  *offset_bytes = it->second.buf.off;
-  *rows = it->second.rows;
-  *cols = it->second.cols;
-  return EDV_OK;
+  for (const DebugTap& t : ctx->plan.taps)
+    if (t.buf.name == name) {
+      *offset_bytes = t.buf.off;
+      *rows = t.rows;
+      *cols = t.cols;
+      return EDV_OK;
+    }
+  return set_err(ctx, EDV_ERR_ARG, "edv_debug_tap: unknown tap '%s'", name);
 }
 
 // Enumerate the named workspace buffers of the current plan (range / saturation checks of the 16-bit
@@ -1095,12 +1086,11 @@ int edv_debug_tap(edv_ctx* ctx, const char* name, size_t* offset_bytes, long lon
 int edv_plan_buffer(edv_ctx* ctx, int index, char* name, int name_cap, size_t* offset_bytes, size_t* bytes, int* elem_bytes) {
   if (!ctx || !ctx->plan.valid || index < 0 || !name || name_cap < 1 || !offset_bytes || !bytes || !elem_bytes) return EDV_ERR_ARG;
   if (index >= (int)ctx->plan.bufs.size()) return EDV_ERR_ARG;
-  auto it = ctx->plan.bufs.begin();
-  std::advance(it, index);
-  snprintf(name, name_cap, "%s", it->first.c_str());
-  *offset_bytes = it->second.off;
-  *bytes = it->second.bytes;
-  *elem_bytes = it->second.elem;
+  const Buf& b = ctx->plan.bufs[index];
+  snprintf(name, name_cap, "%s", b.name.c_str());
+  *offset_bytes = b.off;
+  *bytes = b.bytes;
+  *elem_bytes = b.elem;
   return EDV_OK;
 }
 

@@ -123,11 +123,11 @@ inline void upsample(Launch& L, int dtype, const void* x, void* y, int F, int h,
   L.check("upsample");
 }
 
-inline void resize_f32(Launch& L, const float* x, float* y, int F, int h, int w, int oh, int ow, int sigmoid = 0) {
+inline void resize_f32(Launch& L, const float* x, float* y, int F, int h, int w, int oh, int ow) {
   if (!L.ok()) return;
   long long total = (long long)F * oh * ow;
   L.note(0, ((double)F * h * w + (double)F * oh * ow) * 4);
-  edv::launch_k(resize_f32_kernel, dim3(nblk(total, 256)), dim3(256), 0, L.stream, x, y, F, h, w, oh, ow, sigmoid);
+  edv::launch_k(resize_f32_kernel, dim3(nblk(total, 256)), dim3(256), 0, L.stream, x, y, F, h, w, oh, ow);
   L.check("resize_f32");
 }
 
