@@ -71,8 +71,20 @@ __global__ void preprocess_patches_kernel(const void* __restrict__ src, T* __res
 //   frames[i].astype(float32) / 255 -> cv2.resize(INTER_CUBIC) -> HWC->CHW
 // (endodav.py:195; util/transform.py:109-113,139-158).  Restates OpenCV's float bicubic:
 // A = -0.75, half-pixel centres (fx = (dx + 0.5) * W/w - 0.5), border replicate, horizontal pass
-// then vertical pass, no anti-aliasing.  src uint8 [N,H,W,3] -> dst float32 [N,3,h,w].
+// then vertical pass, no anti-aliasing.  src uint8 [n_src,H,W,3] at element strides (st_n, st_y, st_x, st_c) -> dst float32
+// [N,3,h,w]; output frame i reads source frame frames.src[i] (frames.count == 0: frame i).  Consecutive threads take
+// consecutive dx, so one tap of a warp reads one run of about 32 * W / w source pixels along x: interleaved RGB for NHWC
+// (st_x = 3), the same run in each of the three planes for NCHW memory (st_x = 1).  DESIGN.md section 6 has the
+// measured time of both layouts.
 // ---------------------------------------------------------------------------------------
+// The source frame of every output frame of one launch, passed by value in the kernel parameters: no device
+// allocation, copy or synchronisation, and the host validates every entry before the launch.
+struct FrameTable {
+  static constexpr int kMax = 256;
+  int count;
+  int src[kMax];
+};
+
 __device__ __forceinline__ void cubic_coeffs(float x, float* c) {
   const float A = -0.75f;
   c[0] = ((A * (x + 1) - 5 * A) * (x + 1) + 8 * A) * (x + 1) - 4 * A;
@@ -82,7 +94,8 @@ __device__ __forceinline__ void cubic_coeffs(float x, float* c) {
 }
 
 __global__ void cubic_resize_u8_kernel(const uint8_t* __restrict__ src, float* __restrict__ dst, int N, int H, int W,
-                                       int h, int w) {
+                                       int h, int w, long long st_n, long long st_y, long long st_x, long long st_c,
+                                       const __grid_constant__ FrameTable frames) {
   const long long total = (long long)N * h * w;
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
@@ -105,17 +118,17 @@ __global__ void cubic_resize_u8_kernel(const uint8_t* __restrict__ src, float* _
     xs[k] = min(max(sx + k - 1, 0), W - 1);
     ys[k] = min(max(sy + k - 1, 0), H - 1);
   }
-  const uint8_t* base = src + (size_t)n * H * W * 3;
+  const uint8_t* base = src + (long long)(frames.count ? frames.src[n] : n) * st_n;
   float acc[3] = {0.f, 0.f, 0.f};
 #pragma unroll
   for (int r = 0; r < 4; ++r) {
-    const uint8_t* row = base + (size_t)ys[r] * W * 3;
+    const uint8_t* row = base + ys[r] * st_y;
     float hs[3] = {0.f, 0.f, 0.f};
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-      const uint8_t* px = row + xs[k] * 3;
+      const uint8_t* px = row + xs[k] * st_x;
 #pragma unroll
-      for (int c = 0; c < 3; ++c) hs[c] += ((float)px[c] / 255.0f) * cx[k];
+      for (int c = 0; c < 3; ++c) hs[c] += ((float)px[c * st_c] / 255.0f) * cx[k];
     }
 #pragma unroll
     for (int c = 0; c < 3; ++c) acc[c] += hs[c] * cy[r];

@@ -1288,14 +1288,52 @@ int edv_op_disp_head(int dtype, const void* X, const void* Wt, const float* bias
   return finish(L);
 }
 
+// Both cubic-resize entry points: index == nullptr is the identity in one launch; a table goes out in launches of at
+// most FrameTable::kMax output frames.  The arguments are validated by the callers.
+static void cubic_resize_u8(Launch& L, const uint8_t* src, int H, int W, long long sn, long long sy, long long sx,
+                            long long sc, const int64_t* index, int n, float* dst, int h, int w) {
+  const int per = index ? FrameTable::kMax : n;
+  for (int f0 = 0; f0 < n; f0 += per) {
+    const int cnt = std::min(per, n - f0);
+    FrameTable t = {};
+    if (index) {
+      t.count = cnt;
+      for (int i = 0; i < cnt; ++i) t.src[i] = (int)index[f0 + i];
+    }
+    const long long total = (long long)cnt * h * w;
+    L.note(0, (double)cnt * H * W * 3 + (double)total * 12);
+    cubic_resize_u8_kernel<<<nblk(total, 256), 256, 0, L.stream>>>(src, dst + (size_t)f0 * 3 * h * w, cnt, H, W, h, w, sn,
+                                                                   sy, sx, sc, t);
+    L.check("cubic_resize_u8");
+  }
+}
+
 int edv_op_cubic_resize_u8(const uint8_t* src, float* dst, int N, int H, int W, int h, int w, void* stream) {
   if (!src || !dst || N < 1 || H < 1 || W < 1 || h < 1 || w < 1) return EDV_ERR_ARG;
   Launch L;
   L.stream = (cudaStream_t)stream;
-  const long long total = (long long)N * h * w;
-  L.note(0, (double)N * H * W * 3 + (double)total * 12);
-  cubic_resize_u8_kernel<<<nblk(total, 256), 256, 0, L.stream>>>(src, dst, N, H, W, h, w);
-  L.check("cubic_resize_u8");
+  cubic_resize_u8(L, src, H, W, (long long)H * W * 3, (long long)W * 3, 3, 1, nullptr, N, dst, h, w);
+  return finish(L);
+}
+
+int edv_op_cubic_resize_u8_gather(const uint8_t* src, int n_src, int H, int W, long long stride_n, long long stride_y,
+                                  long long stride_x, long long stride_c, const int64_t* index_host, int n, float* dst, int h,
+                                  int w, void* stream) {
+  const char* fn = "edv_op_cubic_resize_u8_gather";
+  if (!src || !index_host || !dst) return set_err(nullptr, EDV_ERR_ARG, "%s: null src, index or dst", fn);
+  if (n < 1 || n_src < 1 || H < 1 || W < 1 || h < 1 || w < 1) return set_err(nullptr, EDV_ERR_ARG, "%s: empty problem", fn);
+  if (stride_n < 1 || stride_y < 1 || stride_x < 1 || stride_c < 1)
+    return set_err(nullptr, EDV_ERR_ARG, "%s: strides must be positive", fn);
+  // the last byte of the source must have a 64-bit offset (the kernel forms it as n*sn + y*sy + x*sx + c*sc)
+  const __int128 extent = (__int128)(n_src - 1) * stride_n + (__int128)(H - 1) * stride_y + (__int128)(W - 1) * stride_x +
+                          (__int128)2 * stride_c;
+  if (extent > (__int128)INT64_MAX) return set_err(nullptr, EDV_ERR_ARG, "%s: source extent overflows 64-bit offsets", fn);
+  for (int i = 0; i < n; ++i)
+    if (index_host[i] < 0 || index_host[i] >= n_src)
+      return set_err(nullptr, EDV_ERR_ARG, "%s: index[%d] = %lld outside [0, %d)", fn, i, (long long)index_host[i], n_src);
+  Launch L;
+  L.stream = (cudaStream_t)stream;
+  cubic_resize_u8(L, src, H, W, stride_n, stride_y, stride_x, stride_c, index_host, n, dst, h, w);
   return finish(L);
 }
 

@@ -16,14 +16,14 @@ DTYPES = {"fp32": EDV_F32, "f32": EDV_F32, "float32": EDV_F32, "bf16": EDV_BF16,
           "fp16": EDV_F16, "f16": EDV_F16, "float16": EDV_F16}
 TORCH_DTYPE = {EDV_F32: torch.float32, EDV_BF16: torch.bfloat16, EDV_F16: torch.float16}
 
-ABI_VERSION = 15  # must equal EDV_ABI_VERSION of include/endodav_b200.h (argtypes below are mirrored by hand)
+ABI_VERSION = 16  # must equal EDV_ABI_VERSION of include/endodav_b200.h (argtypes below are mirrored by hand)
 
 EXPORTS = [
     "edv_abi_version", "edv_create", "edv_destroy", "edv_last_error", "edv_set_weight", "edv_plan", "edv_forward", "edv_forward_u8",
     "edv_output_shape", "edv_launch_count", "edv_set_debug", "edv_debug_tap", "edv_plan_buffer", "edv_set_graph_mode", "edv_graph_count", "edv_graph_status", "edv_op_gemm",
     "edv_op_attention", "edv_op_temporal_attention", "edv_op_layernorm", "edv_op_groupnorm", "edv_op_upsample",
     "edv_op_resize_f32", "edv_profile", "edv_profile_reset", "edv_profile_collect", "edv_profile_get",
-    "edv_op_disp_head", "edv_op_cubic_resize_u8", "edv_op_stitch_window", "edv_op_stitch_plan",
+    "edv_op_disp_head", "edv_op_cubic_resize_u8", "edv_op_cubic_resize_u8_gather", "edv_op_stitch_window", "edv_op_stitch_plan",
     "edv_op_disp_to_depth", "edv_op_compute_errors", "edv_op_attention_timeline", "edv_op_linear_timeline", "edv_op_linear_residual_ln",
     "edv_op_preprocess_patches", "edv_op_tokens_to_patches", "edv_op_rowln_act", "edv_op_resblock_add", "edv_op_im2col3x3",
     "edv_op_geglu_pair", "edv_op_head_dot",
@@ -126,6 +126,7 @@ def load_library():
                                           ctypes.c_float, ctypes.c_float, vp, vp]
     lib.edv_op_layernorm.argtypes = [ci, vp, vp, vp, vp, ci, ci, ctypes.c_float, ci, ci, vp, ci, ci, vp]
     ll, cf = ctypes.c_longlong, ctypes.c_float
+    lib.edv_op_cubic_resize_u8_gather.argtypes = [vp, ci, ci, ci, ll, ll, ll, ll, vp, ci, vp, ci, ci, vp]
     lib.edv_op_preprocess_patches.argtypes = [ci, vp, ci, vp, ci, ci, ci, ci, ci, ci, vp]
     lib.edv_op_tokens_to_patches.argtypes = [ci, vp, vp, ll, ci, ci, ci, vp]
     lib.edv_op_rowln_act.argtypes = [ci, vp, vp, vp, vp, ll, ci, ci, cf, ci, vp]
@@ -446,15 +447,32 @@ def op_disp_head(X, Wt, bias, head_w, oh, ow, sig_sign=0.0):
     return out
 
 
-def op_cubic_resize_u8(frames_u8, h, w, out=None):
-    """uint8 [N,H,W,3] (device) -> float32 [N,3,h,w]: the reference's per-frame cv2 cubic resize of frame/255."""
+def op_cubic_resize_u8(frames_u8, h, w, out=None, index=None):
+    """uint8 [n_src,H,W,3] (device, any positive strides; a size-1 dimension may have any stride) -> float32 [N,3,h,w]: the reference's per-frame cv2 cubic resize of
+    frame/255.  index: the source frame of every output frame (N = len(index)); default every frame in order."""
+    import numpy as np
+
     lib = load_library()
-    N, H, W, _ = frames_u8.shape
+    if frames_u8.dtype != torch.uint8 or frames_u8.dim() != 4 or frames_u8.shape[3] != 3:
+        raise EndoDAVError("op_cubic_resize_u8: frames must be a uint8 [N,H,W,3] tensor, got %s %s"
+                           % (frames_u8.dtype, tuple(frames_u8.shape)))
+    n_src, H, W, _ = frames_u8.shape
+    if index is not None:
+        index = np.ascontiguousarray(index, dtype=np.int64).reshape(-1)
+    N = n_src if index is None else index.size
     if out is None:
         out = torch.empty(N, 3, h, w, dtype=torch.float32, device=frames_u8.device)
     elif tuple(out.shape) != (N, 3, h, w) or out.dtype != torch.float32 or not out.is_contiguous():
         raise EndoDAVError("op_cubic_resize_u8: out must be a contiguous float32 [%d,3,%d,%d] tensor" % (N, h, w))
-    _check(lib.edv_op_cubic_resize_u8(_ptr(frames_u8), _ptr(out), N, H, W, h, w, _stream()), None, "edv_op_cubic_resize_u8")
+    if index is None and frames_u8.is_contiguous():
+        _check(lib.edv_op_cubic_resize_u8(_ptr(frames_u8), _ptr(out), N, H, W, h, w, _stream()), None, "edv_op_cubic_resize_u8")
+        return out
+    if index is None:
+        index = np.arange(n_src, dtype=np.int64)
+    # the stride of a size-1 dimension is never used; torch may report any value for it
+    strides = [s if d > 1 else 1 for s, d in zip(frames_u8.stride(), frames_u8.shape)]
+    _check(lib.edv_op_cubic_resize_u8_gather(_ptr(frames_u8), n_src, H, W, *strides, index.ctypes.data_as(ctypes.c_void_p), N,
+                                             _ptr(out), h, w, _stream()), None, "edv_op_cubic_resize_u8_gather")
     return out
 
 

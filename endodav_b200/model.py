@@ -495,13 +495,33 @@ class endodac(endodav):
     def infer_video_depth(self, frames, batch_size=8, device='cuda'):
         """endodac.infer_video_depth (endodac.py:261-272): independent chunks of ``batch_size`` frames,
         each resized back to the frame size (bilinear, align_corners=True).  The uint8 -> float32/255
-        CHW conversion and the final resize run in the library's kernels."""
-        frames = np.ascontiguousarray(frames)
-        if frames.ndim != 4 or frames.shape[-1] != 3 or frames.dtype != np.uint8:
-            raise ValueError("frames must be uint8 [N,H,W,3]")
+        CHW conversion and the final resize run in the library's kernels.  A CUDA uint8 tensor of any positive strides is
+        read in place and gives a float32 tensor on its device (the contract of ``endodav.infer_video_depth``)."""
+        frames_dev = _video.frames_device(frames, device)
+        if frames_dev is None:
+            frames = np.ascontiguousarray(frames)
+            if frames.ndim != 4 or frames.shape[-1] != 3 or frames.dtype != np.uint8:
+                raise ValueError("frames must be uint8 [N,H,W,3]")
+        elif self._device() != frames_dev:
+            self.to(frames_dev)
         N, H, W, _ = frames.shape
         h, w = self.image_shape
         eng = self._ensure_engine(h // 14, w // 14)
+        if frames_dev is not None:
+            # one input and one resized buffer for every chunk: the forward's captured CUDA graph, keyed by their
+            # pointers, is replayed
+            out = torch.empty(N, H, W, dtype=torch.float32, device=frames_dev)
+            B = min(batch_size, N)
+            x_buf = torch.empty(B, 3, H, W, dtype=torch.float32, device=frames_dev)
+            r_buf = torch.empty(B, H, W, dtype=torch.float32, device=frames_dev)
+            with torch.cuda.device(frames_dev):
+                for c0 in range(0, N, batch_size):
+                    n = min(batch_size, N - c0)
+                    x = _engine.op_cubic_resize_u8(frames, H, W, out=x_buf[:n], index=np.arange(c0, c0 + n))
+                    eng.plan(n, 1, H, W, h, w)
+                    eng.forward(x, resize_to=(H, W), want_pyramid=False, resized_out=r_buf[:n])
+                    out[c0:c0 + n].copy_(r_buf[:n])
+            return out
         out = np.empty((N, H, W), dtype=np.float32)
         with torch.cuda.device(eng.device):
             for c0 in range(0, N, batch_size):

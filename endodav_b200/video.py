@@ -221,7 +221,8 @@ class _GpuStitcher:
     """Device-side replacement of ``stitch_windows`` (endodav.py:213-254): windows are pushed in order, each
     one is aligned and cross-faded by ``edv_op_stitch_window`` on the current stream (no host sync), and the
     frames it makes final are copied asynchronously into the pinned host array that ``finish`` returns
-    (float32 [n_frames,H,W]; torch's pinned-memory cache recycles it once the caller drops it).
+    (float32 [n_frames,H,W]; torch's pinned-memory cache recycles it once the caller drops it), or into the
+    caller's device tensor ``out`` (then no pinned memory is allocated and ``finish`` returns that tensor).
 
     Device memory is bounded: only a segment of ``8 + 22*chunk`` frames of the stitched sequence lives on the
     GPU (frames older than the 8-frame cross-fade tail are final and already on their way to the host); when
@@ -230,7 +231,7 @@ class _GpuStitcher:
 
     SEGMENT_BYTES = 256 << 20
 
-    def __init__(self, n_windows, n_frames, H, W, device, plan=None):
+    def __init__(self, n_windows, n_frames, H, W, device, plan=None, out=None):
         from . import engine as _engine
 
         self._op = _engine.op_stitch_window
@@ -246,7 +247,7 @@ class _GpuStitcher:
         self.plan = torch.from_numpy(plan).to(device)
         self.scratch = torch.empty(4 * int(plan[0] + plan[1]), dtype=torch.float32, device=device)
         self.scale_shift = torch.empty(n_windows, 2, dtype=torch.float32, device=device)
-        self.out = torch.empty(n_frames, H, W, dtype=torch.float32, pin_memory=True)
+        self.out = out if out is not None else torch.empty(n_frames, H, W, dtype=torch.float32, pin_memory=True)
 
     def push(self, win):
         """win: [32,H,W] float32 device tensor = window ``self.k`` resized to the frame size."""
@@ -266,7 +267,7 @@ class _GpuStitcher:
     def finish(self):
         assert self.k == self.nwin
         torch.cuda.current_stream().synchronize()
-        return self.out.numpy()
+        return self.out if self.out.is_cuda else self.out.numpy()
 
 
 def _stitch_plan_or_none(H, W):
@@ -288,25 +289,58 @@ def _dist():
     return None, 0, 1
 
 
+def frames_device(frames, device):
+    """The device the driver runs on for CUDA frames, which is theirs, or None for host frames.  CUDA frames must be a
+    uint8 tensor of logical shape [N,H,W,3] with positive strides (any layout, but no broadcast view); ``device`` may be
+    "cuda" without an index or name the same device."""
+    if not (isinstance(frames, torch.Tensor) and frames.is_cuda):
+        return None
+    if frames.dtype != torch.uint8 or frames.dim() != 4 or frames.shape[3] != 3:
+        raise ValueError("CUDA frames must be a uint8 [N,H,W,3] tensor, got %s %s" % (frames.dtype, tuple(frames.shape)))
+    if any(st < 1 and d > 1 for st, d in zip(frames.stride(), frames.shape)):
+        # a broadcast view (e.g. one grayscale plane expanded to three channels): the resize reads positive strides
+        raise ValueError("CUDA frames must not be a broadcast view (strides %s); materialise it first" % (frames.stride(),))
+    want = torch.device(device)
+    if want.type != "cuda" or (want.index is not None and want != frames.device):
+        raise ValueError("frames are on %s but device=%r names another device" % (frames.device, device))
+    return frames.device
+
+
 def infer_video_depth(model, frames, device="cuda", forward_window=None, distributed=True):
     """frames: uint8 [N,H,W,3] -> float32 [N,H,W] on rank 0 (other ranks return None).
 
+    Host frames (a numpy array, or anything numpy can read) give a numpy array.  A CUDA uint8 tensor of any positive strides
+    (an NCHW decoder batch as ``x.permute(0, 2, 3, 1)``, frame slices, crops) is read in place on its own device and
+    gives a contiguous float32 tensor there, bit-identical to the host path on the same frames.
+
     ``forward_window(clip[1,32,3,h,w] float32 tensor, (H,W)) -> [32,H,W] float32 tensor`` can be
-    injected by tests (index/stitch logic on CPU); by default it is the model's CUDA engine
+    injected by tests (index/stitch logic on CPU, host frames only); by default it is the model's CUDA engine
     with the final resize fused into the same launch sequence."""
-    frames = np.ascontiguousarray(frames)
+    frames_dev = frames_device(frames, device)
+    if frames_dev is None:
+        frames = np.ascontiguousarray(frames)
+    elif forward_window is not None:
+        raise ValueError("forward_window takes host frames only")
     if frames.ndim != 4 or frames.shape[-1] != 3:
-        raise ValueError("frames must be [N,H,W,3], got %s" % (frames.shape,))
+        raise ValueError("frames must be [N,H,W,3], got %s" % (tuple(frames.shape),))
     n, H, W = frames.shape[:3]
     ih, iw = model.image_shape
     new_w, new_h = resize_target(W, H, iw, ih)
-    cache = _FrameCache(frames, new_w, new_h)
+    cache = _FrameCache(frames, new_w, new_h) if frames_dev is None else None
+
+    def deliver(result):
+        """the stitched frames of device input go back to their device in one upload"""
+        return torch.from_numpy(result).to(frames_dev) if frames_dev is not None else result
+
+    def sink():
+        """the device tensor that receives the stitched frames of device input; None: the stitcher's pinned host array"""
+        return torch.empty(n, H, W, dtype=torch.float32, device=frames_dev) if frames_dev is not None else None
     dist, rank, world = _dist() if distributed else (None, 0, 1)
     nwin = num_windows(n)
     mine = shard_windows(nwin, rank, world)
 
     if forward_window is None:
-        dev = torch.device(device)
+        dev = frames_dev if frames_dev is not None else torch.device(device)
         if dev.type != "cuda":
             raise RuntimeError("endodav_b200 has no CPU path (device=%r)" % (device,))
         if dev.index is None:
@@ -316,15 +350,16 @@ def infer_video_depth(model, frames, device="cuda", forward_window=None, distrib
         eng = model._ensure_engine(ih // 14, iw // 14)
         from . import engine as _engine
 
-        gpu_pre = os.environ.get("ENDODAV_PREPROCESS", "gpu").lower() != "host"
-        if frames.dtype != np.uint8:
+        gpu_pre = frames_dev is not None or os.environ.get("ENDODAV_PREPROCESS", "gpu").lower() != "host"
+        if frames_dev is None and frames.dtype != np.uint8:
             # the reference accepts any dtype through ``.astype(np.float32) / 255`` (endodav.py:195); the GPU cubic
             # resize is written for uint8 frames, so other dtypes take the reference's host preprocessing path
             gpu_pre = False
         # two pinned staging buffers: the host fills window j+1 while the GPU runs window j.
         # gpu_pre (default): the raw uint8 frames of the window are uploaded (4x fewer bytes than the
         # resized float clip) and the reference's /255 + cv2 INTER_CUBIC resize + HWC->CHW runs in a
-        # CUDA kernel (edv_op_cubic_resize_u8); ENDODAV_PREPROCESS=host keeps the reference's host path.
+        # CUDA kernel (edv_op_cubic_resize_u8); ENDODAV_PREPROCESS=host keeps the reference's host path for host frames.
+        # Device frames are neither staged nor uploaded: the resize reads them from the caller's tensor.
         # Windows are independent, so WB of them go through the network as one [WB,32,...] clip batch (the
         # engine's batched result is bit-identical to the clips run one by one, test_clip_batch_sweep_*):
         # at 224x280 four windows take 9.1 ms instead of 4 x 3.7 ms.
@@ -344,7 +379,7 @@ def infer_video_depth(model, frames, device="cuda", forward_window=None, distrib
         if gpu_pre:
             # the staging buffers hold raw frames: bound them by the FRAME size too (256 MB each; 1080p -> one window)
             WB = max(1, min(WB, (256 << 20) // (INFER_LEN * H * W * 3)))
-            stager = _Stager(frames, n, mine, WB, H, W)
+            stager = _Stager(frames, n, mine, WB, H, W) if frames_dev is None else None
             pinned = None
         else:
             pinned = [torch.empty(WB, INFER_LEN, 3, new_h, new_w, dtype=torch.float32, pin_memory=True) for _ in range(2)]
@@ -353,7 +388,8 @@ def infer_video_depth(model, frames, device="cuda", forward_window=None, distrib
         # device staging is allocated once and reused (two slots): besides saving allocator traffic this keeps the
         # external pointers of edv_forward stable, so the captured CUDA graph of the forward is replayed for every
         # window batch instead of re-launching ~190 kernels from the host
-        dev_u8 = [torch.empty(WB * INFER_LEN, H, W, 3, dtype=torch.uint8, device=dev) for _ in range(2)] if gpu_pre else None
+        dev_u8 = ([torch.empty(WB * INFER_LEN, H, W, 3, dtype=torch.uint8, device=dev) for _ in range(2)]
+                  if stager is not None else None)
         dev_x = [torch.empty(WB * INFER_LEN, 3, new_h, new_w, dtype=torch.float32, device=dev) for _ in range(2)]
         dev_out = [None, None]
 
@@ -363,26 +399,30 @@ def infer_video_depth(model, frames, device="cuda", forward_window=None, distrib
             slot = calls[0] & 1
             calls[0] += 1
             x = dev_x[slot][: nb * INFER_LEN]
-            if gpu_pre:
-                pslot, buf = stager.fetch(j, nb)
-                xu8 = dev_u8[slot][: nb * INFER_LEN]
-                xu8.copy_(buf, non_blocking=True)
-            else:
-                if copied[slot] is not None:
-                    copied[slot].synchronize()  # the earlier H2D copy out of this buffer has finished
-                buf = pinned[slot]
+            if frames_dev is not None:
                 idx = np.concatenate([window_frame_indices(mine[j + b], n) for b in range(nb)])
-                flat = buf.view(WB * INFER_LEN, 3, new_h, new_w)
-                for i, src in enumerate(idx):
-                    flat[i].copy_(torch.from_numpy(cache.get(int(src))))
-                x.copy_(flat[: nb * INFER_LEN], non_blocking=True)
-            ev = torch.cuda.Event()
-            ev.record()
-            if gpu_pre:
-                stager.uploaded(pslot, ev)
-                _engine.op_cubic_resize_u8(xu8, new_h, new_w, out=x)
+                _engine.op_cubic_resize_u8(frames, new_h, new_w, out=x, index=idx)
             else:
-                copied[slot] = ev
+                if gpu_pre:
+                    pslot, buf = stager.fetch(j, nb)
+                    xu8 = dev_u8[slot][: nb * INFER_LEN]
+                    xu8.copy_(buf, non_blocking=True)
+                else:
+                    if copied[slot] is not None:
+                        copied[slot].synchronize()  # the earlier H2D copy out of this buffer has finished
+                    buf = pinned[slot]
+                    idx = np.concatenate([window_frame_indices(mine[j + b], n) for b in range(nb)])
+                    flat = buf.view(WB * INFER_LEN, 3, new_h, new_w)
+                    for i, src in enumerate(idx):
+                        flat[i].copy_(torch.from_numpy(cache.get(int(src))))
+                    x.copy_(flat[: nb * INFER_LEN], non_blocking=True)
+                ev = torch.cuda.Event()
+                ev.record()
+                if gpu_pre:
+                    stager.uploaded(pslot, ev)
+                    _engine.op_cubic_resize_u8(xu8, new_h, new_w, out=x)
+                else:
+                    copied[slot] = ev
             if out is None:
                 if dev_out[slot] is None:
                     dev_out[slot] = torch.empty(WB * INFER_LEN, H, W, dtype=torch.float32, device=dev)
@@ -395,7 +435,7 @@ def infer_video_depth(model, frames, device="cuda", forward_window=None, distrib
             # (edv_op_stitch_window, no host sync); the frames a window makes final are copied back through a
             # small pinned ring while the next windows run.
             with torch.cuda.device(dev):
-                st = _GpuStitcher(nwin, n, H, W, dev, splan)
+                st = _GpuStitcher(nwin, n, H, W, dev, splan, sink())
                 for j in range(0, nwin, WB):
                     nb = min(WB, nwin - j)
                     d = launch(j, nb).view(nb, INFER_LEN, H, W)
@@ -426,7 +466,7 @@ def infer_video_depth(model, frames, device="cuda", forward_window=None, distrib
                         arr = ring[j % RING].numpy()
                         yield arr.copy() if j == 0 else arr   # window 0's frames are kept by reference in the output list
 
-            return stitch_windows(stream(), n)
+            return deliver(stitch_windows(stream(), n))
 
         per = (nwin + world - 1) // world
         if gpu_stitch and os.environ.get("ENDODAV_GATHER", "rounds").lower() != "single":
@@ -439,8 +479,9 @@ def infer_video_depth(model, frames, device="cuda", forward_window=None, distrib
                 side = torch.cuda.Stream(device=dev) if rank == 0 else None
                 st = None
                 if rank == 0:
+                    dest = sink()                     # allocated on this stream, which hands the result to the caller
                     with torch.cuda.stream(side):
-                        st = _GpuStitcher(nwin, n, H, W, dev, splan)
+                        st = _GpuStitcher(nwin, n, H, W, dev, splan, dest)
                 # Three rotating sets of gather buffers (round r uses set r % 3): bounded memory however long the video,
                 # and stable pointers, so the forward's captured CUDA graph is replayed.  Set r % 3 is reused by round
                 # r + 3 once (a) this rank has waited for round r's gather (its `send` is free) and (b) on rank 0 the
@@ -545,10 +586,10 @@ def infer_video_depth(model, frames, device="cuda", forward_window=None, distrib
         return None
     if forward_window is None and gpu_stitch:
         with torch.cuda.device(local_t.device):
-            st = _GpuStitcher(nwin, n, H, W, local_t.device, splan)
+            st = _GpuStitcher(nwin, n, H, W, local_t.device, splan, sink())
             for k in range(nwin):
                 st.push(gathered[k % world][k // world])
             return st.finish()
     host = [g.cpu().numpy() for g in gathered]
     wins = [host[k % world][k // world] for k in range(nwin)]
-    return stitch_windows(wins, n)
+    return deliver(stitch_windows(wins, n))

@@ -30,7 +30,7 @@ typedef struct edv_ctx edv_ctx;
 /* Bumped whenever an entry point's argument list or a struct layout changes.  The ctypes host
  * (endodav_b200/engine.py) mirrors the signatures by hand, so it refuses a library whose
  * edv_abi_version() differs from its own constant instead of calling it with a stale layout. */
-#define EDV_ABI_VERSION 15
+#define EDV_ABI_VERSION 16
 int edv_abi_version(void);
 
 enum edv_status {
@@ -237,6 +237,16 @@ int edv_op_disp_head(int dtype, const void* X, const void* Wt, const float* bias
  * cv2.resize(frame / 255, (w,h), INTER_CUBIC) in CHW order (OpenCV's float bicubic: A=-0.75, half-pixel
  * centres, replicated border).  Replaces endodav.py:195 + util/transform.py:109-113,139-158. */
 int edv_op_cubic_resize_u8(const uint8_t* src, float* dst, int N, int H, int W, int h, int w, void* stream);
+
+/* edv_op_cubic_resize_u8 of a strided source through a frame-index table: dst float32 [n,3,h,w], output frame i is
+ * source frame index_host[i].  Source element (f, y, x, c) of the n_src frames of H x W x 3 uint8 sits at
+ * src[f*stride_n + y*stride_y + x*stride_x + c*stride_c] (strides in elements = bytes): contiguous NHWC, an NCHW batch
+ * viewed as [N,H,W,3], frame slices and crops are all read in place.  index_host is host memory, read during the call
+ * (it travels in the kernel parameters, at most 256 entries per launch).  Returns EDV_ERR_ARG before any launch for a
+ * null pointer, n < 1, an index outside [0, n_src), a stride < 1 or a source extent beyond 64-bit byte offsets. */
+int edv_op_cubic_resize_u8_gather(const uint8_t* src, int n_src, int H, int W, long long stride_n, long long stride_y,
+                                  long long stride_x, long long stride_c, const int64_t* index_host, int n, float* dst, int h,
+                                  int w, void* stream);
 
 /* LayerNorm over the last dim: X float32 -> Y[M,D] `dtype` (M output rows), then + add[(m / add_div) % add_mod][0..D-1]
  * when add is not NULL (the temporal modules' sinusoidal PE of row m's frame: add_div = hw, add_mod = T).
