@@ -1281,10 +1281,20 @@ int edv_op_temporal_attention(int dtype, const void* qkv, void* out, int B, int 
 }
 
 int edv_op_disp_head(int dtype, const void* X, const void* Wt, const float* bias, const float* head_w, float* out, int F,
-                     int H1, int W1, int OH, int OW, int Cin, float sig_sign, void* stream) {
+                     int H1, int W1, int OH, int OW, int Cin, float sig_sign, char* kernel, int kernel_cap, void* stream) {
+  if (kernel && kernel_cap > 0) kernel[0] = 0;
+  if (dtype != EDV_BF16 && dtype != EDV_F16) return set_err(nullptr, EDV_ERR_ARG, "edv_op_disp_head: bad dtype %d (bf16 or f16)", dtype);
+  if (!X || !Wt || !bias || !head_w || !out) return set_err(nullptr, EDV_ERR_ARG, "edv_op_disp_head: null X, Wt, bias, head_w or out");
+  // the producers and the weight staging read X and Wt with 16-byte vector loads
+  if (!aligned16(X) || !aligned16(Wt)) return set_err(nullptr, EDV_ERR_ARG, "edv_op_disp_head: X and Wt must be 16-byte aligned");
+  if (Cin != 32 && Cin != 128) return set_err(nullptr, EDV_ERR_ARG, "edv_op_disp_head: Cin %d (32 or 128)", Cin);
+  // H1 or W1 = 0 would clamp the source row / column to -1 and read before X
+  if (F < 1 || H1 < 1 || W1 < 1 || OH < 1 || OW < 1)
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_disp_head: F, H1, W1, OH and OW must be at least 1");
   Launch L;
   L.stream = (cudaStream_t)stream;
   head_fused(L, dtype, X, Wt, bias, head_w, out, F, H1, W1, OH, OW, Cin, sig_sign);
+  if (kernel && kernel_cap > 0) snprintf(kernel, kernel_cap, "%s", L.kernel.c_str());
   return finish(L);
 }
 

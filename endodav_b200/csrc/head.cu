@@ -10,10 +10,11 @@ void launch_head_fused(Launch& L, const void* x, const void* w, const float* bia
                        int H1, int W1, int OH, int OW, float sig_sign) {
   using namespace tc;
   constexpr auto kern = head_fused_kernel<T, CIN>;
-  smem_opt_in<kern>((int)hf_smem_bytes<CIN>());
   const int tiles_x = (OW + HF_TW - 1) / HF_TW, tiles_y = (OH + HF_TH - 1) / HF_TH;
   const long long total = (long long)F * tiles_x * tiles_y;
   if (total > 0x7fffffffLL) return L.fail(EDV_ERR_ARG, "head_fused: too many tiles");
+  smem_opt_in<kern>((int)hf_smem_bytes<CIN>());
+  L.kernel = std::string("head_fused<") + (std::is_same<T, bf16>::value ? "bf16" : "f16") + ",CIN=" + std::to_string(CIN) + ">";
   const int grid = (int)std::min<long long>(total, num_sms());
   // algorithmic bytes: the low-resolution map once + one float per output pixel (SURVEY.md 8(d))
   L.note(2.0 * F * OH * OW * 32.0 * (9 * CIN + 1), (double)F * H1 * W1 * CIN * sizeof(T) + (double)F * OH * OW * 4);
@@ -22,7 +23,7 @@ void launch_head_fused(Launch& L, const void* x, const void* w, const float* bia
   L.check("head_fused");
 }
 
-bool head_fused_supported(int dtype, int Cin) { return dtype != EDV_F32 && (Cin == 32 || Cin == 128); }
+bool head_fused_supported(int dtype, int Cin) { return (dtype == EDV_BF16 || dtype == EDV_F16) && (Cin == 32 || Cin == 128); }
 
 void head_fused(Launch& L, int dtype, const void* x, const void* w, const float* bias, const float* head_w,
                        float* out, int F, int H1, int W1, int OH, int OW, int Cin, float sig_sign) {

@@ -82,9 +82,9 @@ struct Launch {
   std::string err;
   Profiler* prof = nullptr;
   std::string tag;       // which call site of the forward graph the next launches belong to
-  std::string kernel;    // the GEMM or attention instance launched last, e.g. "gemm_tc<BN=32,BK=64,kind=0x9,tma=0>",
-                         // "temporal_attention_mma<HD=24,PB=2>", "flash_attention_tc<bf16>"
-                         // (edv_op_gemm, edv_op_temporal_attention, edv_op_attention)
+  std::string kernel;    // the GEMM, attention or head instance launched last, e.g. "gemm_tc<BN=32,BK=64,kind=0x9,tma=0>",
+                         // "temporal_attention_mma<HD=24,PB=2>", "flash_attention_tc<bf16>", "head_fused<bf16,CIN=128>"
+                         // (edv_op_gemm, edv_op_temporal_attention, edv_op_attention, edv_op_disp_head)
   double nflops = 0, nbytes = 0;  // algorithmic work of the next launch (set by the launcher)
 
   void note(double flops, double bytes) {

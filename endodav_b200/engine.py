@@ -16,7 +16,7 @@ DTYPES = {"fp32": EDV_F32, "f32": EDV_F32, "float32": EDV_F32, "bf16": EDV_BF16,
           "fp16": EDV_F16, "f16": EDV_F16, "float16": EDV_F16}
 TORCH_DTYPE = {EDV_F32: torch.float32, EDV_BF16: torch.bfloat16, EDV_F16: torch.float16}
 
-ABI_VERSION = 16  # must equal EDV_ABI_VERSION of include/endodav_b200.h (argtypes below are mirrored by hand)
+ABI_VERSION = 17  # must equal EDV_ABI_VERSION of include/endodav_b200.h (argtypes below are mirrored by hand)
 
 EXPORTS = [
     "edv_abi_version", "edv_create", "edv_destroy", "edv_last_error", "edv_set_weight", "edv_plan", "edv_forward", "edv_forward_u8",
@@ -117,7 +117,7 @@ def load_library():
     lib.edv_op_linear_timeline.argtypes = [ci, vp, vp, vp, vp, ci, ci, ci, ci, vp, vp]
     lib.edv_op_attention_timeline.argtypes = [ci, vp, vp, ci, ci, ci, vp, vp]
     lib.edv_op_temporal_attention.argtypes = [ci, vp, vp, ci, ci, ci, ci, vp, ctypes.c_char_p, ci, vp]
-    lib.edv_op_disp_head.argtypes = [ci, vp, vp, vp, vp, vp, ci, ci, ci, ci, ci, ci, ctypes.c_float, vp]
+    lib.edv_op_disp_head.argtypes = [ci, vp, vp, vp, vp, vp, ci, ci, ci, ci, ci, ci, ctypes.c_float, ctypes.c_char_p, ci, vp]
     lib.edv_op_cubic_resize_u8.argtypes = [vp, vp, ci, ci, ci, ci, ci, vp]
     lib.edv_op_stitch_window.argtypes = [vp, ci, ci, ci, vp, vp, ci, vp, vp, vp]
     lib.edv_op_stitch_plan.argtypes = [ci, ci, vp, ctypes.c_longlong]
@@ -438,13 +438,21 @@ def op_temporal_attention(qkv, B, T, hw, C, rope=None):
     return op_temporal_attention_kernel(qkv, B, T, hw, C, rope)[0]
 
 
-def op_disp_head(X, Wt, bias, head_w, oh, ow, sig_sign=0.0):
+def op_disp_head_kernel(X, Wt, bias, head_w, oh, ow, sig_sign=0.0, out=None):
+    """-> (out [F, oh, ow] float32, name of the kernel instance that ran, e.g. "head_fused<bf16,CIN=128>").  X: NHWC
+    [F, H1, W1, Cin]; out: optional caller-owned float32 buffer whose first F*oh*ow elements receive the result."""
     lib = load_library()
     F, H1, W1, Cin = X.shape
-    out = torch.empty(F, oh, ow, dtype=torch.float32, device=X.device)
+    if out is None:
+        out = torch.empty(F, oh, ow, dtype=torch.float32, device=X.device)
+    name = ctypes.create_string_buffer(128)
     _check(lib.edv_op_disp_head(_dt(X), _ptr(X), _ptr(Wt), _ptr(bias), _ptr(head_w), _ptr(out), F, H1, W1, oh, ow, Cin,
-                                ctypes.c_float(sig_sign), _stream()), None, "edv_op_disp_head")
-    return out
+                                ctypes.c_float(sig_sign), name, 128, _stream()), None, "edv_op_disp_head")
+    return out, name.value.decode()
+
+
+def op_disp_head(X, Wt, bias, head_w, oh, ow, sig_sign=0.0):
+    return op_disp_head_kernel(X, Wt, bias, head_w, oh, ow, sig_sign)[0]
 
 
 def op_cubic_resize_u8(frames_u8, h, w, out=None, index=None):

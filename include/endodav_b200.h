@@ -30,7 +30,7 @@ typedef struct edv_ctx edv_ctx;
 /* Bumped whenever an entry point's argument list or a struct layout changes.  The ctypes host
  * (endodav_b200/engine.py) mirrors the signatures by hand, so it refuses a library whose
  * edv_abi_version() differs from its own constant instead of calling it with a stale layout. */
-#define EDV_ABI_VERSION 16
+#define EDV_ABI_VERSION 17
 int edv_abi_version(void);
 
 enum edv_status {
@@ -229,9 +229,12 @@ int edv_op_temporal_attention(int dtype, const void* qkv, void* out, int B, int 
 /* Fused disparity-head tail on an NHWC map X[F,H1,W1,Cin] (16-bit, Cin in {32,128}):
  * bilinear resize (align_corners=True) to (OH,OW) -> 3x3 conv Wt[32, 9*Cin] + bias -> ReLU ->
  * 1x1 conv head_w[0..31] + head_w[32] -> ReLU (sig_sign == 0) or sigmoid(sig_sign * x) -> out[F,OH,OW] f32.
+ * `kernel` (may be NULL) receives the instance that ran, e.g. "head_fused<bf16,CIN=128>".  EDV_ERR_ARG before any
+ * launch for a NULL X, Wt, bias, head_w or out, X or Wt not 16-byte aligned, a dtype other than bf16 / f16, Cin not
+ * in {32,128}, F, H1, W1, OH or OW below 1, and more than 2^31 - 1 output tiles of 16 x 8 pixels.
  * Replaces dpt_pyramid.py:90-93 + dpt.py:118-124 (output_conv2); layers.py:211-217 (HeadDepth). */
 int edv_op_disp_head(int dtype, const void* X, const void* Wt, const float* bias, const float* head_w, float* out, int F,
-                     int H1, int W1, int OH, int OW, int Cin, float sig_sign, void* stream);
+                     int H1, int W1, int OH, int OW, int Cin, float sig_sign, char* kernel, int kernel_cap, void* stream);
 
 /* Host preprocessing of infer_video_depth on the GPU: uint8 RGB frames [N,H,W,3] -> float32 [N,3,h,w] =
  * cv2.resize(frame / 255, (w,h), INTER_CUBIC) in CHW order (OpenCV's float bicubic: A=-0.75, half-pixel

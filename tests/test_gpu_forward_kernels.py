@@ -361,7 +361,10 @@ COVERED = {
     "gemm_bres_kernel": ["test_gpu_ops::test_linear_kernels_agree_bitwise", "test_gpu_epilogues::test_epilogue_matches_reference"],
     "conv3x3_halo_kernel": ["test_gpu_ops::test_conv3x3_16bit", "test_gpu_epilogues::test_epilogue_matches_reference"],
     "gemm_ln_kernel": ["test_gpu_ops::test_linear_residual_layernorm"],
-    "head_fused_kernel": ["test_gpu_ops::test_disp_head_fused"],
+    "head_fused_kernel": ["test_gpu_head::test_head_dpt_shapes", "test_gpu_head::test_head_conv_head_shapes",
+                          "test_gpu_head::test_head_tails", "test_gpu_head::test_head_small_shapes",
+                          "test_gpu_head::test_head_grid_sizes", "test_gpu_head::test_head_frames_are_independent",
+                          "test_gpu_head::test_head_poisoned_neighbour"],
     "stitch_leaf_kernel": ["test_gpu_stitch::test_stitch_matches_numpy_chain"],
     "stitch_tree_solve_kernel": ["test_gpu_stitch::test_stitch_matches_numpy_chain"],
     "stitch_identity_kernel": ["test_gpu_stitch::test_stitch_matches_numpy_chain"],

@@ -267,28 +267,6 @@ def test_pyramid_downscale_matches_scale_factor_half():
     assert float((got - ref).abs().max()) <= 1e-5
 
 
-# ---- fused disparity-head tail ---------------------------------------------------------------------
-@pytest.mark.parametrize("dtype", DT16)
-@pytest.mark.parametrize("Fr,h,w,oh,ow,C,sig", [(2, 40, 56, 70, 98, 32, 0.0), (1, 128, 160, 224, 280, 32, 0.0),
-                                                 (1, 16, 24, 28, 42, 128, 0.0), (2, 9, 13, 18, 26, 32, 1.0),
-                                                 (1, 5, 5, 5, 5, 32, -1.0), (1, 296, 296, 518, 518, 32, 0.0)])
-def test_disp_head_fused(dtype, Fr, h, w, oh, ow, C, sig):
-    """upsample -> conv3x3 -> ReLU -> 1x1 -> ReLU|sigmoid in one kernel vs. the same chain in fp32 torch
-    (the upsampled map is rounded to the 16-bit dtype exactly where the unfused path rounds it)."""
-    X = _rand((Fr, h, w, C), dtype, 31)
-    Wt = _rand((32, 9 * C), dtype, 32, (9 * C) ** -0.5)
-    b = _rand((32,), torch.float32, 33, 0.1)
-    hw = _rand((33,), torch.float32, 34, 0.3)
-    got = eng.op_disp_head(X, Wt, b, hw, oh, ow, sig)
-    up = F.interpolate(X.float().permute(0, 3, 1, 2), size=(oh, ow), mode="bilinear", align_corners=True).to(dtype).double()
-    w4 = Wt.double().reshape(32, 3, 3, C).permute(0, 3, 1, 2)
-    y = F.relu(F.conv2d(up, w4, b.double(), padding=1))
-    s = (y * hw[:32].double().view(1, 32, 1, 1)).sum(1) + hw[32].double()
-    ref = (F.relu(s) if sig == 0.0 else torch.sigmoid(sig * s)).float()
-    err = (got - ref).abs()
-    assert float(err.max()) <= 2e-3 * max(1.0, float(ref.abs().max())), float(err.max())
-
-
 def test_linear_kernels_agree_bitwise():
     """The tcgen05 linear kernels that shape selects between must agree bit for bit on the same operands (same fp32
     accumulation order per output element), for act = none and ReLU:
