@@ -4,6 +4,8 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cfloat>
+#include <climits>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -1228,13 +1230,29 @@ int edv_op_linear_timeline(int dtype, const void* A, const void* W, const float*
 }
 
 int edv_op_linear_residual_ln(int dtype, const void* A, const void* W, const float* bias, float* x_inout, const float* gamma,
-                              const float* beta, float eps, void* xn_out, int M, int N, int K, long long* timeline_dev, void* stream) {
-  if (!A || !W || !x_inout || M < 1) return EDV_ERR_ARG;
+                              const float* beta, float eps, void* xn_out, int M, int N, int K, long long* timeline_dev, char* kernel,
+                              int kernel_cap, void* stream) {
+  if (kernel && kernel_cap > 0) kernel[0] = 0;
+  if (dtype != EDV_BF16 && dtype != EDV_F16)
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_linear_residual_ln: bad dtype %d (bf16 or f16)", dtype);
+  if (!A || !W || !x_inout) return set_err(nullptr, EDV_ERR_ARG, "edv_op_linear_residual_ln: null A, W or x");
+  // A, W, x and xn are the base addresses of TMA tensor maps
+  if (!aligned16(A) || !aligned16(W) || !aligned16(x_inout) || !aligned16(xn_out))
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_linear_residual_ln: A, W, x and xn must be 16-byte aligned");
+  // a partial set would silently skip the LayerNorm (or normalise into nothing)
+  const int do_ln = (gamma && beta && xn_out) ? 1 : 0;
+  if (!do_ln && (gamma || beta || xn_out))
+    return set_err(nullptr, EDV_ERR_ARG, "edv_op_linear_residual_ln: gamma, beta and xn must be all set or all NULL");
+  // the kernel counts tiles as (M + 127) / 128 in int
+  if (M < 1 || M > INT_MAX - 127) return set_err(nullptr, EDV_ERR_ARG, "edv_op_linear_residual_ln: M %d out of range", M);
+  if (N != 384) return set_err(nullptr, EDV_ERR_ARG, "edv_op_linear_residual_ln: N %d (384 only)", N);
+  if (K < 64 || K % 64) return set_err(nullptr, EDV_ERR_ARG, "edv_op_linear_residual_ln: K %d (a positive multiple of 64)", K);
+  if (!(eps >= 0.f && eps <= FLT_MAX)) return set_err(nullptr, EDV_ERR_ARG, "edv_op_linear_residual_ln: eps must be finite and >= 0");
   Launch L;
   L.stream = (cudaStream_t)stream;
-  const int do_ln = (gamma && beta && xn_out) ? 1 : 0;
   if (timeline_dev && cudaMemsetAsync(timeline_dev, 0, 64 * sizeof(long long), L.stream) != cudaSuccess) return EDV_ERR_CUDA;
   gemm_ln(L, dtype, A, W, bias, x_inout, xn_out, gamma, beta, eps, M, N, K, do_ln, timeline_dev);
+  if (kernel && kernel_cap > 0) snprintf(kernel, kernel_cap, "%s", L.kernel.c_str());
   return finish(L);
 }
 

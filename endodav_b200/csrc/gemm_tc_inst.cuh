@@ -176,6 +176,7 @@ void launch_gemm_ln(Launch& L, int dtype, const void* A, const void* W, const fl
   smem_opt_in<kern>((int)GL_SMEM);
   const int m_tiles = (M + GT_BM - 1) / GT_BM;
   const int grid = 2 * std::min(m_tiles, num_sms() / 2);   // clusters of two CTAs, one 128-row tile per pair at a time
+  L.kernel = std::string("gemm_ln<") + (std::is_same<T, bf16>::value ? "bf16" : "f16") + ">";
   // algorithmic work: 2 M N K; bytes: A + W + the fp32 stream read and written once + xn written once
   L.note(2.0 * M * GL_N * K, ((double)M * K + (double)GL_N * K) * 2 + (double)M * GL_N * (8 + (do_ln ? 2 : 0)));
   edv::launch_k(kern, dim3(grid), dim3(GL_THREADS), GL_SMEM, L.stream, tmA, tmB, tmX, tmXn, bias, gamma, beta, eps, M, K, m_tiles, do_ln, tim);
@@ -184,7 +185,7 @@ void launch_gemm_ln(Launch& L, int dtype, const void* A, const void* W, const fl
 
 #ifdef EDV_GEMM_TU_LN
 bool gemm_ln_supported(int dtype, int N, int K) {
-  return dtype != EDV_F32 && N == tc::GL_N && K % 64 == 0 && K >= 64;
+  return (dtype == EDV_BF16 || dtype == EDV_F16) && N == tc::GL_N && K % 64 == 0 && K >= 64;
 }
 void gemm_ln(Launch& L, int dtype, const void* A, const void* W, const float* bias, float* x, void* xn, const float* gamma,
              const float* beta, float eps, int M, int N, int K, int do_ln, long long* tim) {

@@ -16,7 +16,7 @@ DTYPES = {"fp32": EDV_F32, "f32": EDV_F32, "float32": EDV_F32, "bf16": EDV_BF16,
           "fp16": EDV_F16, "f16": EDV_F16, "float16": EDV_F16}
 TORCH_DTYPE = {EDV_F32: torch.float32, EDV_BF16: torch.bfloat16, EDV_F16: torch.float16}
 
-ABI_VERSION = 17  # must equal EDV_ABI_VERSION of include/endodav_b200.h (argtypes below are mirrored by hand)
+ABI_VERSION = 18  # must equal EDV_ABI_VERSION of include/endodav_b200.h (argtypes below are mirrored by hand)
 
 EXPORTS = [
     "edv_abi_version", "edv_create", "edv_destroy", "edv_last_error", "edv_set_weight", "edv_plan", "edv_forward", "edv_forward_u8",
@@ -113,7 +113,7 @@ def load_library():
                                     ctypes.POINTER(ctypes.c_double)]
     lib.edv_op_gemm.argtypes = [ci, ci, ctypes.POINTER(EdvGemmDesc), ctypes.c_char_p, ci, vp]
     lib.edv_op_attention.argtypes = [ci, ci, vp, vp, ci, ci, ci, ctypes.c_char_p, ci, vp]
-    lib.edv_op_linear_residual_ln.argtypes = [ci, vp, vp, vp, vp, vp, vp, ctypes.c_float, vp, ci, ci, ci, vp, vp]
+    lib.edv_op_linear_residual_ln.argtypes = [ci, vp, vp, vp, vp, vp, vp, ctypes.c_float, vp, ci, ci, ci, vp, ctypes.c_char_p, ci, vp]
     lib.edv_op_linear_timeline.argtypes = [ci, vp, vp, vp, vp, ci, ci, ci, ci, vp, vp]
     lib.edv_op_attention_timeline.argtypes = [ci, vp, vp, ci, ci, ci, vp, vp]
     lib.edv_op_temporal_attention.argtypes = [ci, vp, vp, ci, ci, ci, ci, vp, ctypes.c_char_p, ci, vp]
@@ -365,16 +365,25 @@ def op_linear(A, W, bias=None, act=0, engine=ENGINE_TC):
     return C
 
 
-def op_linear_residual_ln(A, W, bias, x, gamma=None, beta=None, eps=1e-6, timeline=None):
-    """x (float32 [M,384], updated IN PLACE) += A W^T + bias; returns LayerNorm(x) in A's dtype (None without gamma).
-    timeline: optional int64 [64] device tensor receiving the kernel's own epilogue time stamps."""
+def op_linear_residual_ln_kernel(A, W, bias, x, gamma=None, beta=None, eps=1e-6, xn=None, timeline=None):
+    """-> (xn, name of the kernel instance that ran, e.g. "gemm_ln<bf16>").  x (float32 [M,384], updated IN PLACE) +=
+    A W^T + bias; xn = LayerNorm(x) in A's dtype, None without gamma.  xn: optional caller-owned buffer whose first M rows
+    receive it.  timeline: optional int64 [64] device tensor receiving the kernel's own epilogue time stamps."""
     lib = load_library()
     M, K = A.shape
     N = W.shape[0]
-    xn = torch.empty(M, N, dtype=A.dtype, device=A.device) if gamma is not None else None
+    if gamma is not None and xn is None:
+        xn = torch.empty(M, N, dtype=A.dtype, device=A.device)
+    name = ctypes.create_string_buffer(128)
     _check(lib.edv_op_linear_residual_ln(_dt(A), _ptr(A), _ptr(W), _ptr(bias), _ptr(x), _ptr(gamma), _ptr(beta), ctypes.c_float(eps),
-                                         _ptr(xn), M, N, K, _ptr(timeline), _stream()), None, "edv_op_linear_residual_ln")
-    return xn
+                                         _ptr(xn), M, N, K, _ptr(timeline), name, 128, _stream()), None, "edv_op_linear_residual_ln")
+    return xn, name.value.decode()
+
+
+def op_linear_residual_ln(A, W, bias, x, gamma=None, beta=None, eps=1e-6, timeline=None):
+    """x (float32 [M,384], updated IN PLACE) += A W^T + bias; returns LayerNorm(x) in A's dtype (None without gamma).
+    timeline: optional int64 [64] device tensor receiving the kernel's own epilogue time stamps."""
+    return op_linear_residual_ln_kernel(A, W, bias, x, gamma, beta, eps, timeline=timeline)[0]
 
 
 def op_linear_timeline(A, W, bias=None, act=0):

@@ -30,7 +30,7 @@ typedef struct edv_ctx edv_ctx;
 /* Bumped whenever an entry point's argument list or a struct layout changes.  The ctypes host
  * (endodav_b200/engine.py) mirrors the signatures by hand, so it refuses a library whose
  * edv_abi_version() differs from its own constant instead of calling it with a stale layout. */
-#define EDV_ABI_VERSION 17
+#define EDV_ABI_VERSION 18
 int edv_abi_version(void);
 
 enum edv_status {
@@ -195,11 +195,16 @@ int edv_op_linear_timeline(int dtype, const void* A, const void* W, const float*
 
 /* Row-owning GEMM with fused residual add and LayerNorm (ViT-S, N = 384 only; 16-bit dtypes):
  *   x_inout[M,N] (float32, in place) += A[M,K] W[N,K]^T + bias;  xn_out[M,N] (`dtype`) = LayerNorm(x; gamma, beta, eps).
- * gamma / beta / xn_out NULL: residual update only.  timeline_dev: optional 64 clock64 stamps of the first cluster's
- * epilogue (slot table in csrc/gemm_ln.cuh), else NULL.  Replaces `x = x + ls(proj(.))` / `x = x + ls(fc2(.))` followed by
- * the next norm (layers/block.py:110-116,143-145; LayerScale is folded into W / bias by pack.py). */
+ * gamma, beta and xn_out all NULL: residual update only.  bias may be NULL.  timeline_dev: optional 64 clock64 stamps of the
+ * first cluster's epilogue (slot table in csrc/gemm_ln.cuh), else NULL.  `kernel` (may be NULL) receives the instance that
+ * ran, e.g. "gemm_ln<bf16>".  EDV_ERR_ARG before any launch for a dtype other than bf16 / f16, a NULL A, W or x_inout,
+ * A, W, x_inout or xn_out not 16-byte aligned, gamma / beta / xn_out neither all set nor all NULL, M < 1 or
+ * M > INT_MAX - 127, N != 384, K < 64 or not a multiple of 64, and a negative or non-finite eps.
+ * Replaces `x = x + ls(proj(.))` / `x = x + ls(fc2(.))` followed by the next norm (layers/block.py:110-116,143-145;
+ * LayerScale is folded into W / bias by pack.py). */
 int edv_op_linear_residual_ln(int dtype, const void* A, const void* W, const float* bias, float* x_inout, const float* gamma,
-                              const float* beta, float eps, void* xn_out, int M, int N, int K, long long* timeline_dev, void* stream);
+                              const float* beta, float eps, void* xn_out, int M, int N, int K, long long* timeline_dev, char* kernel,
+                              int kernel_cap, void* stream);
 
 /* Spatial multi-head attention over token-major qkv [F*S, 3*heads*64] (q pre-scaled) ->
  * out [F*S, heads*64].  16-bit with EDV_ENGINE_TC runs the tcgen05 kernel; float32 (under either engine) and

@@ -360,7 +360,10 @@ COVERED = {
     "gemm_tc_kernel": ["test_gpu_ops::test_linear_16bit", "test_gpu_epilogues::test_epilogue_matches_reference"],
     "gemm_bres_kernel": ["test_gpu_ops::test_linear_kernels_agree_bitwise", "test_gpu_epilogues::test_epilogue_matches_reference"],
     "conv3x3_halo_kernel": ["test_gpu_ops::test_conv3x3_16bit", "test_gpu_epilogues::test_epilogue_matches_reference"],
-    "gemm_ln_kernel": ["test_gpu_ops::test_linear_residual_layernorm"],
+    "gemm_ln_kernel": ["test_gpu_gemm_ln::test_gemm_ln_forward_shapes", "test_gpu_gemm_ln::test_gemm_ln_grid_edges",
+                       "test_gpu_gemm_ln::test_gemm_ln_ring_edges", "test_gpu_gemm_ln::test_gemm_ln_families",
+                       "test_gpu_gemm_ln::test_gemm_ln_shapes", "test_gpu_gemm_ln::test_gemm_ln_rows_do_not_depend_on_position",
+                       "test_gpu_gemm_ln::test_gemm_ln_dependent_launches"],
     "head_fused_kernel": ["test_gpu_head::test_head_dpt_shapes", "test_gpu_head::test_head_conv_head_shapes",
                           "test_gpu_head::test_head_tails", "test_gpu_head::test_head_small_shapes",
                           "test_gpu_head::test_head_grid_sizes", "test_gpu_head::test_head_frames_are_independent",

@@ -14,6 +14,7 @@ run attn 300 python -m pytest tests/test_gpu_ops.py -m gpu -q --tb=short -k "att
 run ops_simt 600 python -m pytest tests/test_gpu_ops.py -m gpu -q --tb=short -k "fp32 or temporal or norm or upsample or resize or pyramid or cubic"
 run ops_tc 600 python -m pytest tests/test_gpu_ops.py -m gpu -q --tb=short -k "16bit or bitwise or peaked"
 run head 600 python -m pytest tests/test_gpu_head.py -m gpu -q --tb=short
+run gemm_ln 600 python -m pytest tests/test_gpu_gemm_ln.py -m gpu -q --tb=short
 run fwd_fp32 900 python -m pytest tests/test_gpu_forward.py -m gpu -q --tb=short -k "fp32 or video or order or preprocessing"
 run fwd_16 900 python -m pytest tests/test_gpu_forward.py -m gpu -q --tb=short -k "16bit or determ or repacked or full_size or sweep"
 run smoke 600 python -c "import __graft_entry__ as g; g.smoke()"
